@@ -23,6 +23,8 @@ Intermediate -> Final merge across ranks, and the finalisation of all groups int
   configs : the other BASELINE configs at full size (2: 10 M ungrouped, 3: 60 M TPC-H Q1, 4: 200 M rows / 1 M groups with
           COUNT+SUM DISTINCT), sharded over the same ranks, each with scan time, rows/s, roofline fraction and check.
   cpu_baseline : oracle_ref.c (kind "port") on a bounded sample of config-5 documents, all host cores (N = 1 only).
+  --dump-outputs DIR : the groups of the last timed config-5 step as DIR/<name>.npy (see dump_arrays); the keyspace is
+          seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -146,6 +148,31 @@ def gen_docs_parallel(cref, config, seed, first, n, threads=8, newline=True):
     return buf, offs
 
 
+DUMP_NAMES = ["count", "count_v", "sum_v", "min_v", "max_v"]  # file names of AGGS, in order
+
+
+def dump_arrays(w, res):
+    """The groups of a config-5 result, ordered by group id, as float arrays: group_id (0 = MISSING key, 1 = NULL key,
+    2 + i = the i-th word of the workload's sorted vocabulary), one array per aggregate (float64, exact while |value| < 2^53,
+    NaN for NULL), and agg_class (the N1QL class of every aggregate value: an integer SUM and a float SUM differ)."""
+    import numpy as np
+    rows = res.rows()
+    gid = np.array(w.group_ids(res), dtype=np.float64)
+    val = np.array([[np.nan if v is None else float(v) for v in a] for _k, a in rows], dtype=np.float64).reshape(len(rows), len(AGGS))
+    cls = res.arrays()[2].astype(np.float32).reshape(len(rows), len(AGGS))
+    return gid, val, cls
+
+
+def write_dump(path, gid, val, cls):
+    import numpy as np
+    order = np.argsort(gid, kind="stable")
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "group_id.npy"), gid[order])
+    for j, name in enumerate(DUMP_NAMES):
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(val[order, j]))
+    np.save(os.path.join(path, "agg_class.npy"), cls[order])
+
+
 def same_value(a, b, tol=1e-12):
     """bit-exact, the int / float class of a value included; float64 sums within the north-star tolerance"""
     if isinstance(a, float) and isinstance(b, float):
@@ -233,7 +260,7 @@ def run_ours(args):
             os.environ["NCCL_DEBUG"] = "WARN"  # keep NCCL's version banner off stdout (one JSON line only)
         dist.init_process_group("nccl", device_id=dev)
     q.init(local)
-    K, W = max(1, args.steps), max(args.warmup, 3)
+    K, W = args.steps, max(args.warmup, 3)
     peak, peak_src = peaks()
     trace = bool(os.environ.get("N1GPU_TRACE"))
 
@@ -364,6 +391,15 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     value = w5.rows * K / (ms / 1e3)
     check5 = checked(w5, dq5, res)
+    dump = None
+    if args.dump_outputs:
+        dump = dump_arrays(w5, res)
+        if world > 1:  # rank 0 writes every rank's groups (a replicated merge leaves all of them on rank 0)
+            parts = [None] * world
+            dist.gather_object(dump, parts if rank == 0 else None, dst=0)
+            if rank == 0 and not dq5.replicated:
+                import numpy as np
+                dump = tuple(np.concatenate(x) for x in zip(*parts))
     # the kernel's own duration (roofline) and the latency of one step: K more steps, one at a time, CUDA events around every
     # nq_scan launch on its stream (with two steps in flight an event pair would also time the wait for the SMs)
     scan_ns = []
@@ -610,6 +646,8 @@ def run_ours(args):
         "cpu_baseline": cpu,
         "configs": configs,
     }
+    if dump is not None:
+        write_dump(args.dump_outputs, *dump)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -650,7 +688,7 @@ def run_reference(args):
         return
     from oracle import cref
     cores = os.cpu_count() or 1
-    K, W = max(1, args.steps), max(1, args.warmup)
+    K, W = args.steps, max(1, args.warmup)
     sample = args.cpu_sample
     buf, offs = gen_docs_parallel(cref, 5, 42, 0, sample)
     t0 = time.perf_counter()
@@ -698,7 +736,12 @@ def main():
     ap.add_argument("--e2e-operator", type=int, default=1, help="0: skip the operator-level e2e figure (N = 1)")
     ap.add_argument("--e2e-peer", type=int, default=1, help="0: the e2e steps merge with NCCL instead of the peer arena")
     ap.add_argument("--soak", type=float, default=1.0, help="seconds of untimed stepping before the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the groups of the last timed config-5 step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     # stdout carries exactly ONE JSON line: libraries that print banners to fd 1 (NCCL's version line) are sent to
     # stderr for the duration of the run, and the JSON line goes to the real stdout at the end.
     sys.stdout.flush()
