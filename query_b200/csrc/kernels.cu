@@ -490,7 +490,8 @@ __global__ void __launch_bounds__(1024, 1) k_part_aggregate(const PartPeers P, u
         }
         __syncthreads();
         // a warp per group: lane k folds bitmap words k, k + 32, ... (bank == lane), then a shuffle reduction
-        const i64 neg_below = value_is_int ? (value_bias < 0 ? -value_bias : 0) : 0;  // codes below this are negative values
+        // codes below this are negative values (unsigned: -INT64_MIN does not fit an i64)
+        const u64 neg_below = value_is_int && value_bias < 0 ? 0ULL - (u64)value_bias : 0;
         for (u32 g = warp; g < G; g += nwarps) {
             u64 cnt = 0, code_sum = 0, nneg = 0;
             for (u32 k = lane; k < WPG; k += 32) {
@@ -501,7 +502,7 @@ __global__ void __launch_bounds__(1024, 1) k_part_aggregate(const PartPeers P, u
                     // sum of the set bit positions: 32 * k * popc + sum over j of 2^j * popc(w & bits whose position has bit j)
                     code_sum += (u64)(32u * k) * __popc(w) + __popc(w & 0xaaaaaaaau) + 2u * __popc(w & 0xccccccccu) + 4u * __popc(w & 0xf0f0f0f0u) +
                                 8u * __popc(w & 0xff00ff00u) + 16u * __popc(w & 0xffff0000u);
-                    const i64 lo = (i64)(32u * k);
+                    const u64 lo = 32u * k;
                     if (neg_below > lo) nneg += neg_below >= lo + 32 ? (u64)__popc(w) : (u64)__popc(w & ((1u << (u32)(neg_below - lo)) - 1u));
                 }
             }
