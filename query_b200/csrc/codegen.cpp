@@ -26,6 +26,11 @@ namespace n1 {
 
 namespace {
 
+// N1GPU_* tuning and test knobs, read when a query is compiled: a flag is on when its value starts with '1'; a number
+// is the value's atoi, `fallback` when the variable is not set (each call site checks the range it accepts)
+bool env_flag(const char* name) { const char* v = getenv(name); return v && *v == '1'; }
+int env_int(const char* name, int fallback) { const char* v = getenv(name); return v ? atoi(v) : fallback; }
+
 struct StrCtx {
     int dict_col = -1;
     std::vector<std::string> locals;  // sorted constants when no dictionary is involved
@@ -50,7 +55,7 @@ struct Gen {
     std::map<int, std::string> colvar;  // per-row cache of column Val variables
     std::vector<i64> consts;            // payloads handed to the kernel as p.cst[k] (at most 32; more stay literals)
     bool const_args = true;
-    explicit Gen(const Table& tt) : t(tt) { const char* e = getenv("N1GPU_CONST_LITERALS"); const_args = !(e && *e == '1'); }
+    explicit Gen(const Table& tt) : t(tt) { const_args = !env_flag("N1GPU_CONST_LITERALS"); }
     // the payload of a constant as an expression: a kernel argument slot of its own (numbered by occurrence, never by
     // value: the text must not depend on the payloads), else a literal
     std::string payload_ref(i64 bits) {
@@ -242,8 +247,7 @@ PackComp make_comp(const Table& t, const Expr& e, const char* what) {
     // offset packing: exactly one payload class, bounded
     {
         const bool has_i = ti.mask & bit(C_INT), has_f = ti.mask & bit(C_FLOAT), has_s = ti.mask & bit(C_STRING);
-        const char* no = getenv("N1GPU_NO_OFFSET_PACK");
-        if (!(no && *no == '1') && pc.classes.size() > 1 && !has_f && (has_i != has_s) && (!has_i || pc.biased) && pb < 62) {
+        if (!env_flag("N1GPU_NO_OFFSET_PACK") && pc.classes.size() > 1 && !has_f && (has_i != has_s) && (!has_i || pc.biased) && pb < 62) {
             const int pcls = has_i ? C_INT : C_STRING;
             const u64 range = has_i ? (u64)ti.hi - (u64)ti.lo + 1 : (u64)std::max<i64>(1, t.cols[pc.dict_col].stats.ndict);
             const int nfree = (int)pc.classes.size() - 1;
@@ -393,8 +397,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     // does the chain also compute plain MIN and MAX of this (INT-or-absent) operand?  Then a SUM over it reads the sign mix
     // of its ints off them (value/integer.go:266-277 only asks whether both signs occurred)
     auto int_minmax_of = [&](const std::string& ot) {
-        const char* ns = getenv("N1GPU_NO_SIGN_FROM_MINMAX");
-        if (ns && *ns == '1') return false;
+        if (env_flag("N1GPU_NO_SIGN_FROM_MINMAX")) return false;
         bool mn = false, mx = false;
         for (auto& x : aggs) {
             if (x->kind != EK::AGG || x->distinct || x->star || x->ops.empty() || x->ops[0]->str() != ot) continue;
@@ -440,7 +443,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             if (ap.star || (ap.opmask & ~counted) == 0) ap.w_cnt = rows_word();  // every selected row counts
             else ap.w_cnt = add_word(OP_ADD_U64, (ap.kind == AggKind::COUNT ? "cnt:" : "cntn:") + ot, true);
         } else if ((ap.kind == AggKind::SUM || ap.kind == AggKind::AVG) && (ap.opmask & bit(C_INT)) && (ap.opmask & bit(C_FLOAT)) &&
-                   opnd->ti.imax * std::max(1.0, total_rows_bound) < 9.0e15 && !(getenv("N1GPU_NO_FCARRY") && *getenv("N1GPU_NO_FCARRY") == '1')) {
+                   opnd->ti.imax * std::max(1.0, total_rows_bound) < 9.0e15 && !env_flag("N1GPU_NO_FCARRY")) {
             // INT and FLOAT values mixed, ints provably small: one float64 word carries both (see AggPlan::fcarry)
             const std::string ot = opnd->str();
             ap.fcarry = true;
@@ -527,14 +530,12 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             u64 tight = 1;
             std::vector<u64> dom;
             for (auto& pc : kp.keys) { const u64 d = comp_values(t, pc); dom.push_back(d); tight = d ? tight * d : 0; }
-            const char* nt = getenv("N1GPU_NO_TIGHT");
-            if (tight > 0 && (i64)tight < kp.dense_slots && kp.ndistinct == 0 && !(nt && *nt == '1')) { kp.dense_dom = dom; kp.dense_slots = (i64)tight; }
+            if (tight > 0 && (i64)tight < kp.dense_slots && kp.ndistinct == 0 && !env_flag("N1GPU_NO_TIGHT")) { kp.dense_dom = dom; kp.dense_slots = (i64)tight; }
         }
         // A handful of groups (TPC-H Q1: 6) would serialise every row on the same few shared-memory words.  When the
         // whole table is <= 48 words, every thread keeps its own copy in shared memory (bank = thread: conflict-free
         // plain read-modify-write, no atomics) and the copies are folded once per block.
-        const char* np = getenv("N1GPU_NO_PRIV");
-        if (kp.dense_slots * W <= 48 && !(np && *np == '1')) {
+        if (kp.dense_slots * W <= 48 && !env_flag("N1GPU_NO_PRIV")) {
             kp.dense_priv = true;
             // Block shape: cells x 8 bytes per thread decide how many threads an SM holds (config 3: 42 cells = 336 bytes ->
             // 2 blocks x 256 threads = 16 warps, a quarter of the SM: ncu shows the scan latency-bound, issue 53 %, DRAM 48 %).
@@ -542,12 +543,12 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             // instead (config 3: 1 x 640 threads = 20 warps; 718 -> 645 us per 60 M rows).  The private cells stay conflict-free
             // for any multiple of 32.
             const i64 cells = kp.dense_slots * W;
-            const char* pb = getenv("N1GPU_PRIV_BLOCK");
+            const int pb = env_int("N1GPU_PRIV_BLOCK", 0);
             auto blocks_of = [&](int block) {  // private cells + the per-warp fold buffer + the reserved KiB of every block
                 return (int)std::min<i64>((i64)(227 * 1024) / (cells * 8 * block + cells * 8 * (block / 32) + 1536), 2048 / block);
             };
             int best_block = 256;
-            if (pb && atoi(pb) >= 32 && atoi(pb) <= 1024 && atoi(pb) % 32 == 0) best_block = atoi(pb);
+            if (pb >= 32 && pb <= 1024 && pb % 32 == 0) best_block = pb;
             else if (blocks_of(256) < 4) {
                 int best_warps = blocks_of(256) * 8;
                 for (int block = 128; block <= 1024; block += 32) {
@@ -563,26 +564,23 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         // A packed key of few bits indexes the HBM table directly: no key array, no hash probe, no insert race, the
         // table (config 5: 2^19 slots x 6 words = 25 MB) stays in L2, and because slot == key on every rank the
         // multi-GPU merge is element-wise (all_gather + k_merge_words, stream-ordered) instead of a record exchange.
-        const char* nd = getenv("N1GPU_NO_DIRECT");
         const double slots = kp.key_bits <= 22 ? (double)((i64)1 << kp.key_bits) : 1e30;
         // (every partition must take the same decision - their states are merged slot by slot - so it is based on the rows
         // of the whole keyspace when they are declared, never on this partition's own share)
-        if (!(nd && *nd == '1') && slots * W * 8 <= 256.0 * 1024 * 1024 && slots <= 8.0 * std::max<double>((double)layout_rows, 131072.0)) {
+        if (!env_flag("N1GPU_NO_DIRECT") && slots * W * 8 <= 256.0 * 1024 * 1024 && slots <= 8.0 * std::max<double>((double)layout_rows, 131072.0)) {
             kp.mode = MODE_DENSE;
             kp.dense_global = true;
             kp.dense_slots = (i64)1 << kp.key_bits;
         } else kp.mode = MODE_HASH64;
         // shared-memory front cache for hot keys (Zipf-skewed GROUP BY)
-        const char* nc = getenv("N1GPU_NO_CACHE");
-        if (!(nc && *nc == '1')) {
+        if (!env_flag("N1GPU_NO_CACHE")) {
             // cell layout (see n1ql_device.cuh "Cells of the front cache")
             for (int w = 0; w < W; ++w) {
                 const int op = kp.word_ops[w];
                 int kind = CK_64;
                 // an integer sum whose addends are within +-2^31: ONE 32-bit cell, the (rare) carries go straight to the table word
-                const char* nw1 = getenv("N1GPU_NO_WIDE1");
                 const bool small_addends = kp.word_lo[w] <= kp.word_hi[w] && kp.word_lo[w] > -((i64)1 << 31) && kp.word_hi[w] < ((i64)1 << 31);
-                if (op == OP_ADD_U64) kind = kp.word_count[w] ? CK_CNT : ((small_addends && kp.dense_global && !(nw1 && *nw1 == '1')) ? CK_WIDE1 : CK_WIDE);
+                if (op == OP_ADD_U64) kind = kp.word_count[w] ? CK_CNT : ((small_addends && kp.dense_global && !env_flag("N1GPU_NO_WIDE1")) ? CK_WIDE1 : CK_WIDE);
                 else if (op == OP_OR_U64) kind = CK_OR32;
                 else if (op != OP_ADD_F64 && kp.word_lo[w] <= kp.word_hi[w] && (u64)kp.word_hi[w] - (u64)kp.word_lo[w] <= 0xfffffffcULL) kind = CK_MM32;
                 kp.cell_kind.push_back(kind);
@@ -590,17 +588,14 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
                 else { kp.cell_idx.push_back(kp.cache_n32); kp.cache_n32 += kind == CK_WIDE ? 2 : 1; }
             }
             kp.cell_pair.assign((size_t)W, 0);
-            {
-                const char* npair = getenv("N1GPU_NO_MM_PAIR");
-                const char* ncheck = getenv("N1GPU_NO_CELL_CHECK");
-                if (!(npair && *npair == '1') && !(ncheck && *ncheck == '1'))
-                    for (int w = 0; w + 1 < W; ++w)
-                        if (kp.cell_kind[w] == CK_MM32 && kp.cell_kind[w + 1] == CK_MM32 && kp.cell_idx[w + 1] == kp.cell_idx[w] + 1 && kp.cell_pair[w] == 0) {
-                            kp.cell_pair[w] = 1; kp.cell_pair[w + 1] = 2; ++w;
-                        }
-            }
-            const char* nk = getenv("N1GPU_NO_KEY32");
-            kp.cache_key32 = kp.key_bits <= 31 && !(nk && *nk == '1');  // u32 keys in buckets of four (cache_claim_b4)
+            if (!env_flag("N1GPU_NO_MM_PAIR"))
+                for (int w = 0; w + 1 < W; ++w)
+                    if (kp.cell_kind[w] == CK_MM32 && kp.cell_kind[w + 1] == CK_MM32 && kp.cell_idx[w + 1] == kp.cell_idx[w] + 1 && kp.cell_pair[w] == 0) {
+                        kp.cell_pair[w] = 1; kp.cell_pair[w + 1] = 2; ++w;
+                    }
+            // u32 keys, direct-mapped (cache_claim_1).  Buckets of four keys were removed: 5.19 against 4.95 ms per 1 B
+            // config-5 rows (profiles/r02_config5_ablation.jsonl)
+            kp.cache_key32 = kp.key_bits <= 31 && !env_flag("N1GPU_NO_KEY32");
             const int slot_bytes = (kp.cache_key32 ? 4 : 8) + 8 * kp.cache_n64 + 4 * kp.cache_n32;
             // The five 256-thread blocks of an SM each cache the same hot keys in their own 44 KiB; one 1024-thread block
             // caches five times as many distinct keys in the SM's 220 KiB.  Measured on config 5 (Zipf over 100 k keys,
@@ -608,14 +603,14 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             // 3-4 scattered L2 reductions, one LSU wavefront each, and LSU wavefronts are what the kernel runs out of.
             // So: the small block when its cache holds every group anyway or the key domain is far beyond any cache
             // (uniform high-cardinality keys: occupancy matters more), the large block in between.
-            const char* kb = getenv("N1GPU_CACHE_KB");      // shared memory per block spent on the cache
-            const char* bt = getenv("N1GPU_CACHE_BLOCK");   // threads per block
-            const char* lb = getenv("N1GPU_MIN_BLOCKS");    // resident blocks per SM
+            const int kb = env_int("N1GPU_CACHE_KB", 0);     // shared memory per block spent on the cache
+            const int bt = env_int("N1GPU_CACHE_BLOCK", 0);  // threads per block
+            const int lb = env_int("N1GPU_MIN_BLOCKS", 0);   // resident blocks per SM
             const double slots_small = 44.0 * 1024 / slot_bytes, slots_large = 220.0 * 1024 / slot_bytes;
-            kp.block = bt && atoi(bt) >= 64 ? atoi(bt) / 32 * 32 : (est > 0.8 * slots_small && est <= 64.0 * slots_large ? 1024 : 256);
-            cache_blocks = lb && atoi(lb) > 0 ? atoi(lb) : std::max(1, 1280 / kp.block);
+            kp.block = bt >= 64 ? bt / 32 * 32 : (est > 0.8 * slots_small && est <= 64.0 * slots_large ? 1024 : 256);
+            cache_blocks = lb > 0 ? lb : std::max(1, 1280 / kp.block);
             // the resident blocks of an SM share 220 of its 227 KiB (each block also pays 1 KiB of system shared memory)
-            const i64 budget = (kb && atoi(kb) > 0 ? atoi(kb) : 220 / cache_blocks) * 1024;
+            const i64 budget = (kb > 0 ? kb : 220 / cache_blocks) * 1024;
             i64 cs = budget / slot_bytes / 64 * 64;
             const i64 need = (i64)std::min(4.0 * std::max(est, 1.0), 1e9);  // never more than the groups need
             if (cs > need) cs = std::max<i64>(64, (need + 63) / 64 * 64);
@@ -633,11 +628,10 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     // statistics say those are the minority.  Every partition must decide alike, so the decision only uses agreed
     // numbers: the declared keyspace rows with exchanged statistics, this table's own rows otherwise.
     if (kp.cache_slots > 0 && w_rows == 0) {
-        const char* nc = getenv("N1GPU_NO_COMPLEMENT");
         bool forced = false;
         for (auto& c : t.cols) forced = forced || c.stats_forced;
         const i64 denom = t.global_rows > 0 ? std::max(t.global_rows, t.nrows) : (forced ? 0 : t.nrows);
-        for (size_t a = 0; a < aggs.size() && !(nc && *nc == '1') && denom > 0; ++a) {
+        for (size_t a = 0; a < aggs.size() && !env_flag("N1GPU_NO_COMPLEMENT") && denom > 0; ++a) {
             const Expr& e = *aggs[a];
             if (e.star || e.distinct || e.ops.empty()) continue;
             const Expr* opnd = e.ops[0].get();
@@ -653,8 +647,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     // bounds a skewed GROUP BY (profiles/r01_atomic_probe.txt: 190 G scattered RED/s whatever their width).  Row
     // counters are therefore packed two per 64-bit word (32-bit fields) when no counter can reach 2^32 over all ranks.
     {
-        const char* np = getenv("N1GPU_NO_PACK");
-        const bool pack = kp.cache_slots > 0 && kp.ndistinct == 0 && !(np && *np == '1') && total_rows_bound < 4294967295.0;
+        const bool pack = kp.cache_slots > 0 && kp.ndistinct == 0 && !env_flag("N1GPU_NO_PACK") && total_rows_bound < 4294967295.0;
         kp.phys_of.assign(W, -1); kp.shift_of.assign(W, 0); kp.bits_of.assign(W, 64);
         int pending = -1;  // counter waiting for a partner
         for (int w = 0; w < W; ++w) {
@@ -684,16 +677,15 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         // with a dependent compare-and-swap, and 2^bits / 8 bytes instead of 16 bytes per row - config 4's 2^30
         // entries are 128 MiB, about the size of the L2, where the hash set is 4 GiB of random DRAM sectors.
         // Chosen when the bitmap is no larger than the hash set would be.
-        const char* nb = getenv("N1GPU_NO_BITMAP");
         const double bitmap_bytes = kp.entry_bits <= 36 ? (double)((u64)1 << kp.entry_bits) / 8.0 : 1e30;
-        kp.set_bitmap = !(nb && *nb == '1') && bitmap_bytes <= std::max(65536.0, 16.0 * (double)std::max<i64>(layout_rows, 1) * kp.ndistinct);
+        kp.set_bitmap = !env_flag("N1GPU_NO_BITMAP") && bitmap_bytes <= std::max(65536.0, 16.0 * (double)std::max<i64>(layout_rows, 1) * kp.ndistinct);
         // A bitmap the size of the L2 (config 4: 128 MiB) turns every row into a random DRAM sector read-modify-write.
         // The scan then runs in passes over slices of the entry range small enough to stay L2-resident: the columns
         // are streamed once per pass (cheap next to random DRAM), the bits land in L2.
         if (kp.set_bitmap) {
-            const char* sp = getenv("N1GPU_SET_PASSES");
+            const int sp = env_int("N1GPU_SET_PASSES", 0);
             int passes = 1;
-            if (sp && atoi(sp) >= 1) passes = atoi(sp);
+            if (sp >= 1) passes = sp;
             // measured (config 4, 200 M rows, 128 MiB bitmap; profiles/r01_config4_bitmap_passes.jsonl): 1 pass 5.58 ms,
             // 2 passes 3.23 ms, 4 passes 3.45 ms, 8 passes 5.41 ms - a pass costs ~0.65 ms of streaming and key work, so
             // the slices are made just small enough (<= 64 MiB) for most of their sectors to stay in the 126 MB L2
@@ -854,8 +846,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     // ---- partitioned DISTINCT aggregation (see KernelPlan::part) --------------------------------------------------
     std::string part_value_code;
     {
-        const char* np = getenv("N1GPU_NO_PART");
-        bool ok = kp.mode == MODE_DENSE && kp.dense_global && kp.ndistinct == 1 && kp.cache_slots > 0 && !(np && *np == '1');
+        bool ok = kp.mode == MODE_DENSE && kp.dense_global && kp.ndistinct == 1 && kp.cache_slots > 0 && !env_flag("N1GPU_NO_PART");
         const AggPlan* da = nullptr;
         const Expr* dexpr = nullptr;
         for (size_t a = 0; a < kp.aggs.size() && ok; ++a) {
@@ -872,17 +863,12 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         if (ok) {
             const int KB = kp.key_bits, VB = da->dcomp.bits();
             int PB = std::max(1, std::max(KB + VB - 20, KB - 12));   // a partition's bitmap <= 2^20 bits, <= 4096 groups
-            const char* fp = getenv("N1GPU_PART");                   // "1": also for keyspaces too small to profit (tests)
-            const bool force = fp && *fp == '1';
+            const bool force = env_flag("N1GPU_PART");               // also for keyspaces too small to profit (tests)
             ok = VB >= 1 && VB <= 12 && PB <= 10 && PB < KB && (KB - PB) + 1 + VB <= 32 && (force || layout_rows >= ((i64)1 << (PB + 12)));
             if (ok) {
                 kp.part = true;
                 kp.part_bits = PB; kp.part_gbits = KB - PB; kp.part_vbits = VB;
-                {
-                    const char* pbk = getenv("N1GPU_PART_BLOCK");
-                    if (pbk && (atoi(pbk) == 512 || atoi(pbk) == 256)) kp.part_block = atoi(pbk);
-                }
-                kp.part_bincap = std::max(8, std::min(48, (int)((192 * 1024 / (1024 / kp.part_block)) / (4 << PB))));
+                kp.part_bincap = std::max(8, std::min(48, 192 * 1024 / (4 << PB)));
                 kp.part_smem = (4 << PB) * (1 + kp.part_bincap);
                 g.body.clear();
                 g.ind = "                    ";
@@ -907,10 +893,8 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     for (int c : kp.used_cols) kp.scan_bytes_per_row += t.scan_bytes(c);
 
     // ---- assemble the kernel ------------------------------------------------------------------------------------
-    std::vector<int> pre_words;  // physical min / max / or words whose current value a miss reads ahead (direct table)
     std::string s;
     s += "// generated by libn1gpu codegen: one specialised scan kernel for this Filter + Group chain\n";
-    { const char* nc = getenv("N1GPU_NO_CELL_CHECK"); if (nc && *nc == '1') s += "#define NQ_NO_CELL_CHECK 1\n"; }
     s += "#include \"n1ql_device.cuh\"\n";
     s += strf("#define NQ_W %d\n", W);
     s += "#define ACCIF(k, OP, x, c) if (c) { ACC(k, OP, x); }\n";
@@ -928,24 +912,14 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     else if (cached) {
         s += strf("#define NQ_CS %d\n", kp.cache_slots);
         // table update of a cache miss, per logical word: packed counters gather in a register (one RED per physical
-        // word and row, issued after the row's aggregate code); min / max / or words can read the slot first
-        // (in the direct-indexed table the slot is the key itself, so those reads can be issued for all four rows
-        // before the cached rows are updated)
-        // Measured on config 5 (tools/sweep_config5.py, 200 M rows): reading first LOSES 20 % (1 277 -> 1 563 us; read ahead
-        // 1 766 us) - the kernel is bound by LSU wavefronts, and a scattered load costs as many as the reduction it
-        // saves.  Both stay experiment knobs: N1GPU_MMCHECK=1 (read first), N1GPU_MMCHECK=2 (read ahead).
-        const char* nm = getenv("N1GPU_MMCHECK");
-        const bool mmcheck = nm && (*nm == '1' || *nm == '2');
-        const bool mmpre = mmcheck && kp.dense_global && *nm == '2';
+        // word and row, issued after the row's aggregate code), every other word is one reduction.  The table's min / max /
+        // or word is not read before its reduction: on config 5 reading first lost 20 % (1 277 -> 1 563 us per 200 M rows,
+        // reading ahead for all four rows 1 766 us) and 43 % per 1 B rows (profiles/r02_config5_ablation.jsonl) - the
+        // kernel is bound by LSU wavefronts, and a scattered load costs as many as the reduction it saves.
         for (int w = 0; w < W; ++w) {
-            const int P = kp.phys_of[w], op = kp.word_ops[w];
-            const bool chk = mmcheck && op != OP_ADD_U64 && op != OP_ADD_F64;
+            const int P = kp.phys_of[w];
             if (kp.bits_of[w] != 64) s += strf("#define ACCM_%d(OP, val_) pk%d += (u64)(val_) << %d\n", w, P, kp.shift_of[w]);
-            else if (chk && mmpre) {
-                s += strf("#define ACCM_%d(OP, val_) table_word_known<OP>(&p.acc[%dULL * cap + (u64)slot], (u64)(val_), mm[j][%d])\n", w, P, (int)pre_words.size());
-                pre_words.push_back(P);
-            }
-            else s += strf("#define ACCM_%d(OP, val_) %s<OP>(&p.acc[%dULL * cap + (u64)slot], (u64)(val_))\n", w, chk ? "table_word_checked" : "atomic_word", P);
+            else s += strf("#define ACCM_%d(OP, val_) atomic_word<OP>(&p.acc[%dULL * cap + (u64)slot], (u64)(val_))\n", w, P);
         }
         for (int w = 0; w < W; ++w) {
             std::string hit;
@@ -968,39 +942,11 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             }
             s += strf("#define ACCH_%d(OP, val_) %s\n", w, hit.c_str());
         }
-        // Register groups (experiment knob N1GPU_REG_GROUPS=1, off by default).  When the single key component has
-        // payload-free classes (MISSING / NULL / a boolean), those few groups take a large share of the rows (config 5: one
-        // row in five has no string key) and every one of them is a shared-memory atomic on the same few cells.  Each
-        // thread can keep their accumulators in registers instead; warps reduce them at the end of the kernel and lane 0
-        // applies one atomic per word to the direct-indexed table (slot = packed key = class index).
-        // Measured per 1 B config-5 rows: the hand-written prototype (tools/proto5.cu, 32-bit keys and values) gains 15 %
-        // from it (5.33 -> 4.55 ms); in the generated kernel the same idea LOSES 16 % (4.93 -> 5.72 ms straight-line
-        // and masked, 5.63 predicated under the `pass` branch, 5.89 branched): ~55 extra instructions per row against the
-        // prototype's ~16, on a kernel that is already issue-limited.  Kept under test for narrower aggregate lists.
-        {
-            const char* nr = getenv("N1GPU_REG_GROUPS");
-            const PackComp& pc0 = kp.keys[0];
-            if (nr && *nr == '1' && kp.keys.size() == 1 && kp.dense_global && kp.ndistinct == 0 && kp.set_passes <= 1 && pc0.nfree >= 1 &&
-                pc0.nfree <= 2 && W * pc0.nfree <= 16)
-                kp.reg_groups = pc0.nfree;
-        }
-        for (int w = 0; w < W && kp.reg_groups; ++w) {
-            std::string upd;
-            switch (kp.cell_kind[w]) {
-                case CK_CNT: upd = strf("rg##G##_%d += (u32)(val_) & rgm##G", w); break;
-                case CK_WIDE: case CK_WIDE1: upd = strf("rg##G##_%d += (u64)(val_) & (((u64)rgm##G << 32) | rgm##G)", w); break;
-                case CK_MM32: upd = strf("if (rgh##G) reg_mm32<OP>(rg##G##_%d, (u64)(val_), %lluULL)", w, (unsigned long long)kp.word_lo[w]); break;
-                case CK_OR32: upd = strf("rg##G##_%d |= (u32)(val_) & rgm##G", w); break;
-                default: upd = strf("if (rgh##G) rg##G##_%d = word_combine(OP, rg##G##_%d, (u64)(val_))", w, w); break;
-            }
-            s += strf("#define RACC_%d(G, OP, val_) %s\n", w, upd.c_str());
-        }
     }
     else s += "#define ACC(k, OP, x) if (nq_first) atomic_word<OP>(&p.acc[(u64)(k) * cap + (u64)slot], (u64)(x))\n";
     {
         // resident blocks per SM the register allocator must allow (tuning knob N1GPU_MIN_BLOCKS; 0 = compiler's choice)
-        const char* lb = getenv("N1GPU_MIN_BLOCKS");
-        int minb = lb ? atoi(lb) : 0;
+        int minb = env_int("N1GPU_MIN_BLOCKS", 0);
         s += strf("#define NQ_BLOCK %d\n", kp.block);
         if (minb == 0 && cached) minb = cache_blocks;  // the front cache is sized for this many resident blocks
         // One 1024-thread block per SM at 64 registers per thread owns the whole register file: no other kernel - the next
@@ -1008,8 +954,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         // ends.  Capped at 56 registers the scan leaves 8 K registers per SM, enough for a 256-thread block of those, so a
         // second step in flight overlaps its merge and finalisation with this scan.  (__maxnreg__ replaces
         // __launch_bounds__: the two cannot be combined.)
-        const char* mr = getenv("N1GPU_MAXREG");
-        const int cap_regs = mr ? atoi(mr) : (cached && kp.block == 1024 ? 56 : 0);
+        const int cap_regs = cached && kp.block == 1024 ? 56 : 0;
         if (cap_regs > 0 && cap_regs * kp.block <= 65536) s += strf("extern \"C\" __global__ void __maxnreg__(%d) nq_scan(const NqParams p) {\n", cap_regs);
         else if (minb > 0) s += strf("extern \"C\" __global__ void __launch_bounds__(NQ_BLOCK, %d) nq_scan(const NqParams p) {\n", minb);
         else s += "extern \"C\" __global__ void __launch_bounds__(NQ_BLOCK) nq_scan(const NqParams p) {\n";
@@ -1018,8 +963,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         // An ungrouped scan consumes nothing that a stream-preceding kernel produces (its table was sealed with a
         // device synchronisation, its state belongs to this query handle alone), so the next kernel of the stream
         // may be scheduled as soon as SMs free up: programmatic dependent launch.
-        const char* np = getenv("N1GPU_NO_PDL");
-        kp.pdl = kp.mode == MODE_UNGROUPED && !(np && *np == '1');
+        kp.pdl = kp.mode == MODE_UNGROUPED && !env_flag("N1GPU_NO_PDL");
         if (kp.pdl) s += "    asm volatile(\"griddepcontrol.launch_dependents;\");\n";
     }
     // later passes over a sliced DISTINCT bitmap only set bits: the group table was fed by pass 0
@@ -1040,7 +984,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             s += "    extern __shared__ u64 s_dyn[];\n";
             if (kp.cache_key32) {
                 s += strf("    u64* const s_c64 = s_dyn;             // [%d][NQ_CS] 64-bit cells\n", kp.cache_n64);
-                s += strf("    u32* const s_ckey = (u32*)(s_dyn + %d * NQ_CS);  // [NQ_CS] cached group keys in buckets of four (all ones = empty)\n", kp.cache_n64);
+                s += strf("    u32* const s_ckey = (u32*)(s_dyn + %d * NQ_CS);  // [NQ_CS] cached group keys, direct-mapped (all ones = empty)\n", kp.cache_n64);
                 s += strf("    u32* const s_c32 = s_ckey + NQ_CS;    // [%d][NQ_CS] 32-bit cells\n", kp.cache_n32);
             } else {
                 s += "    u64* const s_ckey = s_dyn;            // [NQ_CS] cached group keys (all ones = empty)\n";
@@ -1064,16 +1008,6 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             s += "    bool cache_on = nq_first;  // per warp: switched off after 4 tiles when fewer than 1 in 4 rows hit\n";
             s += "    unsigned nlook = 0, nhit = 0; int tiles = 0;\n";
         }
-        for (int gi = 0; gi < kp.reg_groups; ++gi)
-            for (int w = 0; w < W; ++w) {
-                const int op = kp.word_ops[w];
-                switch (kp.cell_kind[w]) {
-                    case CK_CNT: case CK_OR32: s += strf("    u32 rg%d_%d = 0;\n", gi, w); break;
-                    case CK_WIDE: case CK_WIDE1: s += strf("    u64 rg%d_%d = 0;\n", gi, w); break;
-                    case CK_MM32: s += strf("    u32 rg%d_%d = %s;\n", gi, w, (op == OP_MIN_I64 || op == OP_MIN_U64) ? "0xffffffffu" : "0u"); break;
-                    default: s += strf("    u64 rg%d_%d = word_identity(%s);\n", gi, w, op_name(op)); break;
-                }
-            }
     }
     s += "    const i64 nrows = p.nrows;\n";
     s += "    const int lane = threadIdx.x & 31;\n";
@@ -1105,52 +1039,19 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             s += "                pass = pass && w_true;\n";
         }
         s += "            cs[j] = -2; kk[j] = 0;\n";
-        if (kp.reg_groups) {
-            // Straight-line and predicated, outside the `pass` branch: one row in five takes this path in config 5, so
-            // nearly every warp would run both sides of a branch, and accumulators updated under a branch cost a register
-            // move per update at the join (measured: branched 5.89 ms, predicated under the branch 5.63 ms per 1 B rows,
-            // against 4.94 ms without register groups).
-            s += "            {\n";
-            s += key_code;
-            for (int gi = 0; gi < kp.reg_groups; ++gi) {
-                s += strf("                    { const bool rgh%d = pass && klo == %dULL; const u32 rgm%d = rgh%d ? 0xffffffffu : 0u; (void)rgm%d;\n", gi, gi, gi, gi, gi);
-                s += strf("#define ACC(k, OP, val_) RACC_##k(%d, OP, val_)\n", gi);
-                s += agg_code;
-                s += "#undef ACC\n";
-                s += "                    }\n";
-            }
-            s += "            if (pass) {\n";
-            s += "                    kk[j] = klo;\n";
-            s += strf("                    if (klo < %dULL) cs[j] = -3;  // register group: no probe, no atomic\n", kp.reg_groups);
-            s += "                    else {\n";
-        } else {
-            s += "            if (pass) {\n";
-            s += key_code;
-            s += "                    kk[j] = klo;\n";
-        }
+        // MISSING / NULL keys (one row in five of config 5, two slots) are cached like any other key.  Register
+        // accumulators for them were removed: -16 % per 1 B config-5 rows (4.95 -> 5.72 ms, profiles/r02_config5_ablation.jsonl),
+        // ~55 extra instructions per row on a kernel whose issue slots are already 68 % busy.
+        s += "            if (pass) {\n";
+        s += key_code;
+        s += "                    kk[j] = klo;\n";
         s += "                    ++nlook;\n";
-        {
-            const char* cw = getenv("N1GPU_CACHE_WAYS");  // 4: buckets of four keys (one LDS.128), default: direct-mapped
-            if (kp.cache_key32 && cw && atoi(cw) == 4) s += "                    cs[j] = cache_on ? cache_claim_b4(s_ckey, NQ_CS / 4, (u32)klo * 0x9E3779B1u, (u32)klo) : -1;\n";
-            else if (kp.cache_key32) s += "                    cs[j] = cache_on ? cache_claim_1(s_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, (u32)klo) : -1;\n";
-        }
-        if (kp.cache_key32) {}
+        if (kp.cache_key32) s += "                    cs[j] = cache_on ? cache_claim_1(s_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, (u32)klo) : -1;\n";
         else if (kp.key_bits <= 32) s += "                    cs[j] = cache_on ? cache_claim_n(s_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, klo) : -1;\n";
         else s += "                    cs[j] = cache_on ? cache_claim_n(s_ckey, NQ_CS, (u32)(mix64(klo) >> 32), klo) : -1;\n";
         s += "                    nhit += cs[j] >= 0;\n";
-        if (kp.reg_groups) s += "                    }\n            }\n";
         s += "            }\n";
         s += "        }\n";
-        if (!pre_words.empty()) {
-            s += strf("        u64 mm[4][%d];  // current table value of the min / max / or words of a missed row\n", (int)pre_words.size());
-            s += "#pragma unroll\n";
-            s += "        for (int j = 0; j < 4; ++j) {\n";
-            for (size_t i = 0; i < pre_words.size(); ++i) s += strf("            mm[j][%d] = 0;\n", (int)i);
-            s += "            if (cs[j] == -1) {\n";
-            for (size_t i = 0; i < pre_words.size(); ++i) s += strf("                mm[j][%d] = __ldcg(&p.acc[%dULL * cap + kk[j]]);\n", (int)i, pre_words[i]);
-            s += "            }\n";
-            s += "        }\n";
-        }
         s += "#define ACC(k, OP, val_) if (nq_first) ACCH_##k(OP, val_)\n";
         s += "#pragma unroll\n";
         s += "        for (int j = 0; j < 4; ++j) {\n";
@@ -1251,47 +1152,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             }
         }
         s += "    }\n";
-        // register groups: warp reduction, then one atomic per word from lane 0
-        for (int gi = 0; gi < kp.reg_groups; ++gi) {
-            s += "    {\n";
-            for (int P = 0; P < PW; ++P) {
-                std::string v;
-                for (int w = 0; w < W; ++w)
-                    if (kp.phys_of[w] == P && kp.bits_of[w] != 64) {
-                        // counters (row counts of one warp fit 32 bits) and class-seen bits
-                        const char* red = kp.cell_kind[w] == CK_OR32 ? "__reduce_or_sync" : "__reduce_add_sync";
-                        v += strf("%s((u64)%s(0xffffffffu, rg%d_%d) << %d)", v.empty() ? "" : " | ", red, gi, w, kp.shift_of[w]);
-                    }
-                if (!v.empty()) s += strf("        { const u64 v = %s; if (lane == 0 && v) atomicAdd(&p.acc[%dULL * cap + %dULL], v); }\n", v.c_str(), P, gi);
-            }
-            for (int w = 0; w < W; ++w) {
-                if (kp.bits_of[w] != 64) continue;
-                const int op = kp.word_ops[w];
-                const std::string dst = strf("&p.acc[%dULL * cap + %dULL]", kp.phys_of[w], gi);
-                const bool mn = op == OP_MIN_I64 || op == OP_MIN_U64;
-                switch (kp.cell_kind[w]) {
-                    case CK_CNT:
-                        s += strf("        { const u64 v = __reduce_add_sync(0xffffffffu, rg%d_%d); if (lane == 0 && v) atomic_word<%s>(%s, v); }\n", gi, w, op_name(op), dst.c_str());
-                        break;
-                    case CK_OR32:
-                        s += strf("        { const u64 v = __reduce_or_sync(0xffffffffu, rg%d_%d); if (lane == 0 && v) atomic_word<%s>(%s, v); }\n", gi, w, op_name(op), dst.c_str());
-                        break;
-                    case CK_MM32:
-                        s += strf("        { const u32 c = %s(0xffffffffu, rg%d_%d); if (lane == 0 && c != %s) atomic_word<%s>(%s, (u64)(c - 1u) + %lluULL); }\n",
-                                  mn ? "__reduce_min_sync" : "__reduce_max_sync", gi, w, mn ? "0xffffffffu" : "0u", op_name(op), dst.c_str(),
-                                  (unsigned long long)kp.word_lo[w]);
-                        break;
-                    default:  // 64-bit sums and unranged words
-                        s += strf("        { const u64 v = warp_reduce_word<%s>(rg%d_%d); if (lane == 0 && v != word_identity(%s)) atomic_word<%s>(%s, v); }\n",
-                                  op_name(op), gi, w, op_name(op), op_name(op), dst.c_str());
-                        break;
-                }
-            }
-            s += "    }\n";
-        }
     }
-    const char* nhw = getenv("N1GPU_NO_HOSTWRITE");  // experiment knob: skip the zero-copy result store
-    const bool hostw = !(nhw && *nhw == '1');
     if (kp.mode == MODE_UNGROUPED) {
         // Block epilogue: warp-shuffle reduce every word, one barrier, then thread w folds word w's 8 warp values in
         // order.  Order-independent words (integer add / min / max / or) go straight into persistent accumulators
@@ -1315,7 +1176,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         s += "    if (last_block_arrives(p.ticket)) {\n";
         s += "        if (threadIdx.x < NQ_W && nq_ops[threadIdx.x] != OP_ADD_F64) {\n";
         s += "            const u64 v = atomicExch(&p.acc[threadIdx.x], word_identity(nq_ops[threadIdx.x]));\n";
-        s += hostw ? "            p.final_dev[threadIdx.x] = v; p.final_host[threadIdx.x] = v;\n" : "            p.final_dev[threadIdx.x] = v;\n";
+        s += "            p.final_dev[threadIdx.x] = v; p.final_host[threadIdx.x] = v;\n";
         s += "        }\n";
         {
             int fi = 0;
@@ -1329,8 +1190,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
                 s += "#pragma unroll\n";
                 s += "            for (int k = 1; k < 5; ++k) v = word_combine(OP_ADD_F64, v, t[k]);\n";
                 s += "            v = block_reduce_word<OP_ADD_F64>(v, scratch);\n";
-                s += hostw ? strf("            if (threadIdx.x == 0) { p.final_dev[%d] = v; p.final_host[%d] = v; }\n", w, w)
-                           : strf("            if (threadIdx.x == 0) { p.final_dev[%d] = v; }\n", w);
+                s += strf("            if (threadIdx.x == 0) { p.final_dev[%d] = v; p.final_host[%d] = v; }\n", w, w);
                 s += "        }\n";
                 ++fi;
             }
@@ -1374,9 +1234,9 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         std::string q;
         q += "// generated by libn1gpu codegen: the partitioning kernel of this chain's partitioned DISTINCT aggregation\n";
         q += "#include \"n1ql_device.cuh\"\n";
-        q += strf("#define NQ_BLOCK %d\n", kp.part_block);
+        q += strf("#define NQ_BLOCK %d\n", PART_THREADS);
         q += strf("#define NP %d\n#define BINCAP %d\n#define GBITS %d\n#define ROUND_TILES 8\n", 1 << kp.part_bits, kp.part_bincap, kp.part_gbits);
-        q += strf("extern \"C\" __global__ void __launch_bounds__(NQ_BLOCK, %d) nq_scan(const NqParams p) {\n", 1024 / kp.part_block);
+        q += "extern \"C\" __global__ void __launch_bounds__(NQ_BLOCK, 1) nq_scan(const NqParams p) {\n";
         q += "    extern __shared__ u32 s_part[];\n";
         q += "    __shared__ int s_stop;\n";
         q += "    u32* const s_cnt = s_part;        // [NP] records staged per partition in this round\n";

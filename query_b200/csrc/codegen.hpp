@@ -12,6 +12,9 @@ namespace n1 {
 
 enum : int { MODE_UNGROUPED = 0, MODE_DENSE = 1, MODE_HASH64 = 2, MODE_HASH128 = 3 };
 enum : int { CK_CNT = 0, CK_WIDE = 1, CK_MM32 = 2, CK_OR32 = 3, CK_64 = 4, CK_WIDE1 = 5 };
+// threads per block of the partitioning kernel (KernelPlan::part), one block per SM.  Two 512-thread blocks with half
+// the bins each lost (config 4, 200 M rows: 1.59 -> 1.78 ms; four 256-thread blocks 2.55 ms; DESIGN.md section 9)
+constexpr int PART_THREADS = 1024;
 
 // One bit-packed component: a group-key value or the value of a DISTINCT entry.
 struct PackComp {
@@ -84,7 +87,7 @@ struct KernelPlan {
     bool pdl = false;            // launched with programmatic stream serialization (ungrouped scans)
     int dyn_smem = 0;            // dynamic shared memory the kernel is launched with
     int block = 256;             // threads per block (a block scans block * 4 rows per iteration)
-    bool cache_key32 = false;    // front-cache keys are u32 in 16-byte buckets of four (packed key <= 31 bits)
+    bool cache_key32 = false;    // front-cache keys are u32, direct-mapped (packed key <= 31 bits)
     int cache_slots = 0;         // HASH64: slots of the per-block shared-memory front cache (0 = none)
     // front-cache cell of every word: kind (CK_*) and index of its first cell among the 32-bit / 64-bit cell arrays
     std::vector<int> cell_kind, cell_idx;
@@ -92,9 +95,6 @@ struct KernelPlan {
     // that ONE 64-bit shared-memory load fetches both for the read-before-atomic check: 0 none, 1 first of a pair, 2 second
     std::vector<int> cell_pair;
     int cache_n32 = 0, cache_n64 = 0;
-    // groups whose key is one of the first `reg_groups` packed values (the payload-free classes of a single key component:
-    // MISSING / NULL keys - 20 % of config 5's rows on two groups) are aggregated in per-thread REGISTERS, outside the cache
-    int reg_groups = 0;
     std::vector<AggPlan> aggs;
     int ndistinct = 0, abits = 0, entry_bits = 0;
     bool set128 = false;
@@ -107,12 +107,11 @@ struct KernelPlan {
     // (static) kernel gives every partition to one block, whose share of the bitmap and of the counters fits shared memory,
     // and leaves the finished accumulator words in the group table.  part_* describe the record.
     bool part = false;
-    std::string part_source;     // the partitioning kernel (entry nq_scan, 1024 threads)
+    std::string part_source;     // the partitioning kernel (entry nq_scan, PART_THREADS threads)
     int part_bits = 0;           // partitions = 2^part_bits, taken from the top of the packed group key
     int part_gbits = 0;          // record bits [0, gbits): group key inside its partition; bit gbits: has a value
     int part_vbits = 0;          // record bits above: the packed DISTINCT value
     int part_bincap = 48;        // records a block stages per partition and round in shared memory
-    int part_block = 1024;       // threads per block of the partition kernel (N1GPU_PART_BLOCK: 512 = two blocks per SM with half the bins)
     int part_smem = 0;           // dynamic shared memory of the partitioning kernel
     // payloads of constants / bound parameters, passed to the kernel as NqParams::cst (the source only names the slot)
     std::vector<i64> consts;

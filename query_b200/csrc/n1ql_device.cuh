@@ -301,19 +301,6 @@ template <int OP> NQ_DEV void atomic_word(u64* p, u64 x) {
     else if (OP == OP_MAX_U64) atomicMax(p, x);
     else atomicOr(p, x);
 }
-// Min / max / or into an HBM table word that is read first: an L2 load costs the SM -> L2 request path less than a
-// reduction, and a settled group leaves the word unchanged for almost every row.  The load may be stale; these words
-// only ever move one way, so a stale value can only cause a reduction that was not needed, never skip one that was.
-template <int OP> NQ_DEV void table_word_known(u64* p, u64 x, u64 cur);
-template <int OP> NQ_DEV void table_word_checked(u64* p, u64 x) { table_word_known<OP>(p, x, __ldcg(p)); }
-template <int OP> NQ_DEV void table_word_known(u64* p, u64 x, u64 cur) {  // `cur`: a value the word held earlier
-    if (OP == OP_MIN_I64) { if ((i64)x < (i64)cur) atomicMin((i64*)p, (i64)x); }
-    else if (OP == OP_MAX_I64) { if ((i64)x > (i64)cur) atomicMax((i64*)p, (i64)x); }
-    else if (OP == OP_MIN_U64) { if (x < cur) atomicMin(p, x); }
-    else if (OP == OP_MAX_U64) { if (x > cur) atomicMax(p, x); }
-    else if (OP == OP_OR_U64) { if ((cur & x) != x) atomicOr(p, x); }
-    else atomic_word<OP>(p, x);
-}
 NQ_DEV void atomic_word_dyn(int op, u64* p, u64 x) {
     switch (op) {
         case OP_ADD_U64: atomic_word<OP_ADD_U64>(p, x); break;
@@ -408,34 +395,10 @@ NQ_DEV int cache_claim_n(u64* ckeys, u32 slots, u32 hash, u64 key) {
     return -1;
 }
 
-// The same for packed keys of <= 31 bits: u32 keys in 16-byte buckets of four.  One 128-bit shared-memory load
-// fetches the whole bucket, so a lookup costs one instruction and one latency where the linear probe above pays up to
-// four dependent 64-bit loads - once the cache is full, every row of a key that is not cached walked all four.
-// Slots only ever change from empty to a key and every thread tries the slots of a bucket in the same order, so a key
-// settles in exactly one slot (and the block-end flush is additive, so even a duplicate would be harmless).
-NQ_DEV int cache_claim_b4(u32* ckeys, u32 nbuckets, u32 hash, u32 key) {
-    const u32 b = __umulhi(hash, nbuckets) * 4u;
-    u32 k[4];
-    asm volatile("ld.volatile.shared.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(k[0]), "=r"(k[1]), "=r"(k[2]), "=r"(k[3]) : "r"((u32)__cvta_generic_to_shared(ckeys + b)) : "memory");
-    int s = -1;  // select chain, not branches: the lanes of a warp match in different slots
-    s = k[3] == key ? (int)b + 3 : s;
-    s = k[2] == key ? (int)b + 2 : s;
-    s = k[1] == key ? (int)b + 1 : s;
-    s = k[0] == key ? (int)b : s;
-    if (s >= 0 || k[3] != 0xffffffffu) return s;  // found, or full (slots fill in order: the last one taken = full)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        if (k[i] != 0xffffffffu) continue;
-        const u32 old = atomicCAS(&ckeys[b + i], 0xffffffffu, key);
-        if (old == 0xffffffffu || old == key) return (int)b + i;
-    }
-    return -1;
-}
-
-// Direct-mapped variant: one slot per key, one 32-bit load.  Measured on config 5 (tools/proto5.cu, 1 B rows): the bucket
-// probe above costs a 16-byte load per lane (4 shared-memory wavefronts at best) and a 4-way select chain for every row;
-// the single probe misses a few more keys and is still 6 % faster overall.
+// The same for packed keys of <= 31 bits: u32 keys, direct-mapped - one slot per key, one 32-bit load.  Buckets of four
+// keys (one 16-byte load per lane, 4 shared-memory wavefronts at best, and a 4-way select chain for every row) miss fewer
+// keys and were still slower: 6 % in tools/proto5.cu, 5.19 against 4.95 ms per 1 B config-5 rows in the generated kernel
+// (profiles/r02_config5_ablation.jsonl).
 NQ_DEV int cache_claim_1(u32* ckeys, u32 nslots, u32 hash, u32 key) {
     const u32 b = __umulhi(hash, nslots);
     const u32 k = *(volatile u32*)&ckeys[b];
@@ -468,20 +431,12 @@ NQ_DEV void cache_add_carry(u32* lo, u64 x, u64* table_word) {
     const u32 h = (u32)(x >> 32) + ((u32)(old + xl) < xl ? 1u : 0u);
     if (h) atomicAdd(table_word, (u64)h << 32);
 }
-// per-thread register accumulators of the register groups (see codegen.cpp): ranged min / max keep the cache cells' image
-template <int OP> NQ_DEV void reg_mm32(u32& r, u64 x, u64 bias) {
-    const u32 v = (u32)(x - bias) + 1u;
-    if (OP == OP_MIN_I64 || OP == OP_MIN_U64) r = v < r ? v : r; else r = v > r ? v : r;
-}
 // (read first: a shared-memory load costs about half an atomic, and a group's min / max settle after a few rows; a
-// stale read can only cause an atomic that was not needed)
+// stale read can only cause an atomic that was not needed.  Round 1's unconditional atomic was slower: 1 520 against
+// 1 497 us per 200 M config-5 rows, profiles/r01_config5_sweep.jsonl)
 template <int OP> NQ_DEV void cache_mm32(u32* c, u64 x, u64 bias) {
     const u32 v = (u32)(x - bias) + 1u;
-#ifdef NQ_NO_CELL_CHECK
-    const u32 cur = (OP == OP_MIN_I64 || OP == OP_MIN_U64) ? 0xffffffffu : 0u;
-#else
     const u32 cur = *(volatile u32*)c;
-#endif
     if (OP == OP_MIN_I64 || OP == OP_MIN_U64) { if (v < cur) atomicMin(c, v); } else { if (v > cur) atomicMax(c, v); }
 }
 // the same with the cell's current value already in a register (two interleaved cells fetched by one 64-bit load)

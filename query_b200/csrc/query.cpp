@@ -107,7 +107,7 @@ std::unique_ptr<Query> Query::compile(Table* t, const std::string& alias, const 
     for (int w = 0; w < q->ops.n; ++w) q->ops.op[w] = q->kp.phys_ops[w];
     if (have_device()) {
         q->kernel = jit_load(q->kp.source, q->kp.dyn_smem, q->kp.block);
-        if (q->kp.part) q->part_kernel = jit_load(q->kp.part_source, q->kp.part_smem, q->kp.part_block);
+        if (q->kp.part) q->part_kernel = jit_load(q->kp.part_source, q->kp.part_smem, PART_THREADS);
         CK(cudaStreamCreateWithFlags(&q->own_stream, cudaStreamNonBlocking));
         q->stream = q->own_stream;
         CK(cudaEventCreate(&q->ev0));
@@ -294,9 +294,9 @@ void Query::launch_scan() {
         p.set_keys = (u64*)recs;
         p.keys = (u64*)cur;
         p.set_mask = part_cap;
-        const i64 tile = (i64)kp.part_block * 4;
+        const i64 tile = (i64)PART_THREADS * 4;
         const i64 tiles = (table->nrows + tile - 1) / tile;
-        const int pgrid = (int)std::max<i64>(1, std::min<i64>((tiles + 7) / 8, (i64)device_sm_count() * (1024 / kp.part_block)));
+        const int pgrid = (int)std::max<i64>(1, std::min<i64>((tiles + 7) / 8, (i64)device_sm_count()));
         jit_launch(*part_kernel, pgrid, stream, &p, sizeof p, false);
         PartPeers P;
         memset(&P, 0, sizeof P);

@@ -170,13 +170,13 @@ _GROUPED = [x for x in QUERIES if x[2]]
 
 @pytest.mark.parametrize("knob", ["N1GPU_NO_DIRECT", "N1GPU_NO_BITMAP", "N1GPU_NO_OFFSET_PACK", "N1GPU_NO_CACHE", "N1GPU_NO_PACK",
                                   "N1GPU_NO_KEY32", "N1GPU_NO_COMPLEMENT", "N1GPU_CACHE_BLOCK=1024", "N1GPU_CACHE_BLOCK=256",
-                                  "N1GPU_MMCHECK=1", "N1GPU_MMCHECK=2", "N1GPU_SET_PASSES=4", "N1GPU_NO_FCARRY", "N1GPU_NO_TIGHT", "N1GPU_PART",
-                                  "N1GPU_CACHE_WAYS=4", "N1GPU_NO_WIDE1", "N1GPU_NO_SIGN_FROM_MINMAX", "N1GPU_REG_GROUPS",
+                                  "N1GPU_SET_PASSES=4", "N1GPU_NO_FCARRY", "N1GPU_NO_TIGHT", "N1GPU_PART",
+                                  "N1GPU_NO_WIDE1", "N1GPU_NO_SIGN_FROM_MINMAX",
                                   "N1GPU_PRIV_BLOCK=640", "N1GPU_PRIV_BLOCK=96", "N1GPU_NO_MM_PAIR"])
 @pytest.mark.parametrize("name,where,keys,aggs", _GROUPED, ids=[x[0] for x in _GROUPED])
 def test_grouped_matrix_through_the_alternate_layouts(name, where, keys, aggs, knob, monkeypatch):
     """The planner picks direct-indexed tables, DISTINCT bitmaps, offset-packed keys, the shared-memory front cache
-    (u32 keys in buckets, one large or five small blocks per SM), packed table counters and complemented COUNT(x)
+    (direct-mapped u32 keys, one large or five small blocks per SM), packed table counters and complemented COUNT(x)
     counters whenever statistics allow; the layouts they replace (open addressing, hash sets, class-bits packing,
     uncached updates, 64-bit cache keys, one counter per word) stay reachable for wider keys / larger keyspaces and are
     kept under test by switching each choice off (or, for the tuning knobs, on)."""
@@ -186,13 +186,13 @@ def test_grouped_matrix_through_the_alternate_layouts(name, where, keys, aggs, k
     run_both(docs, "d", where, keys, aggs, "%s %s" % (name, knob))
 
 
-@pytest.mark.parametrize("block", ["256", "1024", "1024-reg", "1024-wide", "1024-4way"])
+@pytest.mark.parametrize("block", ["256", "1024", "1024-wide"])
 def test_skewed_string_keys_with_missing_and_null(block, monkeypatch):
     """BASELINE config 5 shape at oracle size: Zipf-skewed string keys, MISSING / NULL keys and values, more groups than
     the front cache holds (misses take the table path), both block shapes; bit-exact against the oracle."""
     block, _, variant = block.partition("-")
-    for knob in {"reg": ["N1GPU_REG_GROUPS"], "wide": ["N1GPU_NO_WIDE1", "N1GPU_NO_SIGN_FROM_MINMAX"], "4way": ["N1GPU_CACHE_WAYS"]}.get(variant, []):
-        monkeypatch.setenv(knob, "4" if knob.endswith("WAYS") else "1")
+    for knob in {"wide": ["N1GPU_NO_WIDE1", "N1GPU_NO_SIGN_FROM_MINMAX"]}.get(variant, []):
+        monkeypatch.setenv(knob, "1")
     monkeypatch.setenv("N1GPU_CACHE_BLOCK", block)
     monkeypatch.setenv("N1GPU_CACHE_KB", "2")  # a 2 KiB cache: most of the 3 000 keys miss
     docs = config5_docs(20000, 3000, 11)

@@ -325,14 +325,12 @@ LAYOUTS = {
     "direct-cache256": (["gd"], {"N1GPU_CACHE_BLOCK": "256"}, "hbm-direct", ["cache_claim_1("], []),
     "direct-cache1024": (["gd"], {"N1GPU_CACHE_BLOCK": "1024"}, "hbm-direct", ["cache_claim_1("], []),
     "direct-nocache": (["gd"], {"N1GPU_NO_CACHE": "1"}, "hbm-direct", [], ["cache_claim"]),
-    "direct-reg": (["gd"], {"N1GPU_REG_GROUPS": "1"}, "hbm-direct", ["rg0_", "rg1_"], []),
     "direct-nopair": (["gd"], {"N1GPU_NO_MM_PAIR": "1"}, "hbm-direct", [], ["mmp"]),
-    "direct-nocheck": (["gd"], {"N1GPU_NO_CELL_CHECK": "1"}, "hbm-direct", ["NQ_NO_CELL_CHECK"], []),
     "direct-nosign": (["gd"], {"N1GPU_NO_SIGN_FROM_MINMAX": "1"}, "hbm-direct", [], []),
     "hash64": (["gd"], {"N1GPU_NO_DIRECT": "1"}, "hbm-hash-64", [], []),
     "hash128": (["gw1", "gw2"], {}, "hbm-hash-128", [], []),
 }
-MM_LAYOUTS = ["ungrouped", "dense-priv", "direct-cache1024", "direct-reg", "direct-nopair", "direct-nocheck", "hash64"]
+MM_LAYOUTS = ["ungrouped", "dense-priv", "direct-cache1024", "direct-nopair", "hash64"]
 
 
 def _query(table, keys, aggs, env, monkeypatch, params=None, where=None):
@@ -345,9 +343,9 @@ def _query(table, keys, aggs, env, monkeypatch, params=None, where=None):
 
 
 def _layout_aggs(fx, layout):
-    """Thread-private tables hold at most 48 words and register groups at most 16: with FLOAT addends MIN / MAX need
-    class words, so those two layouts leave them out."""
-    return ["count(*)", "sum(%s)" % X, "avg(%s)" % X] if layout in ("dense-priv", "direct-reg") and T_FLOAT in fx.tags else AGGS
+    """Thread-private tables hold at most 48 words: with FLOAT addends MIN / MAX need class words, so that layout leaves
+    them out."""
+    return ["count(*)", "sum(%s)" % X, "avg(%s)" % X] if layout == "dense-priv" and T_FLOAT in fx.tags else AGGS
 
 
 def _run_layout(fx, layout, monkeypatch):

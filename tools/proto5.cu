@@ -7,7 +7,8 @@
 //   (-DPROTO_MODE=1 / 2 builds the two experiment modes described at k_scan_q's g_match / g_pack)
 //
 // Variants
-//   base   the kernel codegen.cpp emits today for this query (tools/_build/k5.cu, SoA table, per-row phases)
+//   base   the kernel codegen.cpp emitted for this query when the harness was written (proto5_base.cuh: SoA table,
+//          per-row phases, u32 cache keys in buckets of four)
 //   q      register groups for the payload-free key classes (MISSING / NULL keys), a per-warp shared-memory queue
 //          that compacts the remaining rows into full 32-lane batches for the front cache, a second queue that
 //          compacts cache misses, slot-major (one 32-byte sector per group) HBM table updated by lane pairs
