@@ -153,8 +153,11 @@ int n1gpu_query_compile(n1gpu_table* t, const char* alias, const char* where, co
 /* The same for a prepared statement: `$name` / `$1` in the expressions (algebra/param_named.go:63, param_positional.go;
  * Stringer text expression/stringer.go:611-620) take the values of the request (execution.Context.NamedArg /
  * PositionalArg, execution/context.go): param_names[i] ("name", "$name", "1") is bound to the JSON scalar text
- * param_values[i] ("10", "2.5", "\"abc\"", "true", "null").  A parameter without a value fails like the reference's
- * Evaluate ("No value for named parameter $x.").  Constants and parameter values reach the kernel as ARGUMENTS - the
+ * param_values[i] ("10", "2.5", "\"abc\"", "true", "null"), or to a JSON array of such scalars ("[1, 2.5, \"a\", null]").
+ * An array is legal only as the right operand of IN / NOT IN (`x IN $ids`); anywhere else, nested in an array, or an
+ * object, it is N1GPU_E_INELIGIBLE.  The list is probed as a device-resident set whose contents are kernel data, so
+ * every binding of the statement, whatever its length, shares one compiled kernel.  A parameter without a value fails
+ * like the reference's Evaluate ("No value for named parameter $x.").  Constants and parameter values reach the kernel as ARGUMENTS - the
  * generated source only fixes their class - so every binding of a statement, and statements that differ in a bound,
  * share one compiled kernel (n1gpu_jit_stats counts compilations and reuses).                                       */
 int n1gpu_query_compile_params(n1gpu_table* t, const char* alias, const char* where, const char* const* group_keys,

@@ -382,7 +382,8 @@ class Query:
     """A compiled Filter + InitialGroup/IntermediateGroup/FinalGroup chain (n1gpu_query)."""
 
     def __init__(self, table, alias, where, group_keys, aggregates, params=None):
-        """params: {name or position: python scalar} for the `$name` / `$1` parameters of a prepared statement"""
+        """params: {name or position: python scalar} for the `$name` / `$1` parameters of a prepared statement; a list of
+        scalars is accepted as the right operand of IN / NOT IN (`x IN $ids`) and is probed as a device-resident set"""
         self.table = table
         self.aggregates = list(aggregates)
         self.group_keys = list(group_keys)

@@ -318,7 +318,9 @@ int n1gpu_query_compile_params(n1gpu_table* t, const char* alias, const char* wh
         for (int i = 0; i < nparams; ++i) {
             REQUIRE(param_names && param_names[i] && param_values && param_values[i]);
             const char* n = param_names[i];
-            params.push_back(ParamValue{n[0] == '$' ? n + 1 : n, parse_param_value(param_values[i])});
+            ParamValue pv = parse_param_value(param_values[i]);
+            pv.name = n[0] == '$' ? n + 1 : n;
+            params.push_back(std::move(pv));
         }
         auto q = Query::compile(&t->t, alias, where, keys, aggs, params);
         *out = new n1gpu_query{std::move(q)};

@@ -19,6 +19,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
 #include <map>
 #include <set>
 
@@ -46,6 +47,69 @@ const char* cls_name(int c) {
     return n[c];
 }
 
+// the INSET_* flags of n1ql_device.cuh
+enum : u32 { INSET_MISSING = 1, INSET_NULL = 2, INSET_VALUED = 4, INSET_FALSE = 8, INSET_TRUE = 16, INSET_IEMPTY = 32, INSET_P63 = 64 };
+
+// open-addressing table of `keys` at load <= 0.25 (short clusters: a warp waits for its longest probe), probed like
+// inset_probe (n1ql_device.cuh)
+std::vector<u64> inset_table(std::vector<u64> keys) {
+    std::sort(keys.begin(), keys.end());
+    keys.erase(std::unique(keys.begin(), keys.end()), keys.end());
+    if (keys.empty()) return {};
+    u64 cap = 2;
+    while (cap < 4 * keys.size()) cap <<= 1;
+    if (cap > ((u64)1 << 31)) N1_THROW(N1GPU_E_INELIGIBLE, "IN list of %zu numbers", keys.size());
+    std::vector<u64> tab(cap, ~(u64)0);
+    for (u64 k : keys) {
+        u64 s = ((u32)((u32)k ^ (u32)(k >> 32)) * 0x9E3779B1u) >> (1 + __builtin_clz((u32)cap));  // inset_slot
+        while (tab[s] != ~(u64)0) s = (s + 1) & (cap - 1);
+        tab[s] = k;
+    }
+    return tab;
+}
+
+// the set of `x IN [constants]`; string elements are looked up in the dictionary of the operand column `dict_col`
+InSet build_inset(const Table& t, const Expr& list, int dict_col) {
+    InSet s;
+    std::vector<u64> ik, fk;
+    if (dict_col >= 0) s.bits.assign((t.cols[dict_col].dict.size() + 31) / 32 + 1, 0u);
+    for (auto& el : list.ops) {
+        const HValue& v = el->cval;
+        s.flags |= v.cls == C_MISSING ? INSET_MISSING : INSET_VALUED;
+        switch (v.cls) {
+            case C_NULL: s.flags |= INSET_NULL; break;
+            case C_FALSE: s.flags |= INSET_FALSE; break;
+            case C_TRUE: s.flags |= INSET_TRUE; break;
+            case C_INT: {
+                if ((u64)v.bits == ~(u64)0) s.flags |= INSET_IEMPTY; else ik.push_back((u64)v.bits);
+                const double d = (double)v.bits;  // float64 image for FLOAT rows (v_eq: float64(a) == float64(b))
+                u64 b;
+                memcpy(&b, &d, 8);
+                fk.push_back(d == 0.0 ? 0 : b);
+                break;
+            }
+            case C_FLOAT: {
+                const double d = v.f();
+                if (d != d) break;  // NaN equals nothing
+                if (d == 9223372036854775808.0) s.flags |= INSET_P63;
+                fk.push_back(d == 0.0 ? 0 : (u64)v.bits);
+                break;
+            }
+            case C_STRING: {
+                if (dict_col < 0) break;  // the operand is never a string
+                const auto& d = t.cols[dict_col].dict;
+                auto it = std::lower_bound(d.begin(), d.end(), v.s);
+                if (it != d.end() && *it == v.s) { const size_t r = (size_t)(it - d.begin()); s.bits[r >> 5] |= 1u << (r & 31); }
+                break;
+            }
+            default: break;
+        }
+    }
+    s.ikeys = inset_table(ik);
+    s.fkeys = inset_table(fk);
+    return s;
+}
+
 struct Gen {
     const Table& t;
     std::string body;
@@ -54,6 +118,8 @@ struct Gen {
     std::string ind = "                ";
     std::map<int, std::string> colvar;  // per-row cache of column Val variables
     std::vector<i64> consts;            // payloads handed to the kernel as p.cst[k] (at most 32; more stay literals)
+    std::vector<InSet> in_sets;         // handed to the kernel as p.inset[k]
+    std::map<const Expr*, int> in_set_of;  // an IN emitted twice (operand of two aggregates) uses one set
     bool const_args = true;
     explicit Gen(const Table& tt) : t(tt) { const_args = !env_flag("N1GPU_CONST_LITERALS"); }
     // the payload of a constant as an expression: a kernel argument slot of its own (numbered by occurrence, never by
@@ -179,6 +245,23 @@ struct Gen {
                 return r;
             }
             case EK::IN: {
+                const Expr& list = *e.ops[1];
+                const bool str_opnd = e.ops[0]->ti.mask & bit(C_STRING);
+                if (in_takes_set(e)) {
+                    if (str_opnd && !e.ops[0]->ti.plain_col) N1_THROW(N1GPU_E_INELIGIBLE, "IN over an array parameter with a constant string operand");
+                    std::string x = emit(*e.ops[0], nullptr), r = nv();
+                    auto it = in_set_of.find(&e);
+                    int k;
+                    if (it != in_set_of.end()) k = it->second;
+                    else {
+                        if ((int)in_sets.size() >= MAX_IN_SETS) N1_THROW(N1GPU_E_INELIGIBLE, "more than %d IN sets in one chain", MAX_IN_SETS);
+                        k = (int)in_sets.size();
+                        in_sets.push_back(build_inset(t, list, str_opnd ? e.ops[0]->ti.dict_col : -1));
+                        in_set_of[&e] = k;
+                    }
+                    line(strf("const Val %s = in_set(%s, p.inset[%d]);", r.c_str(), x.c_str(), k));
+                    return r;
+                }
                 StrCtx c2 = make_ctx(e);
                 std::string x = emit(*e.ops[0], &c2);
                 std::string h = nv("h"), m = nv("m"), n = nv("n"), r = nv();
@@ -1230,6 +1313,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     s += "}\n";
     kp.source = s;
     kp.consts = g.consts;
+    kp.in_sets = std::move(g.in_sets);
     if (kp.part) {
         std::string q;
         q += "// generated by libn1gpu codegen: the partitioning kernel of this chain's partitioned DISTINCT aggregation\n";

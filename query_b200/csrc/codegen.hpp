@@ -33,6 +33,15 @@ struct PackComp {
     int bits() const { return cbits + pbits; }
 };
 
+// IN evaluated through a device-resident set (NqInSet, n1ql_device.cuh) instead of one in_arg per element: see
+// in_takes_set (expr.hpp).  The kernel text names only the set's slot, so every binding of a statement shares one cubin.
+constexpr int MAX_IN_SETS = 8;  // NQ_MAX_INSETS
+struct InSet {
+    std::vector<u32> bits;         // STRING: bitmap over the operand column's dictionary ranks
+    std::vector<u64> ikeys, fkeys; // INT / FLOAT hash tables (all ones = empty slot)
+    u32 flags = 0;                 // INSET_* of n1ql_device.cuh
+};
+
 struct AggPlan {
     AggKind kind = AggKind::COUNT;
     bool distinct = false, star = false;
@@ -115,6 +124,7 @@ struct KernelPlan {
     int part_smem = 0;           // dynamic shared memory of the partitioning kernel
     // payloads of constants / bound parameters, passed to the kernel as NqParams::cst (the source only names the slot)
     std::vector<i64> consts;
+    std::vector<InSet> in_sets;  // NqParams::inset[k]
     std::vector<int> used_cols;
     int scan_bytes_per_row = 0;
     std::string source;

@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <charconv>
+#include <cstring>
 
 #include "json.hpp"
 #include "table.hpp"
@@ -57,6 +58,7 @@ std::string Expr::str() const {
         case EK::IS_VALUED: return "(" + ops[0]->str() + " is valued)";
         case EK::IS_NOT_VALUED: return "(" + ops[0]->str() + " is not valued)";
         case EK::ARRAY: {
+            if (!param.empty()) return "$" + param;
             std::string s = "[";
             for (size_t i = 0; i < ops.size(); ++i) { if (i) s += ", "; s += ops[i]->str(); }
             return s + "]";
@@ -333,19 +335,22 @@ static u32 nonnum_bits(u32 m) { return m & (bit(C_NULL) | M_BOOL | bit(C_STRING)
 
 void bind_params(Expr& e, const std::vector<ParamValue>& params) {
     if (e.kind == EK::PARAM) {
-        for (auto& pv : params)
-            if (pv.name == e.name) { e.kind = EK::CONST; e.cval = pv.value; e.param = e.name; return; }
+        for (auto& pv : params) {
+            if (pv.name != e.name) continue;
+            e.param = e.name;
+            if (!pv.is_array) { e.kind = EK::CONST; e.cval = pv.value; return; }
+            e.kind = EK::ARRAY;
+            for (auto& v : pv.elems) { ExprP c(new Expr(EK::CONST)); c->cval = v; e.ops.push_back(std::move(c)); }
+            return;
+        }
         N1_THROW(N1GPU_E_INVALID, "No value for %s parameter $%s.", isdigit((unsigned char)e.name[0]) ? "positional" : "named", e.name.c_str());
     }
     for (auto& o : e.ops) bind_params(*o, params);
 }
 
-HValue parse_param_value(const std::string& text) {
-    json::Scanner sc(text.data(), text.data() + text.size());
-    sc.ws();
-    if (sc.p >= sc.end) N1_THROW(N1GPU_E_INVALID, "empty parameter value");
+static HValue scalar_param(json::Scanner& sc, const std::string& text) {
     HValue v;
-    const char c = *sc.p;
+    const char c = sc.p < sc.end ? *sc.p : '\0';
     if (c == '"') {
         const char *rb, *re; bool esc;
         if (!sc.string_raw(rb, re, esc)) N1_THROW(N1GPU_E_PARSE, "bad string parameter value");
@@ -354,17 +359,48 @@ HValue parse_param_value(const std::string& text) {
     } else if (c == '-' || isdigit((unsigned char)c)) {
         bool ii; i64 iv; double dv;
         if (!sc.number(ii, iv, dv)) N1_THROW(N1GPU_E_PARSE, "bad number parameter value");
-        v = ii ? HValue::integer(iv) : new_num(dv);
+        v = ii ? HValue::integer(iv) : new_num(dv);  // value.NewValue canonicalisation, as for literals
     } else {
-        const std::string w(sc.p, sc.end);
-        if (w.compare(0, 4, "true") == 0) { v = HValue::boolean(true); sc.p += 4; }
-        else if (w.compare(0, 5, "false") == 0) { v = HValue::boolean(false); sc.p += 5; }
-        else if (w.compare(0, 4, "null") == 0) { v = HValue::null(); sc.p += 4; }
-        else N1_THROW(N1GPU_E_INELIGIBLE, "parameter value %s is not a scalar (arrays / objects stay on the Go operators)", text.c_str());
+        auto word = [&](const char* w, size_t n) { return (size_t)(sc.end - sc.p) >= n && memcmp(sc.p, w, n) == 0; };
+        if (word("true", 4)) { v = HValue::boolean(true); sc.p += 4; }
+        else if (word("false", 5)) { v = HValue::boolean(false); sc.p += 5; }
+        else if (word("null", 4)) { v = HValue::null(); sc.p += 4; }
+        else N1_THROW(N1GPU_E_INELIGIBLE, "parameter value %s is not a scalar or an array of scalars (nested arrays / objects stay on the Go operators)", text.c_str());
     }
+    return v;
+}
+
+ParamValue parse_param_value(const std::string& text) {
+    json::Scanner sc(text.data(), text.data() + text.size());
+    sc.ws();
+    if (sc.p >= sc.end) N1_THROW(N1GPU_E_INVALID, "empty parameter value");
+    ParamValue pv;
+    if (*sc.p == '[') {
+        pv.is_array = true;
+        ++sc.p;
+        sc.ws();
+        if (sc.p < sc.end && *sc.p == ']') ++sc.p;
+        else for (;;) {
+            sc.ws();
+            pv.elems.push_back(scalar_param(sc, text));
+            sc.ws();
+            if (sc.p < sc.end && *sc.p == ',') { ++sc.p; continue; }
+            if (sc.p < sc.end && *sc.p == ']') { ++sc.p; break; }
+            N1_THROW(N1GPU_E_PARSE, "bad array parameter value %s", text.c_str());
+        }
+    } else pv.value = scalar_param(sc, text);
     sc.ws();
     if (sc.p != sc.end) N1_THROW(N1GPU_E_PARSE, "trailing characters in parameter value %s", text.c_str());
-    return v;
+    return pv;
+}
+
+bool in_takes_set(const Expr& in) {
+    const Expr& list = *in.ops[1];
+    if (!list.param.empty()) return true;  // array parameter: an operand that is a string constant is refused in codegen
+    if (list.ops.size() <= IN_CHAIN_MAX) return false;
+    for (auto& el : list.ops) if (el->kind != EK::CONST) return false;
+    const TypeInfo& x = in.ops[0]->ti;
+    return !(x.mask & bit(C_STRING)) || x.plain_col;
 }
 
 void bind_and_analyze(Expr& e, const std::string& alias, const Table& t) {
@@ -387,7 +423,11 @@ void bind_and_analyze(Expr& e, const std::string& alias, const Table& t) {
     }
     if (e.kind == EK::IDENT) N1_THROW(N1GPU_E_INELIGIBLE, "bare identifier %s", e.str().c_str());
     if (e.kind == EK::PARAM) N1_THROW(N1GPU_E_INVALID, "No value for parameter $%s.", e.name.c_str());
-    for (auto& o : e.ops) bind_and_analyze(*o, alias, t);
+    for (size_t i = 0; i < e.ops.size(); ++i) {
+        if (e.ops[i]->kind == EK::ARRAY && !(e.kind == EK::IN && i == 1))
+            N1_THROW(N1GPU_E_INELIGIBLE, "array value outside the right operand of IN: %s", e.ops[i]->str().c_str());
+        bind_and_analyze(*e.ops[i], alias, t);
+    }
     auto any_has = [&](u32 bits) { for (auto& o : e.ops) if (o->ti.mask & bits) return true; return false; };
     auto string_dict = [&]() {  // the one dictionary string operands of a comparison live in
         int d = -1;
@@ -497,10 +537,12 @@ void bind_and_analyze(Expr& e, const std::string& alias, const Table& t) {
             break;
         }
         case EK::IN: {
-            if (e.ops[1]->kind != EK::ARRAY) N1_THROW(N1GPU_E_INELIGIBLE, "IN over a non-literal array: %s", e.str().c_str());
+            if (e.ops[1]->kind != EK::ARRAY) N1_THROW(N1GPU_E_INELIGIBLE, "IN over a non-array: %s", e.str().c_str());
             u32 m = M_BOOL;
             u32 all = e.ops[0]->ti.mask;
-            for (auto& el : e.ops[1]->ops) all |= el->ti.mask;
+            // a set: NULL whatever the elements (a NULL row, or a NULL element), MISSING when a literal list may hold one
+            if (in_takes_set(e)) all |= bit(C_NULL) | (e.ops[1]->param.empty() ? bit(C_MISSING) : 0);
+            else for (auto& el : e.ops[1]->ops) all |= el->ti.mask;
             if (all & bit(C_MISSING)) m |= bit(C_MISSING);
             if (all & bit(C_NULL)) m |= bit(C_NULL);
             ti.mask = m;

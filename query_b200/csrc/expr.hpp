@@ -42,7 +42,7 @@ struct Expr {
     std::vector<std::unique_ptr<Expr>> ops;
     HValue cval;             // CONST
     std::string name;        // IDENT / FIELD name; PARAM: the name or position after '$'
-    std::string param;       // CONST that stands for a bound parameter: its name (the Stringer text stays "$name")
+    std::string param;       // CONST / ARRAY that stands for a bound parameter: its name (the Stringer text stays "$name")
     AggKind agg = AggKind::COUNT;
     bool distinct = false;
     bool star = false;       // count(*)
@@ -65,10 +65,24 @@ void collect_paths(const Expr& e, const std::string& alias, std::vector<std::str
 
 // Replaces every PARAM by the constant bound to it (execution.Context.NamedArg / PositionalArg); a parameter without a
 // value throws N1GPU_E_INVALID ("No value for named parameter $x", algebra/param_named.go:70-72).
-struct ParamValue { std::string name; HValue value; };
+// An array value binds to an ARRAY of constants, which is legal only as the right operand of IN (bind_and_analyze).
+struct ParamValue {
+    std::string name;
+    HValue value;
+    bool is_array = false;
+    std::vector<HValue> elems;  // is_array: the elements
+};
 void bind_params(Expr& e, const std::vector<ParamValue>& params);
-// a JSON scalar (number, string, true, false, null) as a constant; arrays / objects are outside the subset
-HValue parse_param_value(const std::string& json_text);
+// a JSON scalar (number, string, true, false, null) as a constant, or a JSON array of such scalars; nested arrays and
+// objects are outside the subset.  The name is left empty.
+ParamValue parse_param_value(const std::string& json_text);
+
+// `x IN list` is probed as a device-resident set, not unrolled into one in_arg per element, when the list is bound to an
+// array parameter (whatever its length) or is a literal list of more than IN_CHAIN_MAX constants (DESIGN.md section 3.1);
+// a string-capable operand must then be a dictionary column.  Needs the operand analysed.  For such an IN the analysis
+// keeps the result's classes independent of the elements, so that the kernel text does not depend on them either.
+constexpr size_t IN_CHAIN_MAX = 16;
+bool in_takes_set(const Expr& in);
 
 // Binds FIELD chains to columns of `t` and computes TypeInfo bottom-up.
 void bind_and_analyze(Expr& e, const std::string& alias, const Table& t);

@@ -467,6 +467,60 @@ NQ_DEV void pack_bits(u64& lo, u64& hi, int& pos, u64 v, int nbits) {
     pos += nbits;
 }
 
+// ---- IN over a device-resident set ------------------------------------------------------------------
+// The fold of in_arg / in_fin over a list of constants, restated over a set built on the host (codegen.cpp, build_inset):
+//   STRING  bitmap over the operand column's dictionary ranks (an element absent from the dictionary sets no bit)
+//   INT     open-addressing table of the INT elements (linear probing, load <= 0.25)
+//   FLOAT   the same over the float64 images of the FLOAT elements and of the INT elements (v_eq compares any pair that is
+//           not INT / INT as float64); -0.0 is stored and probed as +0.0, NaN never matches
+// An INT row equals a FLOAT element only through rounding: integral floats below 2^63 in magnitude are INTs after
+// canonicalisation, so 2^63 is the only FLOAT element an INT row can hit (INSET_P63).  NQ_U64_MAX marks an empty slot;
+// an INT element of that value is the flag INSET_IEMPTY (a float key never has those bits: they are a NaN).
+#define NQ_MAX_INSETS 8
+#define INSET_MISSING 1u   // some element is MISSING
+#define INSET_NULL 2u      // some element is NULL
+#define INSET_VALUED 4u    // some element is not MISSING
+#define INSET_FALSE 8u
+#define INSET_TRUE 16u
+#define INSET_IEMPTY 32u   // the INT element -1 (the empty-slot marker)
+#define INSET_P63 64u      // the FLOAT element 2^63
+struct NqInSet {
+    const u32* bits;  // STRING: bit r <=> dictionary rank r is an element
+    const u64* keys;  // INT table [icap], then FLOAT table [fcap]
+    u32 icap, fcap;   // powers of two, 0: no table
+    u32 flags;
+    u32 pad;
+};
+// home slot: Fibonacci hashing of the key folded to 32 bits (one 32-bit multiply; mix64 costs two 64-bit ones per row)
+NQ_DEV u32 inset_slot(u64 key, u32 cap) { return (((u32)key ^ (u32)(key >> 32)) * 0x9E3779B1u) >> (1 + __clz(cap)); }
+NQ_DEV bool inset_probe(const u64* __restrict__ keys, u32 cap, u64 key) {
+    if (cap == 0) return false;
+    u32 slot = inset_slot(key, cap);
+    for (;;) {
+        const u64 cur = __ldg(&keys[slot]);
+        if (cur == key) return true;
+        if (cur == NQ_U64_MAX) return false;
+        slot = (slot + 1) & (cap - 1);
+    }
+}
+NQ_DEV Val in_set(Val x, const NqInSet& d) {
+    if (x.c == C_MISSING) return x;
+    bool hit = false;
+    if (x.c == C_INT) {
+        hit = (u64)x.b == NQ_U64_MAX ? (d.flags & INSET_IEMPTY) != 0 : inset_probe(d.keys, d.icap, (u64)x.b);
+        if (!hit && (d.flags & INSET_P63)) hit = (double)x.b == 9223372036854775808.0;
+    } else if (x.c == C_FLOAT) {
+        const double f = as_f(x.b);
+        if (f == f) hit = inset_probe(d.keys + d.icap, d.fcap, f == 0.0 ? 0ULL : (u64)x.b);
+    } else if (x.c == C_STRING) {
+        const u64 r = (u64)x.b >> 1;
+        hit = (__ldg(&d.bits[r >> 5]) >> (r & 31)) & 1u;
+    } else if (x.c == C_FALSE) hit = d.flags & INSET_FALSE;
+    else if (x.c == C_TRUE) hit = d.flags & INSET_TRUE;
+    else return (d.flags & INSET_VALUED) ? mkv(C_NULL, 0) : ((d.flags & INSET_MISSING) ? mkv(C_MISSING, 0) : mkbool(false));  // NULL row
+    return hit ? mkbool(true) : ((d.flags & INSET_NULL) ? mkv(C_NULL, 0) : ((d.flags & INSET_MISSING) ? mkv(C_MISSING, 0) : mkbool(false)));
+}
+
 // kernel parameter block shared by every generated scan kernel
 struct NqParams {
     i64 nrows;             // rows in this partition
@@ -500,6 +554,8 @@ struct NqParams {
     // execution.Operator.SendStop while the scan runs: a word in HBM that n1gpu_query_cancel sets with an asynchronous copy;
     // lane 0 of every warp polls it once per 32 tiles and the warp leaves the loop
     const int* cancel;
+    // `x IN $list` and IN over long literal lists: the list's contents as kernel data (NqInSet), never kernel text
+    NqInSet inset[NQ_MAX_INSETS];
 };
 NQ_DEV bool nq_cancelled(const NqParams& p, int lane) {
     int c = 0;

@@ -12,6 +12,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <thread>
 #include <unordered_map>
 
@@ -42,8 +43,11 @@ struct NqParamsHost {
     int set_pass, set_shift;
     i64 cst[32];
     const int* cancel;
+    InSetDesc inset[MAX_IN_SETS];
 };
-static_assert(sizeof(NqParamsHost) == 8 + 128 + 128 + 8 * 17 + 256 + 8, "NqParams layout");
+static_assert(sizeof(InSetDesc) == 32, "NqInSet layout");
+static_assert(offsetof(NqParamsHost, cancel) == 8 + 128 + 128 + 8 * 17 + 256, "NqParams layout");
+static_assert(sizeof(NqParamsHost) == 8 + 128 + 128 + 8 * 17 + 256 + 8 + 32 * MAX_IN_SETS, "NqParams layout");
 
 u64 pow2_at_least(u64 n) { u64 p = 1; while (p < n) p <<= 1; return p; }
 
@@ -113,6 +117,7 @@ std::unique_ptr<Query> Query::compile(Table* t, const std::string& alias, const 
         CK(cudaEventCreate(&q->ev0));
         CK(cudaEventCreate(&q->ev1));
         q->alloc_state();
+        q->upload_in_sets();
     } else {
         // no GPU in this process (build / CPU test container): still prove the kernel compiles for sm_100a
         std::string log;
@@ -120,6 +125,37 @@ std::unique_ptr<Query> Query::compile(Table* t, const std::string& alias, const 
         if (q->kp.part) jit_compile_cubin(q->kp.part_source, &log);
     }
     return q;
+}
+
+// One device buffer holds every set of the chain: [bitmap | INT table | FLOAT table] per set, 8-byte aligned.
+void Query::upload_in_sets() {
+    const auto& S = kp.in_sets;
+    if (S.empty()) return;
+    std::vector<size_t> at;
+    size_t words = 0;  // u64 words
+    for (auto& s : S) { at.push_back(words); words += (s.bits.size() + 1) / 2 + s.ikeys.size() + s.fkeys.size(); }
+    std::vector<u64> host(std::max<size_t>(words, 1), 0);
+    for (size_t k = 0; k < S.size(); ++k) {
+        u64* w = host.data() + at[k];
+        memcpy(w, S[k].bits.data(), S[k].bits.size() * 4);
+        w += (S[k].bits.size() + 1) / 2;
+        std::copy(S[k].ikeys.begin(), S[k].ikeys.end(), w);
+        std::copy(S[k].fkeys.begin(), S[k].fkeys.end(), w + S[k].ikeys.size());
+    }
+    d_in_sets.alloc(host.size() * 8);
+    CK(cudaMemcpyAsync(d_in_sets.p, host.data(), host.size() * 8, cudaMemcpyHostToDevice, stream));
+    CK(cudaStreamSynchronize(stream));  // a later scan may run on another stream (n1gpu_query_set_stream)
+    const u64* base = d_in_sets.as<u64>();
+    in_descs.clear();
+    for (size_t k = 0; k < S.size(); ++k) {
+        InSetDesc d{};
+        d.bits = S[k].bits.empty() ? nullptr : (const u32*)(base + at[k]);
+        d.keys = base + at[k] + (S[k].bits.size() + 1) / 2;
+        d.icap = (u32)S[k].ikeys.size();
+        d.fcap = (u32)S[k].fkeys.size();
+        d.flags = S[k].flags;
+        in_descs.push_back(d);
+    }
 }
 
 void Query::rebind(Table* t) {
@@ -246,6 +282,7 @@ void Query::launch_scan() {
     p.nrows = table->nrows;
     for (size_t c = 0; c < table->cols.size(); ++c) { p.col[c] = table->cols[c].d_payload.p; p.tag[c] = table->cols[c].d_tags.as<u8>(); }
     for (size_t k = 0; k < kp.consts.size() && k < 32; ++k) p.cst[k] = kp.consts[k];
+    for (size_t k = 0; k < in_descs.size(); ++k) p.inset[k] = in_descs[k];
     p.cancel = d_cancel.as<int>();
     p.acc = kp.mode == MODE_UNGROUPED ? d_accum.as<u64>() : acc();
     p.partials = d_partials.as<u64>();
