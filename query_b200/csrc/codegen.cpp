@@ -1010,17 +1010,17 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
             if (kp.cell_kind[w] == CK_MM32 && kp.cell_pair[w]) {
                 // interleaved with its neighbour: the hit phase has loaded both cells of the slot with one 64-bit load (mmpN)
                 const int first = kp.cell_pair[w] == 1 ? w : w - 1;
-                hit = strf("cache_mm32_cur<OP>(&s_c32[%s], (u64)(val_), %lluULL, (u32)(mmp%d%s))", cell32(kp, w, "cslot").c_str(), (unsigned long long)kp.word_lo[w],
+                hit = strf("cache_mm32_cur<OP>(a_c32 + 4 * (%s), (u64)(val_), %lluULL, (u32)(mmp%d%s))", cell32(kp, w, "cslot").c_str(), (unsigned long long)kp.word_lo[w],
                            first, kp.cell_pair[w] == 1 ? "" : " >> 32");
                 s += strf("#define ACCH_%d(OP, val_) %s\n", w, hit.c_str());
                 continue;
             }
             switch (kp.cell_kind[w]) {
-                case CK_CNT: hit = strf("atomicAdd(&s_c32[%d * NQ_CS + cslot], (u32)(val_))", ci); break;
+                case CK_CNT: hit = strf("reds_add(a_c32 + 4 * (%d * NQ_CS + cslot), (u32)(val_))", ci); break;
                 case CK_WIDE: hit = strf("cache_add_wide(&s_c32[%d * NQ_CS + cslot], &s_c32[%d * NQ_CS + cslot], (u64)(val_))", ci, ci + 1); break;
-                case CK_WIDE1: hit = strf("cache_add_carry(&s_c32[%d * NQ_CS + cslot], (u64)(val_), &p.acc[%dULL * cap + klo])", ci, kp.phys_of[w]); break;
-                case CK_MM32: hit = strf("cache_mm32<OP>(&s_c32[%d * NQ_CS + cslot], (u64)(val_), %lluULL)", ci, (unsigned long long)kp.word_lo[w]); break;
-                case CK_OR32: hit = strf("cache_or32(&s_c32[%d * NQ_CS + cslot], (u32)(val_))", ci); break;
+                case CK_WIDE1: hit = strf("cache_add_carry(a_c32 + 4 * (%d * NQ_CS + cslot), (u64)(val_), &p.acc[%dULL * cap + klo])", ci, kp.phys_of[w]); break;
+                case CK_MM32: hit = strf("cache_mm32<OP>(a_c32 + 4 * (%d * NQ_CS + cslot), (u64)(val_), %lluULL)", ci, (unsigned long long)kp.word_lo[w]); break;
+                case CK_OR32: hit = strf("cache_or32(a_c32 + 4 * (%d * NQ_CS + cslot), (u32)(val_))", ci); break;
                 default: hit = strf("cache_word64<OP>(&s_c64[%d * NQ_CS + cslot], (u64)(val_))", ci); break;
             }
             s += strf("#define ACCH_%d(OP, val_) %s\n", w, hit.c_str());
@@ -1075,6 +1075,8 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
                 s += strf("    u32* const s_c32 = (u32*)(s_dyn + %d * NQ_CS);  // [%d][NQ_CS] 32-bit cells\n", 1 + kp.cache_n64, kp.cache_n32);
             }
             s += "    (void)s_c64; (void)s_c32;\n";
+            // 32-bit shared addresses made once: the row loop's 32-bit cells and u32 keys are accessed through them
+            s += "    const u32 a_ckey = smem_addr(s_ckey), a_c32 = smem_addr(s_c32); (void)a_ckey; (void)a_c32;\n";
             s += "    for (int i = threadIdx.x; i < NQ_CS; i += NQ_BLOCK) {\n";
             s += kp.cache_key32 ? "        s_ckey[i] = 0xffffffffu;\n" : "        s_ckey[i] = NQ_U64_MAX;\n";
             for (int w = 0; w < W; ++w) {
@@ -1113,27 +1115,39 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         // insert into the HBM table and update it with L2 atomics.
         s += "        u64 kk[4]; int cs[4];  // group key / cache slot (-1: not cached, -2: row not selected)\n";
         s += "        __syncwarp();\n";
-        s += "#pragma unroll\n";
-        s += "        for (int j = 0; j < 4; ++j) {\n";
-        s += "            bool pass = base + j < nrows;\n";
-        s += g.decls;
+        // only the grid's last tile can hold rows at or beyond nrows: phase (1) is emitted twice, and full tiles run the
+        // copy without the per-row 64-bit bounds check
+        std::string p1;
+        p1 += "#pragma unroll\n";
+        p1 += "        for (int j = 0; j < 4; ++j) {\n";
+        p1 += "            bool pass = NQ_IN_RANGE(j);\n";
+        p1 += g.decls;
         if (where) {
-            s += filter_code;
-            s += "                pass = pass && w_true;\n";
+            p1 += filter_code;
+            p1 += "                pass = pass && w_true;\n";
         }
-        s += "            cs[j] = -2; kk[j] = 0;\n";
+        p1 += "            cs[j] = -2; kk[j] = 0;\n";
         // MISSING / NULL keys (one row in five of config 5, two slots) are cached like any other key.  Register
         // accumulators for them were removed: -16 % per 1 B config-5 rows (4.95 -> 5.72 ms, profiles/r02_config5_ablation.jsonl),
         // ~55 extra instructions per row on a kernel whose issue slots are already 68 % busy.
-        s += "            if (pass) {\n";
-        s += key_code;
-        s += "                    kk[j] = klo;\n";
-        s += "                    ++nlook;\n";
-        if (kp.cache_key32) s += "                    cs[j] = cache_on ? cache_claim_1(s_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, (u32)klo) : -1;\n";
-        else if (kp.key_bits <= 32) s += "                    cs[j] = cache_on ? cache_claim_n(s_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, klo) : -1;\n";
-        else s += "                    cs[j] = cache_on ? cache_claim_n(s_ckey, NQ_CS, (u32)(mix64(klo) >> 32), klo) : -1;\n";
-        s += "                    nhit += cs[j] >= 0;\n";
-        s += "            }\n";
+        p1 += "            if (pass) {\n";
+        p1 += key_code;
+        p1 += "                    kk[j] = klo;\n";
+        p1 += "                    ++nlook;\n";
+        if (kp.cache_key32) p1 += "                    cs[j] = cache_on ? cache_claim_1(a_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, (u32)klo) : -1;\n";
+        else if (kp.key_bits <= 32) p1 += "                    cs[j] = cache_on ? cache_claim_n(s_ckey, NQ_CS, (u32)klo * 0x9E3779B1u, klo) : -1;\n";
+        else p1 += "                    cs[j] = cache_on ? cache_claim_n(s_ckey, NQ_CS, (u32)(mix64(klo) >> 32), klo) : -1;\n";
+        p1 += "                    nhit += cs[j] >= 0;\n";
+        p1 += "            }\n";
+        p1 += "        }\n";
+        s += "        if (wbase + 128 <= nrows) {\n";
+        s += "#define NQ_IN_RANGE(j) true\n";
+        s += p1;
+        s += "#undef NQ_IN_RANGE\n";
+        s += "        } else {\n";
+        s += "#define NQ_IN_RANGE(j) (base + (j) < nrows)\n";
+        s += p1;
+        s += "#undef NQ_IN_RANGE\n";
         s += "        }\n";
         s += "#define ACC(k, OP, val_) if (nq_first) ACCH_##k(OP, val_)\n";
         s += "#pragma unroll\n";
@@ -1144,7 +1158,7 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
         s += "                    const int cslot = cs[j]; const u64 klo = kk[j]; (void)klo;\n";
         for (int w = 0; w < W; ++w)
             if (kp.cell_pair[w] == 1)
-                s += strf("                    const u64 mmp%d = *(volatile u64*)&s_c32[%d * NQ_CS + 2 * cslot];  // both cells of the slot: one LDS.64\n", w, kp.cell_idx[w]);
+                s += strf("                    const u64 mmp%d = *(volatile u64*)__cvta_shared_to_generic(a_c32 + 4 * (%d * NQ_CS + 2 * cslot));  // both cells of the slot: one LDS.64\n", w, kp.cell_idx[w]);
         s += g.decls;
         s += agg_code;
         s += "            }\n";

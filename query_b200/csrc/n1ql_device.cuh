@@ -377,6 +377,22 @@ NQ_DEV i64 table_find128(const ulonglong2* __restrict__ keys, u64 cap_mask, u64 
 }
 #endif
 
+// 32-bit shared-state-space addresses of the front cache.  Through a generic pointer the compiler rebuilds the block's
+// shared window (S2R SR_CgaCtaId + LEA) at every cache access of the row loop (config 5: 8 times per tile); the address
+// made once by smem_addr is opaque to it, so it stays in a register and every access is one LDS / ATOMS [reg + imm].
+NQ_DEV u32 smem_addr(const void* p) {
+    u32 a;
+    asm volatile("mov.b32 %0, %1;" : "=r"(a) : "r"((u32)__cvta_generic_to_shared(p)));
+    return a;
+}
+NQ_DEV u32 lds_u32(u32 a) { u32 v; asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
+NQ_DEV u32 atoms_add(u32 a, u32 x) { u32 o; asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(o) : "r"(a), "r"(x)); return o; }
+NQ_DEV void reds_add(u32 a, u32 x) { asm volatile("red.shared.add.u32 [%0], %1;" :: "r"(a), "r"(x)); }
+NQ_DEV void reds_min(u32 a, u32 x) { asm volatile("red.shared.min.u32 [%0], %1;" :: "r"(a), "r"(x)); }
+NQ_DEV void reds_max(u32 a, u32 x) { asm volatile("red.shared.max.u32 [%0], %1;" :: "r"(a), "r"(x)); }
+NQ_DEV void reds_or(u32 a, u32 x) { asm volatile("red.shared.or.b32 [%0], %1;" :: "r"(a), "r"(x)); }
+NQ_DEV u32 atoms_cas(u32 a, u32 c, u32 x) { u32 o; asm volatile("atom.shared.cas.b32 %0, [%1], %2, %3;" : "=r"(o) : "r"(a), "r"(c), "r"(x)); return o; }
+
 // Per-block shared-memory front cache of the HBM group table (hot keys of a skewed GROUP BY are aggregated with
 // shared-memory atomics and reach HBM once per block): claims or finds `key` within 4 probes, else -1 (miss).
 // (any slot count, not only powers of two: the slot is the high part of hash * slots)
@@ -399,14 +415,16 @@ NQ_DEV int cache_claim_n(u64* ckeys, u32 slots, u32 hash, u64 key) {
 // keys (one 16-byte load per lane, 4 shared-memory wavefronts at best, and a 4-way select chain for every row) miss fewer
 // keys and were still slower: 6 % in tools/proto5.cu, 5.19 against 4.95 ms per 1 B config-5 rows in the generated kernel
 // (profiles/r02_config5_ablation.jsonl).
-NQ_DEV int cache_claim_1(u32* ckeys, u32 nslots, u32 hash, u32 key) {
+// (ckeys: smem_addr of the key array)
+NQ_DEV int cache_claim_1(u32 ckeys, u32 nslots, u32 hash, u32 key) {
     const u32 b = __umulhi(hash, nslots);
-    const u32 k = *(volatile u32*)&ckeys[b];
+    const u32 k = lds_u32(ckeys + 4 * b);
     if (k == key) return (int)b;
     if (k != 0xffffffffu) return -1;
-    const u32 old = atomicCAS(&ckeys[b], 0xffffffffu, key);
+    const u32 old = atoms_cas(ckeys + 4 * b, 0xffffffffu, key);
     return (old == 0xffffffffu || old == key) ? (int)b : -1;
 }
+NQ_DEV int cache_claim_1(u32* ckeys, u32 nslots, u32 hash, u32 key) { return cache_claim_1(smem_addr(ckeys), nslots, hash, key); }
 
 // Cells of the front cache.  Shared memory has native 32-bit atomics only (a 64-bit atomicAdd/Min/Max on shared
 // memory compiles to a compare-and-swap loop, 3-9x slower and collapsing under same-key contention), so a cached
@@ -425,27 +443,26 @@ NQ_DEV void cache_add_wide(u32* lo, u32* hi, u64 x) {
 // One-cell integer sum (addends within +-2^31): the low word is cached, whatever the add carries or borrows goes straight
 // to the table word as a multiple of 2^32 (rare: once per 2^32 / |x| rows; a small negative addend wraps the cell and
 // cancels its own sign extension).  Cell and table word are both plain sums, so the flush just adds the cell.
-NQ_DEV void cache_add_carry(u32* lo, u64 x, u64* table_word) {
+// (the cells of these helpers are smem_addr addresses; the u32* forms convert)
+NQ_DEV void cache_add_carry(u32 lo, u64 x, u64* table_word) {
     const u32 xl = (u32)x;
-    const u32 old = atomicAdd(lo, xl);
+    const u32 old = atoms_add(lo, xl);
     const u32 h = (u32)(x >> 32) + ((u32)(old + xl) < xl ? 1u : 0u);
     if (h) atomicAdd(table_word, (u64)h << 32);
 }
+NQ_DEV void cache_add_carry(u32* lo, u64 x, u64* table_word) { cache_add_carry(smem_addr(lo), x, table_word); }
 // (read first: a shared-memory load costs about half an atomic, and a group's min / max settle after a few rows; a
 // stale read can only cause an atomic that was not needed.  Round 1's unconditional atomic was slower: 1 520 against
 // 1 497 us per 200 M config-5 rows, profiles/r01_config5_sweep.jsonl)
-template <int OP> NQ_DEV void cache_mm32(u32* c, u64 x, u64 bias) {
-    const u32 v = (u32)(x - bias) + 1u;
-    const u32 cur = *(volatile u32*)c;
-    if (OP == OP_MIN_I64 || OP == OP_MIN_U64) { if (v < cur) atomicMin(c, v); } else { if (v > cur) atomicMax(c, v); }
-}
 // the same with the cell's current value already in a register (two interleaved cells fetched by one 64-bit load)
-template <int OP> NQ_DEV void cache_mm32_cur(u32* c, u64 x, u64 bias, u32 cur) {
+template <int OP> NQ_DEV void cache_mm32_cur(u32 c, u64 x, u64 bias, u32 cur) {
     const u32 v = (u32)(x - bias) + 1u;
-    if (OP == OP_MIN_I64 || OP == OP_MIN_U64) { if (v < cur) atomicMin(c, v); } else { if (v > cur) atomicMax(c, v); }
+    if (OP == OP_MIN_I64 || OP == OP_MIN_U64) { if (v < cur) reds_min(c, v); } else { if (v > cur) reds_max(c, v); }
 }
-NQ_DEV void cache_or32(u32* c, u32 bits) {
-    if ((*(volatile u32*)c & bits) != bits) atomicOr(c, bits);
+template <int OP> NQ_DEV void cache_mm32(u32 c, u64 x, u64 bias) { cache_mm32_cur<OP>(c, x, bias, lds_u32(c)); }
+template <int OP> NQ_DEV void cache_mm32(u32* c, u64 x, u64 bias) { cache_mm32<OP>(smem_addr(c), x, bias); }
+NQ_DEV void cache_or32(u32 c, u32 bits) {
+    if ((lds_u32(c) & bits) != bits) reds_or(c, bits);
 }
 template <int OP> NQ_DEV void cache_word64(u64* c, u64 x) {
     if (OP == OP_MIN_I64) { if ((i64)x < *(volatile i64*)c) atomicMin((i64*)c, (i64)x); }
