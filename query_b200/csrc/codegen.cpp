@@ -460,6 +460,8 @@ KernelPlan generate_kernel(const Table& t, const Expr* where, const std::vector<
     auto add_word = [&](int op, const std::string& key, bool counter = false, i64 lo = 1, i64 hi = 0) {
         auto it = shared.find(key);
         if (it != shared.end()) return it->second;
+        // checked here, before any index is stored: FinalAgg keeps word indices in a signed char
+        if (kp.word_ops.size() == 64) N1_THROW(N1GPU_E_INELIGIBLE, "more than 64 accumulator words per group");
         kp.word_ops.push_back(op);
         kp.word_count.push_back(counter);
         kp.word_lo.push_back(lo);

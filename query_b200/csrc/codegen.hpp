@@ -42,29 +42,11 @@ struct InSet {
     u32 flags = 0;                 // INSET_* of n1ql_device.cuh
 };
 
-struct AggPlan {
-    AggKind kind = AggKind::COUNT;
-    bool distinct = false, star = false;
+// One aggregate: what finalises it (FinalAgg, final_group.hpp) and what only the code generator needs
+struct AggPlan : FinalAgg {
+    bool star = false;
     std::string text;          // the aggregate's Stringer text (the key of the "aggregates" attachment)
     u32 opmask = 0;            // classes the operand may take
-    // accumulator word indices (-1 = absent)
-    int w_cnt = -1;
-    int w_isum = -1;           // exact single-word int sum (range proves no overflow)
-    int w_ilo = -1, w_ihi = -1;  // split int sum: sum of low 32 bits / sum of (x >> 32)
-    int w_nint = -1, w_neg = -1;  // ints summed / negative ints among them (intValue.Add: mixed signs -> float64)
-    int w_fsum = -1, w_nflt = -1;
-    // "float-carried" sum of an operand that mixes INT and FLOAT values whose ints are provably small (|x| * rows < 2^53):
-    // every number is added to ONE float64 word (integers that small add exactly in float64, so an all-INT group still
-    // gets its exact int64 sum), w_nnum counts the numbers, and three bits of a shared OR word remember whether a float,
-    // a negative int or a non-negative int was seen (the int / float class of the result: value/integer.go:266-277).
-    // the sign mix of the summed ints read off MIN / MAX of the same operand (any negative <=> min < 0, any non-negative
-    // <=> max >= 0) instead of a counter of negatives: one accumulator word (and one cache cell) less
-    int w_sgn_min = -1, w_sgn_max = -1;
-    bool fcarry = false;
-    int w_nnum = -1, w_flags = -1, flag_shift = 0;
-    int w_seen = -1, w_mi = -1, w_mf = -1, w_ms = -1;
-    int w_seen_cnt = -1, seen_class = -1;  // single-class operand: "seen" = (this count word > 0) ? bit(seen_class) : 0
-    int dict_col = -1;
     int distinct_id = -1;      // index among DISTINCT aggregates
     PackComp dcomp;
 };

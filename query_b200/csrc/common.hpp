@@ -13,15 +13,10 @@
 #include <vector>
 
 #include "../../include/n1gpu.h"
+#include "final_group.hpp"
 
 namespace n1 {
 
-typedef long long i64;           // same types as the device library (n1ql_device.cuh)
-typedef unsigned long long u64;
-typedef uint32_t u32;
-typedef uint8_t u8;
-
-enum : int { C_MISSING = 0, C_NULL = 1, C_FALSE = 2, C_TRUE = 3, C_INT = 4, C_FLOAT = 5, C_STRING = 6, C_OTHER = 7 };
 enum : int { OP_ADD_U64 = 0, OP_ADD_F64 = 1, OP_MIN_I64 = 2, OP_MAX_I64 = 3, OP_MIN_U64 = 4, OP_MAX_U64 = 5, OP_OR_U64 = 6 };
 
 inline u32 bit(int c) { return 1u << c; }
@@ -59,6 +54,8 @@ struct HValue {
     u8 cls = C_MISSING;
     i64 bits = 0;
     std::string s;
+    HValue() = default;
+    HValue(FinalVal v) : cls((u8)v.cls), bits(v.bits) {}  // a number from final_group.hpp (new_num)
     static HValue missing() { return HValue(); }
     static HValue null() { HValue v; v.cls = C_NULL; return v; }
     static HValue boolean(bool b) { HValue v; v.cls = b ? C_TRUE : C_FALSE; return v; }
@@ -68,15 +65,6 @@ struct HValue {
     double f() const { double d; memcpy(&d, &bits, 8); return d; }
     double num() const { return cls == C_INT ? (double)bits : f(); }
 };
-
-// Go's int64(float64) on amd64 and value.IsInt (value/integer.go:354-356)
-inline i64 go_i64(double d) {
-    if (!(d >= -9223372036854775808.0 && d < 9223372036854775808.0)) return INT64_MIN;
-    return (i64)d;
-}
-inline bool f_is_int(double d) { return d == (double)go_i64(d); }
-// value.NewValue(float64) (value/value.go:377-382)
-inline HValue new_num(double d) { return f_is_int(d) ? HValue::integer(go_i64(d)) : HValue::flt(d); }
 
 // caching allocators (mem.cpp)
 void* dev_alloc(size_t n, size_t* actual);

@@ -26,8 +26,6 @@ enum class EK {
     ROUND   // round(x [, digits]) - host only: the operators behind FinalGroup (group_tail.cpp); never reaches a kernel
 };
 
-enum class AggKind { COUNT, COUNTN, SUM, AVG, MIN, MAX };
-
 struct TypeInfo {
     u32 mask = 0;          // classes the value may take
     bool ranged = false;   // INT values proven within [lo, hi]

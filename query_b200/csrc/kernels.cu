@@ -2,7 +2,8 @@
 // initialisation, table / DISTINCT set -> record compaction with owner bucketing (the export side of the
 // multi-GPU IntermediateGroup exchange, also the compaction step of finalisation), record -> table merging
 // (CumulateIntermediate: algebra/agg_*.go, execution/group_intermediate.go:56-104), the element-wise merges of
-// small-state chains and the device-side ComputeFinal of DISTINCT aggregates.
+// small-state chains, the device-side ComputeFinal of DISTINCT aggregates and FinalGroup over HBM tables
+// (k_finalize_groups, through final_group.hpp: the one restatement of ComputeFinal, shared with the host finalisation).
 #include <algorithm>
 
 #include "kernels.hpp"
@@ -174,12 +175,6 @@ __global__ void k_merge_records(int kw, u64* keys, u64* acc, u64 cap, OpsArr ops
 // DISTINCT finalisation (ComputeFinal of count/countn/sum/avg DISTINCT: algebra/agg_*_distinct.go): every entry of the
 // (aggregate, group, value) set adds 1 to its group's distinct count and, for SUM/AVG, its value to the group's exact
 // split integer sum / float sum.  kw: how the group slot is found (3 ungrouped, 0 dense, 1 / 2 hash 64 / 128).
-__device__ __forceinline__ u64 take_bits(unsigned __int128& v, int n) {
-    if (n == 0) return 0;
-    const u64 r = n >= 64 ? (u64)v : ((u64)v & ((1ULL << n) - 1));
-    v >>= n;
-    return r;
-}
 __device__ __forceinline__ void distinct_entry(u64 lo, u64 hi, int abits, int key_bits, int kw, const u64* __restrict__ keys, u64 cap,
                                                u64* acc, const DistinctDescs& D) {
     {
@@ -194,30 +189,23 @@ __device__ __forceinline__ void distinct_entry(u64 lo, u64 hi, int abits, int ke
         else slot = table_find128((const ulonglong2*)keys, cap - 1, klo, khi);
         if (slot < 0 || (u64)slot >= cap) return;  // group owned by another rank
         bool decoded = false;
-        int cls = C_MISSING;
-        u64 pv = 0;
+        FinalVal val{C_MISSING, 0};
         for (int a = 0; a < D.n; ++a) {
             const DistinctDesc& d = D.d[a];
             if (d.sid != sid) continue;
             if (!decoded) {  // the value component is packed identically for every aggregate of the set
-                int ci = (int)take_bits(v, d.cbits);
-                pv = take_bits(v, d.pbits);
-                if (d.nfree >= 0) {  // offset packing: one field
-                    ci = pv < (u64)d.nfree ? (int)pv : d.nfree;
-                    pv = pv < (u64)d.nfree ? 0 : pv - (u64)d.nfree;
-                }
-                cls = ci < 8 ? d.classes[ci] : C_MISSING;
+                val = decode_comp(d.value, v);
                 decoded = true;
             }
-            if (d.numbers_only && !(cls == C_INT || cls == C_FLOAT)) continue;
+            if (d.numbers_only && !(val.cls == C_INT || val.cls == C_FLOAT)) continue;
             atomicAdd(&acc[(u64)d.w_cnt * cap + (u64)slot], 1ULL);
-            if (cls == C_INT && d.w_ilo >= 0) {
-                const i64 x = d.biased ? (i64)(pv + (u64)d.bias) : (i64)pv;
+            if (val.cls == C_INT && d.w_ilo >= 0) {
+                const i64 x = val.bits;
                 atomicAdd(&acc[(u64)d.w_ilo * cap + (u64)slot], (u64)x & 0xffffffffULL);
                 atomicAdd(&acc[(u64)d.w_ihi * cap + (u64)slot], (u64)(x >> 32));
                 if (x < 0) atomicAdd(&acc[(u64)d.w_neg * cap + (u64)slot], 1ULL);
-            } else if (cls == C_FLOAT && d.w_fsum >= 0) {
-                atomicAdd((double*)&acc[(u64)d.w_fsum * cap + (u64)slot], __longlong_as_double((i64)pv));
+            } else if (val.cls == C_FLOAT && d.w_fsum >= 0) {
+                atomicAdd((double*)&acc[(u64)d.w_fsum * cap + (u64)slot], __longlong_as_double(val.bits));
                 atomicAdd(&acc[(u64)d.w_nflt * cap + (u64)slot], 1ULL);
             }
         }
@@ -289,46 +277,10 @@ __global__ void k_merge_mailbox(const u64* mail, int nranks, u64 slot_base, u64 
 }
 
 // ---- FinalGroup on the device -------------------------------------------------------------------------------------------
-// Restates ComputeFinal (algebra/agg_count.go:95-149, agg_countn.go:77-129, agg_sum.go:77-136 with value/integer.go:266-277,
-// agg_avg.go:117-131, agg_min.go / agg_max.go:76-127, agg_*_distinct.go) per group and decodes the bit-packed group key
-// (execution/group_final.go:55-118 sends one item per group): one thread per table slot, live groups compacted into flat
-// arrays through a warp-aggregated cursor.  Strings leave as (dictionary column << 40 | rank); the host resolves them.
-struct HV { int cls; i64 bits; };
-__device__ __forceinline__ HV hv(int c, i64 b) { HV v; v.cls = c; v.bits = b; return v; }
-__device__ __forceinline__ HV hv_flt(double d) { return hv(C_FLOAT, __double_as_longlong(d)); }
-__device__ __forceinline__ HV hv_new_num(double d) { const Val v = ::new_num(d); return hv(v.c, v.b); }
-__device__ __forceinline__ double hv_num(HV v) { return v.cls == C_INT ? (double)v.bits : __longlong_as_double(v.bits); }
-__device__ __forceinline__ bool fits_i64(__int128 v) { return v >= (__int128)NQ_I64_MIN && v <= (__int128)NQ_I64_MAX; }
-__device__ __forceinline__ HV sum_value(__int128 itotal, u64 n_nonneg, u64 n_neg, u64 n_flt, double fsum, bool from_zero) {
-    const u64 nI = n_nonneg + n_neg;
-    if (nI + n_flt == 0) return hv(C_NULL, 0);
-    if (n_flt == 0) {
-        const bool same_sign = from_zero ? (n_neg == 0) : (n_neg == 0 || n_nonneg == 0);
-        if (same_sign && fits_i64(itotal)) return hv(C_INT, (i64)itotal);
-        return hv_flt((double)itotal);
-    }
-    if (nI == 0) return hv_flt(fsum);
-    return hv_flt((double)itotal + fsum);
-}
-__device__ __forceinline__ HV decode_comp(const FinalComp& pc, unsigned __int128& bits) {
-    u64 ci = take_bits(bits, pc.cbits);
-    u64 pv = take_bits(bits, pc.pbits);
-    if (pc.nfree >= 0) {
-        ci = pv < (u64)pc.nfree ? pv : (u64)pc.nfree;
-        pv = pv < (u64)pc.nfree ? 0 : pv - (u64)pc.nfree;
-    }
-    const int cls = ci < (u64)pc.nclasses ? pc.classes[ci] : C_MISSING;
-    switch (cls) {
-        case C_INT: return hv(C_INT, pc.biased ? (i64)(pv + (u64)pc.bias) : (i64)pv);
-        case C_FLOAT: return hv(C_FLOAT, (i64)pv);
-        case C_STRING: return hv(C_STRING, (i64)(((u64)pc.dict_col << 40) | (pv & 0xffffffffffULL)));
-        case C_NULL: return hv(C_NULL, 0);
-        case C_FALSE: return hv(C_FALSE, 0);
-        case C_TRUE: return hv(C_TRUE, 0);
-        default: return hv(C_MISSING, 0);
-    }
-}
-
+// One thread per table slot: the slot's words folded over the partial tables, live groups compacted into flat arrays
+// through a warp-aggregated cursor and finalised by final_group (final_group.hpp, the restatement of ComputeFinal and of
+// the key decoding that the host finalisation shares; execution/group_final.go:55-118 sends one item per group).  Strings
+// leave as (dictionary column << 40 | rank); the host resolves them.
 __global__ void __launch_bounds__(256) k_finalize_groups(const FinalDesc D, int kw, const u64* __restrict__ keys, const PeerTables T, const OpsArr ops,
                                                          u64 ws, u64 ss, u64 slot0, u64 slot1, unsigned long long* counter, u64 out_cap,
                                                          u8* key_cls, i64* key_val, u8* agg_cls, i64* agg_val) {
@@ -364,91 +316,8 @@ __global__ void __launch_bounds__(256) k_finalize_groups(const FinalDesc D, int 
         if (!live) continue;
         const u64 g = base + (u64)__popc(m & ((1u << lane) - 1u));
         if (g >= out_cap) continue;
-        u64 w[64];  // logical words: packed counter fields decoded, complemented counters restored
-        for (int l = 0; l < D.LW; ++l) {
-            const u64 v = pw[D.phys_of[l]];
-            w[l] = D.bits_of[l] == 64 ? v : (v >> D.shift_of[l]) & 0xffffffffULL;
-        }
-        for (int l = 0; l < D.LW; ++l) if (D.complement[l]) w[l] = w[0] - w[l];
-        unsigned __int128 kb = ((unsigned __int128)khi << 64) | klo;
-        for (int k = 0; k < D.nkeys; ++k) {
-            const HV kv = decode_comp(D.keys[k], kb);
-            key_cls[g * D.nkeys + k] = (u8)kv.cls;
-            key_val[g * D.nkeys + k] = kv.bits;
-        }
-        for (int a = 0; a < D.naggs; ++a) {
-            const FinalAgg& ap = D.aggs[a];
-            HV out = hv(C_NULL, 0);
-            if (ap.distinct) {
-                const u64 count = w[ap.w_cnt];
-                if (ap.kind == 0 || ap.kind == 1) out = hv(C_INT, (i64)count);   // COUNT / COUNTN DISTINCT
-                else if (count != 0) {
-                    __int128 itotal = 0;
-                    u64 n_neg = 0, n_flt = 0;
-                    double fsum = 0;
-                    if (ap.w_ilo >= 0) itotal = (((__int128)(i64)w[ap.w_ihi]) << 32) + (__int128)w[ap.w_ilo];
-                    if (ap.w_neg >= 0) n_neg = w[ap.w_neg];
-                    if (ap.w_nflt >= 0) n_flt = w[ap.w_nflt];
-                    if (ap.w_fsum >= 0) fsum = __longlong_as_double((i64)w[ap.w_fsum]);
-                    const HV sv = sum_value(itotal, count - n_neg - n_flt, n_neg, n_flt, fsum, true);
-                    out = ap.kind == 2 ? sv : hv_new_num(hv_num(sv) / (double)count);
-                }
-            } else if (ap.kind == 0 || ap.kind == 1) {
-                out = hv(C_INT, (i64)w[ap.w_cnt]);
-            } else if (ap.fcarry) {
-                const u64 count = w[ap.w_nnum], flags = (w[ap.w_flags] >> ap.flag_shift) & 7;
-                const double fs = __longlong_as_double((i64)w[ap.w_fsum]);
-                HV sv;
-                if (count == 0) sv = hv(C_NULL, 0);
-                else if ((flags & 1) || ((flags & 2) && (flags & 4))) sv = hv_flt(fs);
-                else sv = hv(C_INT, (i64)fs);
-                out = (ap.kind == 2 || sv.cls == C_NULL) ? sv : hv_new_num(hv_num(sv) / (double)count);
-            } else if (ap.kind == 2 || ap.kind == 3) {  // SUM / AVG
-                __int128 itotal = 0;
-                u64 n_neg = 0, n_nonneg = 0, n_flt = 0;
-                double fsum = 0;
-                if (ap.w_isum >= 0) itotal = (i64)w[ap.w_isum];
-                else if (ap.w_ilo >= 0) itotal = (((__int128)(i64)w[ap.w_ihi]) << 32) + (__int128)w[ap.w_ilo];
-                if (ap.w_neg >= 0) n_neg = w[ap.w_neg];
-                if (ap.w_nint >= 0) n_nonneg = w[ap.w_nint] - n_neg;
-                if (ap.w_sgn_min >= 0 && ap.w_nint >= 0 && w[ap.w_nint]) {  // the sign mix from MIN / MAX of the operand
-                    const bool any_neg = (i64)w[ap.w_sgn_min] < 0, any_nonneg = (i64)w[ap.w_sgn_max] >= 0;
-                    n_neg = any_neg ? (any_nonneg ? 1 : w[ap.w_nint]) : 0;
-                    n_nonneg = w[ap.w_nint] - n_neg;
-                }
-                if (ap.w_nflt >= 0) n_flt = w[ap.w_nflt];
-                if (ap.w_fsum >= 0) fsum = __longlong_as_double((i64)w[ap.w_fsum]);
-                const HV sv = sum_value(itotal, n_nonneg, n_neg, n_flt, fsum, false);
-                out = (ap.kind == 2 || sv.cls == C_NULL) ? sv : hv_new_num(hv_num(sv) / (double)(n_nonneg + n_neg + n_flt));
-            } else {  // MIN / MAX: the collation winner over the classes seen
-                const bool mn = ap.kind == 4;
-                const u64 seen = ap.w_seen >= 0 ? w[ap.w_seen] : (w[ap.w_seen_cnt] ? (1ULL << ap.seen_class) : 0);
-                const bool hi = seen & (1ULL << C_INT), hf = seen & (1ULL << C_FLOAT);
-                const i64 iv = ap.w_mi >= 0 ? (i64)w[ap.w_mi] : 0;
-                const double fv = ap.w_mf >= 0 ? f64_unordered(w[ap.w_mf]) : 0;
-                HV number;
-                if (hi && hf) {  // intValue.Collate(floatValue): float64 compare (value/integer.go:100-118)
-                    const double ad = (double)iv;
-                    number = (mn ? (ad <= fv) : (ad >= fv)) ? hv(C_INT, iv) : hv_flt(fv);
-                } else number = hi ? hv(C_INT, iv) : hv_flt(fv);
-                const HV str = hv(C_STRING, ap.w_ms >= 0 ? (i64)(((u64)(unsigned short)ap.dict_col << 40) | (w[ap.w_ms] & 0xffffffffffULL)) : 0);
-                const u64 M_NUMB = (1ULL << C_INT) | (1ULL << C_FLOAT);
-                if (seen == 0) out = hv(C_NULL, 0);
-                else if (mn) {
-                    if (seen & (1ULL << C_FALSE)) out = hv(C_FALSE, 0);
-                    else if (seen & (1ULL << C_TRUE)) out = hv(C_TRUE, 0);
-                    else if (seen & M_NUMB) out = number;
-                    else out = str;
-                } else {
-                    if (seen & (1ULL << C_STRING)) out = str;
-                    else if (seen & M_NUMB) out = number;
-                    else if (seen & (1ULL << C_TRUE)) out = hv(C_TRUE, 0);
-                    else out = hv(C_FALSE, 0);
-                }
-            }
-            agg_cls[g * D.naggs + a] = (u8)out.cls;
-            agg_val[g * D.naggs + a] = out.bits;
-        }
+        final_group(D, D.keys, D.nkeys, klo, khi, pw, key_cls + g * D.nkeys, key_val + g * D.nkeys, agg_cls + g * D.naggs,
+                    agg_val + g * D.naggs);
     }
 }
 

@@ -1,6 +1,7 @@
 // kernels.hpp — host launchers of the static kernels in kernels.cu
 #pragma once
 #include "common.hpp"
+#include "final_group.hpp"
 
 namespace n1 {
 
@@ -14,34 +15,14 @@ struct DistinctDesc {
     int sid;           // entry set this aggregate reads (aggregates over the same operand share one)
     int numbers_only;  // COUNTN / SUM / AVG DISTINCT: only numeric entries count (COUNT: every entry)
     int w_cnt, w_ilo, w_ihi, w_neg, w_fsum, w_nflt;  // word indices (-1 = not needed)
-    int cbits, pbits, biased;
-    int nfree;         // >= 0: offset packing (PackComp::nfree)
-    i64 bias;
-    int classes[8];
+    FinalComp value;   // the value component of a set entry
 };
 struct DistinctDescs {
     int n;
     DistinctDesc d[16];
 };
-// ---- device-side FinalGroup (ComputeFinal of every aggregate + key decoding), see k_finalize_groups -----------------------
+// ---- device-side FinalGroup (final_group.hpp), see k_finalize_groups ------------------------------------------------------
 // How the table is addressed: word w of slot i lives at acc[w * ws + i * ss] (word-major: ws = capacity, ss = 1).
-struct FinalComp {   // PackComp as plain data
-    int cbits, pbits, nfree, biased, dict_col, nclasses;
-    i64 bias;
-    int classes[8];
-};
-struct FinalAgg {    // AggPlan as plain data (word indices are LOGICAL words, -1 = absent)
-    signed char kind, distinct, fcarry, seen_class;
-    short dict_col;
-    signed char w_cnt, w_isum, w_ilo, w_ihi, w_nint, w_neg, w_fsum, w_nflt, w_seen, w_mi, w_mf, w_ms, w_seen_cnt, w_nnum, w_flags, flag_shift;
-    signed char w_sgn_min, w_sgn_max;
-};
-struct FinalDesc {
-    int nkeys, naggs, LW, PW;
-    unsigned char phys_of[64], shift_of[64], bits_of[64], complement[64];
-    FinalComp keys[16];
-    FinalAgg aggs[24];
-};
 // The partial tables the groups are read from: one (this rank's) or one per rank, combined word by word with the merge
 // operations on the fly (IntermediateGroup fused into FinalGroup; peers are mapped over NVLink).
 struct PeerTables {

@@ -1,12 +1,7 @@
 // query.cpp — compile / scan / merge / finalise of one Filter + Group chain.
 //
-// Reference behaviour restated in finalize() (file:line under /root/reference):
-//   algebra/agg_count.go:95-149, agg_countn.go:77-129   counts are int64
-//   algebra/agg_sum.go:77-136 + value/integer.go:266-277  int64 sum stays int while every operand shares a
-//       sign class and the total fits, otherwise float64
-//   algebra/agg_avg.go:117-131   float64(sum)/float64(count), then value.NewValue (integral -> int)
-//   algebra/agg_min.go:76-127, agg_max.go:76-127   collation winner over any type, NULL when nothing counted
-//   algebra/agg_*_distinct.go + value/set.go:65-110  DISTINCT sets; SUM starts from int 0 (0 + negative -> float)
+// finalize() finalises the groups on the host or on the device (k_finalize_groups); both run the one restatement of
+// ComputeFinal in final_group.hpp.  Reference behaviour the host side adds:
 //   execution/group_final.go:108-117   no keys and no input -> one row of Default() values
 #include "query.hpp"
 
@@ -106,7 +101,6 @@ std::unique_ptr<Query> Query::compile(Table* t, const std::string& alias, const 
     // rows any one accumulator can see over all partitions: declared (n1gpu_table_set_global_rows), else room for 16 ranks
     const double rows_bound = t->global_rows > 0 ? (double)std::max<i64>(t->global_rows, t->nrows) : (double)std::max<i64>(t->nrows, 1) * 16.0;
     q->kp = generate_kernel(*t, q->where.get(), q->keys, q->aggs, agg_texts, rows_bound);
-    if (q->kp.word_ops.size() > 64) N1_THROW(N1GPU_E_INELIGIBLE, "more than 64 accumulator words per group");
     q->ops.n = (int)q->kp.phys_ops.size();  // physical words: what the table holds and every merge moves
     for (int w = 0; w < q->ops.n; ++w) q->ops.op[w] = q->kp.phys_ops[w];
     if (have_device()) {
@@ -516,67 +510,13 @@ void Query::partial_import(const void* dev_records, i64 n, const void* dev_disti
 
 // ---- finalisation (FinalGroup / ComputeFinal) -----------------------------------------------------------------------
 namespace {
-struct BitReader {
-    unsigned __int128 v;
-    explicit BitReader(u64 lo, u64 hi) : v(((unsigned __int128)hi << 64) | lo) {}
-    u64 take(int n) {
-        if (n == 0) return 0;
-        u64 r = n >= 64 ? (u64)v : ((u64)v & (((u64)1 << n) - 1));
-        v >>= n;
-        return r;
-    }
-};
-
-// a string of a result, until finalize() resolves it: (dictionary column, rank)
-HValue str_ref(int col, u64 rank) { HValue v; v.cls = C_STRING; v.bits = (i64)(((u64)col << 40) | (rank & 0xffffffffffULL)); return v; }
-
-HValue decode_comp(const Table& t, const PackComp& pc, BitReader& br) {
-    u64 ci = br.take(pc.cbits);
-    u64 pv = br.take(pc.pbits);
-    if (pc.nfree >= 0) {  // offset packing: one field
-        ci = pv < (u64)pc.nfree ? pv : (u64)pc.nfree;
-        pv = pv < (u64)pc.nfree ? 0 : pv - (u64)pc.nfree;
-    }
-    int cls = ci < pc.classes.size() ? pc.classes[ci] : C_MISSING;
-    switch (cls) {
-        case C_INT: return HValue::integer(pc.biased ? (i64)(pv + (u64)pc.bias) : (i64)pv);
-        case C_FLOAT: { HValue v; v.cls = C_FLOAT; v.bits = (i64)pv; return v; }
-        case C_STRING: return str_ref(pc.dict_col, pv);
-        case C_NULL: return HValue::null();
-        case C_FALSE: return HValue::boolean(false);
-        case C_TRUE: return HValue::boolean(true);
-        default: return HValue::missing();
-    }
+FinalComp final_comp(const PackComp& pc) {  // the plain data final_group.hpp decodes (keys, DISTINCT entry values)
+    FinalComp c{};
+    c.cbits = pc.cbits; c.pbits = pc.pbits; c.nfree = pc.nfree; c.biased = pc.biased; c.dict_col = pc.dict_col; c.bias = pc.bias;
+    c.nclasses = (int)std::min<size_t>(8, pc.classes.size());
+    for (int i = 0; i < c.nclasses; ++i) c.classes[i] = pc.classes[i];  // the rest stay C_MISSING
+    return c;
 }
-
-double f64_unordered(u64 k) {
-    u64 u = (k >> 63) ? (k & 0x7fffffffffffffffULL) : ~k;
-    double d;
-    memcpy(&d, &u, 8);
-    return d;
-}
-
-bool fits_i64(__int128 v) { return v >= (__int128)INT64_MIN && v <= (__int128)INT64_MAX; }
-
-struct SumState {
-    __int128 itotal = 0;
-    u64 n_nonneg = 0, n_neg = 0, n_flt = 0;
-    double fsum = 0;
-};
-// the SUM value as the reference's NumberValue chain would leave it (see header comment)
-HValue sum_value(const SumState& s, bool from_zero) {
-    u64 nI = s.n_nonneg + s.n_neg;
-    if (nI + s.n_flt == 0) return HValue::null();
-    if (s.n_flt == 0) {
-        bool same_sign = from_zero ? (s.n_neg == 0) : (s.n_neg == 0 || s.n_nonneg == 0);
-        if (same_sign && fits_i64(s.itotal)) return HValue::integer((i64)s.itotal);
-        return HValue::flt((double)s.itotal);
-    }
-    if (nI == 0) return HValue::flt(s.fsum);
-    return HValue::flt((double)s.itotal + s.fsum);
-}
-
-
 }  // namespace
 
 // slot of a shared-memory dense table -> the bit-packed group key (slots are the mixed-radix number of the components
@@ -591,23 +531,19 @@ u64 Query::dense_key(u64 slot) const {
 
 DistinctDescs Query::distinct_descs() const {
     DistinctDescs D{};
-    D.n = 0;
     for (auto& ap : kp.aggs) {
         if (!ap.distinct) continue;
         DistinctDesc& d = D.d[D.n++];
         d.sid = ap.distinct_id;
         d.numbers_only = ap.kind != AggKind::COUNT;
         d.w_cnt = ap.w_cnt; d.w_ilo = ap.w_ilo; d.w_ihi = ap.w_ihi; d.w_neg = ap.w_neg; d.w_fsum = ap.w_fsum; d.w_nflt = ap.w_nflt;
-        d.cbits = ap.dcomp.cbits; d.pbits = ap.dcomp.pbits; d.biased = ap.dcomp.biased; d.bias = ap.dcomp.bias;
-        d.nfree = ap.dcomp.nfree;
-        for (int k = 0; k < 8; ++k) d.classes[k] = k < (int)ap.dcomp.classes.size() ? ap.dcomp.classes[k] : C_MISSING;
+        d.value = final_comp(ap.dcomp);
     }
     return D;
 }
 
 FinalDesc Query::final_desc() const {
-    FinalDesc D;
-    memset(&D, 0, sizeof D);
+    FinalDesc D{};
     D.nkeys = (int)keys.size();
     D.naggs = (int)aggs.size();
     D.LW = (int)kp.word_ops.size();
@@ -616,25 +552,9 @@ FinalDesc Query::final_desc() const {
         D.phys_of[l] = (unsigned char)kp.phys_of[l]; D.shift_of[l] = (unsigned char)kp.shift_of[l];
         D.bits_of[l] = (unsigned char)kp.bits_of[l]; D.complement[l] = kp.word_complement[l] ? 1 : 0;
     }
-    for (int k = 0; k < D.nkeys; ++k) {
-        const PackComp& pc = kp.keys[k];
-        FinalComp& c = D.keys[k];
-        c.cbits = pc.cbits; c.pbits = pc.pbits; c.nfree = pc.nfree; c.biased = pc.biased; c.dict_col = pc.dict_col; c.bias = pc.bias;
-        c.nclasses = (int)std::min<size_t>(8, pc.classes.size());
-        for (int i = 0; i < 8; ++i) c.classes[i] = i < c.nclasses ? pc.classes[i] : C_MISSING;
-    }
-    for (int a = 0; a < D.naggs; ++a) {
-        const AggPlan& ap = kp.aggs[a];
-        FinalAgg& f = D.aggs[a];
-        f.kind = (signed char)ap.kind; f.distinct = ap.distinct; f.fcarry = ap.fcarry; f.seen_class = (signed char)ap.seen_class;
-        f.dict_col = (short)ap.dict_col;
-        f.w_cnt = (signed char)ap.w_cnt; f.w_isum = (signed char)ap.w_isum; f.w_ilo = (signed char)ap.w_ilo; f.w_ihi = (signed char)ap.w_ihi;
-        f.w_nint = (signed char)ap.w_nint; f.w_neg = (signed char)ap.w_neg; f.w_fsum = (signed char)ap.w_fsum; f.w_nflt = (signed char)ap.w_nflt;
-        f.w_seen = (signed char)ap.w_seen; f.w_mi = (signed char)ap.w_mi; f.w_mf = (signed char)ap.w_mf; f.w_ms = (signed char)ap.w_ms;
-        f.w_seen_cnt = (signed char)ap.w_seen_cnt; f.w_nnum = (signed char)ap.w_nnum; f.w_flags = (signed char)ap.w_flags;
-        f.flag_shift = (signed char)ap.flag_shift;
-        f.w_sgn_min = (signed char)ap.w_sgn_min; f.w_sgn_max = (signed char)ap.w_sgn_max;
-    }
+    if (device_final_ok())  // D.keys serves the device only: the host takes chains of more than 16 key components
+        for (int k = 0; k < D.nkeys; ++k) D.keys[k] = final_comp(kp.keys[k]);
+    for (int a = 0; a < D.naggs; ++a) D.aggs[a] = kp.aggs[a];
     return D;
 }
 
@@ -689,7 +609,6 @@ i64 Query::finalize_device(Result& res, const PeerTables& tables, u64 slot0, u64
 
 std::unique_ptr<Result> Query::finalize() {
     const int W = ops.n;
-    const int LW = (int)kp.word_ops.size();
     const int rw = 2 + W;
     std::vector<u64> recs;
     i64 ngroups = 0;
@@ -782,115 +701,26 @@ std::unique_ptr<Result> Query::finalize() {
     res->agg_val.resize((size_t)ngroups * res->naggs);
 
     phase("result allocation");
-    // ComputeFinal of every group; a large group table (config 4: 10^6 groups) is finalised by all host cores
+    // FinalGroup of every group (final_group.hpp, as on the device); a large group table (config 4: 10^6 groups) is
+    // finalised by all host cores
+    const FinalDesc D = final_desc();
+    std::vector<FinalComp> kcomps;
+    for (auto& pc : kp.keys) kcomps.push_back(final_comp(pc));
+    const int nk = res->nkeys, na = res->naggs;
     auto final_range = [&](i64 g0, i64 g1) {
-    for (i64 g = g0; g < g1; ++g) {
-        const u64* r = &recs[(size_t)g * rw];
-        u64 w[64];  // logical words: packed counter fields decoded
-        for (int l = 0; l < LW; ++l) {
-            const u64 v = r[2 + kp.phys_of[l]];
-            w[l] = kp.bits_of[l] == 64 ? v : (v >> kp.shift_of[l]) & 0xffffffffULL;
+        for (i64 g = g0; g < g1; ++g) {
+            const u64* r = &recs[(size_t)g * rw];  // [key lo, key hi, physical words]
+            final_group(D, kcomps.data(), nk, r[0], r[1], r + 2, res->key_cls.data() + g * nk, res->key_val.data() + g * nk,
+                        res->agg_cls.data() + g * na, res->agg_val.data() + g * na);
         }
-        for (int l = 0; l < LW; ++l) if (kp.word_complement[l]) w[l] = w[0] - w[l];  // word 0 = rows in the group
-        BitReader br(r[0], r[1]);
-        for (int k = 0; k < res->nkeys; ++k) {
-            const HValue kv = decode_comp(*table, kp.keys[k], br);
-            res->key_cls[(size_t)g * res->nkeys + k] = kv.cls;
-            res->key_val[(size_t)g * res->nkeys + k] = kv.bits;
-        }
-        for (int a = 0; a < res->naggs; ++a) {
-            const AggPlan& ap = kp.aggs[a];
-            HValue out;
-            if (ap.distinct) {
-                const u64 count = w[ap.w_cnt];
-                if (ap.kind == AggKind::COUNT || ap.kind == AggKind::COUNTN) out = HValue::integer((i64)count);
-                else if (count == 0) out = HValue::null();
-                else {
-                    SumState s;  // entries of SUM/AVG DISTINCT are numbers only
-                    if (ap.w_ilo >= 0) s.itotal = (((__int128)(i64)w[ap.w_ihi]) << 32) + (__int128)w[ap.w_ilo];
-                    if (ap.w_neg >= 0) s.n_neg = w[ap.w_neg];
-                    if (ap.w_nflt >= 0) s.n_flt = w[ap.w_nflt];
-                    if (ap.w_fsum >= 0) memcpy(&s.fsum, &w[ap.w_fsum], 8);
-                    s.n_nonneg = count - s.n_neg - s.n_flt;
-                    HValue sv = sum_value(s, true);
-                    if (ap.kind == AggKind::SUM) out = sv;
-                    else out = new_num(sv.num() / (double)count);
-                }
-            } else if (ap.kind == AggKind::COUNT || ap.kind == AggKind::COUNTN) {
-                out = HValue::integer((i64)w[ap.w_cnt]);
-            } else if (ap.fcarry) {
-                // float-carried sum: integers this small add exactly in float64, so an all-INT group has its exact total
-                const u64 count = w[ap.w_nnum], flags = (w[ap.w_flags] >> ap.flag_shift) & 7;
-                double fs;
-                memcpy(&fs, &w[ap.w_fsum], 8);
-                HValue sv;
-                if (count == 0) sv = HValue::null();
-                else if (flags & 1) sv = HValue::flt(fs);
-                else if ((flags & 2) && (flags & 4)) sv = HValue::flt(fs);   // ints of both signs: intValue.Add went float
-                else sv = HValue::integer((i64)fs);
-                if (ap.kind == AggKind::SUM || sv.cls == C_NULL) out = sv;
-                else out = new_num(sv.num() / (double)count);
-            } else if (ap.kind == AggKind::SUM || ap.kind == AggKind::AVG) {
-                SumState s;
-                if (ap.w_isum >= 0) s.itotal = (i64)w[ap.w_isum];
-                else if (ap.w_ilo >= 0) s.itotal = (((__int128)(i64)w[ap.w_ihi]) << 32) + (__int128)w[ap.w_ilo];
-                if (ap.w_neg >= 0) s.n_neg = w[ap.w_neg];
-                if (ap.w_nint >= 0) s.n_nonneg = w[ap.w_nint] - s.n_neg;
-                if (ap.w_sgn_min >= 0 && ap.w_nint >= 0 && w[ap.w_nint]) {  // the sign mix from MIN / MAX of the operand
-                    const bool any_neg = (i64)w[ap.w_sgn_min] < 0, any_nonneg = (i64)w[ap.w_sgn_max] >= 0;
-                    s.n_neg = any_neg ? (any_nonneg ? 1 : w[ap.w_nint]) : 0;
-                    s.n_nonneg = w[ap.w_nint] - s.n_neg;
-                }
-                if (ap.w_nflt >= 0) s.n_flt = w[ap.w_nflt];
-                if (ap.w_fsum >= 0) memcpy(&s.fsum, &w[ap.w_fsum], 8);
-                HValue sv = sum_value(s, false);
-                if (ap.kind == AggKind::SUM || sv.cls == C_NULL) out = sv;
-                else out = new_num(sv.num() / (double)(s.n_nonneg + s.n_neg + s.n_flt));
-            } else {
-                bool mn = ap.kind == AggKind::MIN;
-                const u64 seen = ap.w_seen >= 0 ? w[ap.w_seen] : (w[ap.w_seen_cnt] ? bit(ap.seen_class) : 0);
-                auto number = [&]() -> HValue {
-                    bool hi = seen & bit(C_INT), hf = seen & bit(C_FLOAT);
-                    i64 iv = ap.w_mi >= 0 ? (i64)w[ap.w_mi] : 0;
-                    double fv = ap.w_mf >= 0 ? f64_unordered(w[ap.w_mf]) : 0;
-                    if (hi && hf) {
-                        double a = (double)iv;  // intValue.Collate(floatValue): float64 compare (value/integer.go:100-118)
-                        bool pick_int = mn ? (a <= fv) : (a >= fv);
-                        return pick_int ? HValue::integer(iv) : HValue::flt(fv);
-                    }
-                    return hi ? HValue::integer(iv) : HValue::flt(fv);
-                };
-                auto str = [&]() { return str_ref(ap.dict_col, w[ap.w_ms]); };
-                if (seen == 0) out = HValue::null();
-                else if (mn) {
-                    if (seen & bit(C_FALSE)) out = HValue::boolean(false);
-                    else if (seen & bit(C_TRUE)) out = HValue::boolean(true);
-                    else if (seen & M_NUM) out = number();
-                    else out = str();
-                } else {
-                    if (seen & bit(C_STRING)) out = str();
-                    else if (seen & M_NUM) out = number();
-                    else if (seen & bit(C_TRUE)) out = HValue::boolean(true);
-                    else out = HValue::boolean(false);
-                }
-            }
-            res->agg_cls[(size_t)g * res->naggs + a] = out.cls;
-            res->agg_val[(size_t)g * res->naggs + a] = out.bits;
-        }
-    }
     };
     {
         const int nthr = ngroups < 32768 ? 1 : (int)std::min<i64>(std::max(1u, std::thread::hardware_concurrency()), 32);
         if (nthr <= 1) final_range(0, ngroups);
         else {
             std::vector<std::thread> pool;
-            std::vector<std::string> errs((size_t)nthr);
-            for (int t = 0; t < nthr; ++t)
-                pool.emplace_back([&, t] {
-                    try { final_range(ngroups * t / nthr, ngroups * (t + 1) / nthr); } catch (const std::exception& e) { errs[(size_t)t] = e.what(); }
-                });
+            for (int t = 0; t < nthr; ++t) pool.emplace_back([&, t] { final_range(ngroups * t / nthr, ngroups * (t + 1) / nthr); });
             for (auto& th : pool) th.join();
-            for (auto& e : errs) if (!e.empty()) N1_THROW(N1GPU_E_INVALID, "%s", e.c_str());
         }
     }
     }  // host finalisation

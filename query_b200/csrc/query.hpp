@@ -202,7 +202,7 @@ struct Query {
     // fills res' flat arrays; returns the number of groups
     i64 finalize_device(Result& res, const PeerTables& tables, u64 slot0, u64 slot1);
     FinalDesc final_desc() const;
-    bool device_final_ok() const { return keys.size() <= 16 && aggs.size() <= 24 && kp.word_ops.size() <= 64 && table->cols.size() < 32768; }
+    bool device_final_ok() const { return keys.size() <= 16 && aggs.size() <= 24 && kp.word_ops.size() <= 64; }
     u64 dense_key(u64 slot) const;
     void rebind(Table* t);
 };
