@@ -151,7 +151,21 @@ namespace execution {
 
 namespace {
 
-struct CacheEntry { std::shared_ptr<Table> table; std::string source; };
+// A resident table and what it was built from: the source tag, and for a directory keyspace every entry (sorted) with the
+// fingerprint of the file its row was read from - the rows are those of the entries whose state is DOC, in order.
+struct Records {
+    std::vector<std::string> entries;
+    std::vector<DocFp> fps;
+    // the directory as readdir listed it, and that listing's sorted order: the next stat pass sorts nothing while the
+    // listing stays the same (sorting 10^6 names costs a quarter of a second)
+    std::vector<std::string> listed;
+    std::vector<u32> order;
+};
+struct CacheEntry {
+    std::shared_ptr<Table> table;
+    std::string source;
+    std::shared_ptr<const Records> recs;  // null: the rows cannot be told apart by entry (a packed keyspace)
+};
 std::mutex g_cache_mu;
 std::map<std::string, CacheEntry> g_tables;  // keyspace dir + columns -> resident shredded table (A.9)
 
@@ -164,10 +178,20 @@ std::string segment_dir() {
     return g_segment_dir;
 }
 
-// What a segment is valid for: the keyspace directory as the file datastore sees it (file.go:711-749) - modification
-// time of the directory (documents added / removed), number of documents, newest document (rewritten in place by
-// UPDATE, file.go:375-471) and their total size.  One stat per document; no document is opened.
-std::string keyspace_source_tag(const std::string& dir) {
+// A keyspace directory as one stat pass sees it.
+struct KeyspaceScan {
+    // What a segment is valid for: the keyspace directory as the file datastore sees it (file.go:711-749) - modification
+    // time of the directory (documents added / removed), number of documents, newest document (rewritten in place by
+    // UPDATE, file.go:375-471) and their total size.
+    std::string tag;
+    std::vector<std::string> entries;  // non-directory entries, sorted (the primary-key order of load_dir)
+    std::vector<DocFp> fps;            // the stat of each entry's document file (document_file)
+    std::vector<std::string> listed;   // see Records
+    std::vector<u32> order;
+};
+
+// One stat per entry (two for an entry that is not its own document file, a.txt -> a.json); no document is opened.
+KeyspaceScan scan_keyspace(const std::string& dir, const Records* prev) {
     DIR* d = opendir(dir.c_str());
     if (!d) N1_THROW(N1GPU_E_IO, "cannot open keyspace directory %s", dir.c_str());
     struct stat ds;
@@ -179,12 +203,21 @@ std::string keyspace_source_tag(const std::string& dir) {
         if (n[0] == '.' && (n[1] == 0 || (n[1] == '.' && n[2] == 0))) continue;
         names.emplace_back(n);
     }
+    std::vector<u32> order;
+    if (prev && prev->listed == names) order = prev->order;
+    else {
+        order.resize(names.size());
+        for (u32 i = 0; i < order.size(); ++i) order[i] = i;
+        std::sort(order.begin(), order.end(), [&](u32 a, u32 b) { return names[a] < names[b]; });
+    }
     // fstatat relative to the open directory, on all cores for a large keyspace (10^4 documents: 7 ms -> under 1 ms; this is
     // the whole cost of a query over a resident keyspace)
     const int dfd = dirfd(d);
     const size_t nthr = names.size() < 2048 ? 1 : std::min<size_t>(std::max(1u, std::thread::hardware_concurrency()), 16);
     struct Part { long long files = 0, bytes = 0, newest_s = 0, newest_ns = 0; };
     std::vector<Part> parts(nthr);
+    std::vector<DocFp> fps(names.size());
+    std::vector<char> is_entry(names.size(), 0);
     auto work = [&](size_t t) {
         Part& p = parts[t];
         for (size_t i = names.size() * t / nthr; i < names.size() * (t + 1) / nthr; ++i) {
@@ -193,6 +226,14 @@ std::string keyspace_source_tag(const std::string& dir) {
             ++p.files;
             p.bytes += (long long)st.st_size;
             if (st.st_mtim.tv_sec > p.newest_s || (st.st_mtim.tv_sec == p.newest_s && st.st_mtim.tv_nsec > p.newest_ns)) { p.newest_s = st.st_mtim.tv_sec; p.newest_ns = st.st_mtim.tv_nsec; }
+            is_entry[i] = 1;
+            const std::string doc = document_file(names[i]);
+            if (doc == names[i]) { fps[i] = DocFp::of(st); continue; }
+            struct stat ss;
+            if (fstatat(dfd, doc.c_str(), &ss, 0) == 0) {
+                if (S_ISDIR(ss.st_mode)) fps[i].state = DocFp::UNREADABLE;
+                else fps[i] = DocFp::of(ss);
+            } else fps[i].state = errno == ENOENT ? DocFp::ABSENT : DocFp::UNREADABLE;
         }
     };
     if (nthr == 1) work(0);
@@ -207,10 +248,98 @@ std::string keyspace_source_tag(const std::string& dir) {
         all.files += p.files; all.bytes += p.bytes;
         if (p.newest_s > all.newest_s || (p.newest_s == all.newest_s && p.newest_ns > all.newest_ns)) { all.newest_s = p.newest_s; all.newest_ns = p.newest_ns; }
     }
-    return strf("dir=%lld.%09lld files=%lld newest=%lld.%09lld bytes=%lld", dir_s, dir_ns, all.files, all.newest_s, all.newest_ns, all.bytes);
+    KeyspaceScan ks;
+    ks.tag = strf("dir=%lld.%09lld files=%lld newest=%lld.%09lld bytes=%lld", dir_s, dir_ns, all.files, all.newest_s, all.newest_ns, all.bytes);
+    ks.entries.reserve((size_t)all.files);
+    ks.fps.reserve((size_t)all.files);
+    for (const u32 i : order)
+        if (is_entry[i]) { ks.entries.push_back(names[i]); ks.fps.push_back(fps[i]); }
+    ks.listed = std::move(names);
+    ks.order = std::move(order);
+    return ks;
 }
 
-std::shared_ptr<Table> resident_table(const std::string& dir, std::vector<std::string> paths) {
+i64 realtime_ns() {
+    struct timespec ts;
+    clock_gettime(CLOCK_REALTIME, &ts);
+    return (i64)ts.tv_sec * 1000000000 + ts.tv_nsec;
+}
+
+// Racily clean files (git's rule): a file changed less than a timestamp tick before it was read can change again within
+// the same tick without its stat showing it.  Every file whose ctime is not older than the start of the load, less this
+// margin (coarse kernel timestamps lag the clock by up to a tick), is read again at the next check.
+const i64 RACY_MARGIN_NS = 20 * 1000000;
+void mark_racy(std::vector<DocFp>& fps, i64 start_ns) {
+    for (DocFp& f : fps) if (f.state == DocFp::DOC && f.ctime_ns >= start_ns - RACY_MARGIN_NS) f.racy = true;
+}
+
+void trace_phase(const char* what, const char* name, double& tp) {
+    static const bool trace = getenv("N1GPU_TRACE") != nullptr;
+    const double t = now_sec();
+    if (trace) fprintf(stderr, "[n1gpu %s] %-10s %8.3f ms\n", what, name, (t - tp) * 1e3);
+    tp = t;
+}
+
+// The cached table refreshed for a directory keyspace that changed: the rows of entries whose fingerprint holds are
+// kept, the documents of changed, new and unreadable entries are read again and shredded into a patch table, the rows of
+// deleted entries drop out, and the device splices the new columns from the old ones and the patch.  Returns the old table
+// itself when no row changed (a touched directory).  The result equals a load of the directory from scratch.
+std::shared_ptr<Table> refresh_table(const std::string& dir, const std::vector<std::string>& paths, const std::shared_ptr<Table>& old_table,
+                                     const Records& old, const KeyspaceScan& now, i64 start_ns, bool host_shred, std::vector<DocFp>& fps, i64* docs_read) {
+    double tp = now_sec();
+    // merge of the two sorted entry lists; old_row[i]: the old row of old entry i (-1: none)
+    std::vector<i64> old_row(old.entries.size(), -1);
+    i64 r = 0;
+    for (size_t i = 0; i < old.entries.size(); ++i) if (old.fps[i].state == DocFp::DOC) old_row[i] = r++;
+    if (r != old_table->nrows) N1_THROW(N1GPU_E_INVALID, "resident table of %s does not match its entries", dir.c_str());
+    std::vector<size_t> reread;           // indices into now.entries
+    std::vector<i64> keep(now.entries.size(), -2);  // the old row kept; -1: no row, as before; -2: read again
+    for (size_t i = 0, o = 0; i < now.entries.size(); ++i) {
+        while (o < old.entries.size() && old.entries[o] < now.entries[i]) ++o;  // deleted entries
+        if (o < old.entries.size() && old.entries[o] == now.entries[i]) {
+            if (old.fps[o].holds(now.fps[i])) { keep[i] = old_row[o]; fps[i] = old.fps[o]; }
+            ++o;
+        }
+        if (keep[i] == -2) reread.push_back(i);
+    }
+    trace_phase("refresh", "diff", tp);
+    std::shared_ptr<Table> patch;
+    std::vector<DocFp> pfps;
+    if (!reread.empty()) {
+        std::vector<std::string> names(reread.size());
+        for (size_t k = 0; k < reread.size(); ++k) names[k] = now.entries[reread[k]];
+        patch = std::make_shared<Table>();
+        for (auto& p : paths) patch->add_column(p);
+        patch->load_entries(dir, names, host_shred ? 0 : -1, &pfps);
+        mark_racy(pfps, start_ns);
+        for (size_t k = 0; k < reread.size(); ++k) fps[reread[k]] = pfps[k];
+        trace_phase("refresh", "read", tp);
+        patch->seal();
+        trace_phase("refresh", "seal", tp);
+        if (patch->nrows == 0) patch.reset();
+    }
+    *docs_read = patch ? patch->nrows : 0;
+    // runs: consecutive new rows from consecutive rows of one source
+    std::vector<SpliceRun> runs;
+    i64 at = 0, prow = 0;
+    auto add = [&](bool from_patch, i64 src) {
+        if (!runs.empty() && runs.back().patch == from_patch && runs.back().src_lo + runs.back().len == src) ++runs.back().len;
+        else runs.push_back(SpliceRun{at, from_patch, src, 1});
+        ++at;
+    };
+    for (size_t k = 0, i = 0; i < now.entries.size(); ++i) {
+        if (keep[i] >= 0) add(false, keep[i]);
+        else if (keep[i] == -2 && pfps[k++].state == DocFp::DOC) add(true, prow++);
+    }
+    if (!patch && at == old_table->nrows && runs.size() <= 1) return old_table;  // the same rows: nothing to splice
+    auto t = std::make_shared<Table>();
+    for (auto& p : paths) t->add_column(p);
+    t->splice(*old_table, patch.get(), runs);
+    trace_phase("refresh", "splice", tp);
+    return t;
+}
+
+std::shared_ptr<Table> resident_table(const std::string& dir, std::vector<std::string> paths, i64* docs_read) {
     std::sort(paths.begin(), paths.end());
     std::string key = dir;
     for (auto& p : paths) { key.push_back('\n'); key += p; }
@@ -222,35 +351,83 @@ std::shared_ptr<Table> resident_table(const std::string& dir, std::vector<std::s
     struct stat pst;
     const bool is_packed = !is_dir && stat(packed.c_str(), &pst) == 0 && S_ISREG(pst.st_mode);
     if (!is_dir && !is_packed) N1_THROW(N1GPU_E_IO, "keyspace directory %s not found", dir.c_str());
-    // the resident table and the segment live as long as this tag holds
-    const std::string tag = is_dir ? keyspace_source_tag(dir)
-                                   : strf("ndjson mtime=%lld.%09lld bytes=%lld", (long long)pst.st_mtim.tv_sec, (long long)pst.st_mtim.tv_nsec, (long long)pst.st_size);
+    // the resident table and the segment live as long as this tag holds; a directory keyspace's table as long as the
+    // fingerprints of its documents hold, and is refreshed from the changed documents when they do not
+    *docs_read = 0;
+    const i64 start_ns = realtime_ns();
+    double tp = now_sec();
+    std::shared_ptr<const Records> prev;
     {
         std::lock_guard<std::mutex> lk(g_cache_mu);
         auto it = g_tables.find(key);
-        if (it != g_tables.end() && it->second.source == tag) return it->second.table;
+        if (it != g_tables.end()) prev = it->second.recs;
     }
-    auto t = std::make_shared<Table>();
-    for (auto& p : paths) t->add_column(p);
+    KeyspaceScan scan;
+    if (is_dir) scan = scan_keyspace(dir, prev.get());
+    const std::string tag = is_dir ? scan.tag
+                                   : strf("ndjson mtime=%lld.%09lld bytes=%lld", (long long)pst.st_mtim.tv_sec, (long long)pst.st_mtim.tv_nsec, (long long)pst.st_size);
+    trace_phase("load", "stat", tp);
     const std::string segs = segment_dir();
-    bool from_segment = false;
-    if (!segs.empty()) {  // persistent columnar segment: skip reading and parsing the documents while nothing changed
-        const std::string file = segs + "/" + strf("%016llx", (unsigned long long)mix64(std::hash<std::string>()(key))) + ".n1seg";
-        from_segment = t->load_segment(file, tag);
-        if (!from_segment) { t->segment_out = file; t->segment_source = tag; }
+    const std::string file = segs.empty() ? std::string() : segs + "/" + strf("%016llx", (unsigned long long)mix64(std::hash<std::string>()(key))) + ".n1seg";
+    CacheEntry old;
+    {
+        std::lock_guard<std::mutex> lk(g_cache_mu);
+        auto it = g_tables.find(key);
+        if (it != g_tables.end()) {
+            if (it->second.source == tag && !it->second.recs) return it->second.table;  // (packed: the tag is all there is)
+            const Records* r = it->second.recs.get();
+            bool holds = is_dir && r && r->entries == scan.entries;
+            for (size_t i = 0; holds && i < scan.fps.size(); ++i) holds = r->fps[i].holds(scan.fps[i]);
+            if (holds) {
+                if (it->second.source == tag) return it->second.table;
+                // a touched directory: the same rows under a new tag (and the segment rewritten under it)
+                it->second.source = tag;
+                if (!file.empty() && have_device()) it->second.table->write_segment(file, tag);
+                return it->second.table;
+            }
+            old = it->second;
+        }
     }
-    if (!from_segment) {
-        // The documents are shredded on the device (raw text -> HBM once, no column crosses PCIe) unless a segment is to be
-        // written from the host shredder's staging, or N1GPU_OPERATOR_SHRED=host asks for the host threads.
-        const char* how = getenv("N1GPU_OPERATOR_SHRED");
-        const bool host = !have_device() || !t->segment_out.empty() || (how && std::string(how) == "host") || paths.empty();
-        const int threads = host ? 0 : -1;
-        if (is_dir) t->load_dir(dir, threads); else t->load_ndjson(packed, threads);
+    // The documents are shredded on the device (raw text -> HBM once, no column crosses PCIe) unless a segment is to be
+    // written from the host shredder's staging, or N1GPU_OPERATOR_SHRED=host asks for the host threads.
+    const char* how = getenv("N1GPU_OPERATOR_SHRED");
+    const bool host_env = (how && std::string(how) == "host") || paths.empty();
+    std::vector<DocFp> fps(scan.fps.size());
+    bool is_rec = true;
+    std::shared_ptr<Table> t;
+    if (is_dir && old.recs && have_device()) {
+        t = refresh_table(dir, paths, old.table, *old.recs, scan, start_ns, host_env, fps, docs_read);
+        t->global_rows = t->nrows;
+        if (!file.empty()) { t->write_segment(file, tag); trace_phase("refresh", "segment", tp); }
+    } else {
+        t = std::make_shared<Table>();
+        for (auto& p : paths) t->add_column(p);
+        bool from_segment = false;
+        if (!file.empty()) {  // persistent columnar segment: skip reading and parsing the documents while nothing changed
+            from_segment = t->load_segment(file, tag);
+            if (!from_segment) { t->segment_out = file; t->segment_source = tag; }
+        }
+        if (from_segment) {  // the stat pass that validated the tag gives the fingerprints
+            fps = scan.fps;
+            i64 docs = 0;
+            for (const DocFp& f : fps) docs += f.state == DocFp::DOC;
+            if (docs != t->nrows) is_rec = false;  // (rows that were not readable then): no refresh from these
+        } else {
+            const bool host = !have_device() || !t->segment_out.empty() || host_env;
+            const int threads = host ? 0 : -1;
+            if (is_dir) t->load_dir(dir, threads, &scan.entries, &fps); else t->load_ndjson(packed, threads);
+            *docs_read = t->nrows;
+        }
+        trace_phase("load", "read", tp);
+        t->global_rows = t->nrows;  // the operator runs the whole keyspace in this process: one partition
+        t->seal();
+        trace_phase("load", "seal", tp);
     }
-    t->global_rows = t->nrows;  // the operator runs the whole keyspace in this process: one partition
-    t->seal();
+    mark_racy(fps, start_ns);
+    std::shared_ptr<const Records> recs;
+    if (is_dir && is_rec) recs = std::make_shared<const Records>(Records{std::move(scan.entries), std::move(fps), std::move(scan.listed), std::move(scan.order)});
     std::lock_guard<std::mutex> lk(g_cache_mu);
-    g_tables[key] = CacheEntry{t, tag};
+    g_tables[key] = CacheEntry{t, tag, recs};
     return t;
 }
 
@@ -449,7 +626,7 @@ std::unique_ptr<GpuGroupAggregate> BuildWithTail(const std::string& plan_json, c
     for (auto& k : op->keys) collect_paths(*parse_expr(k), alias, paths);
     for (auto& a : op->aggregates) collect_paths(*parse_expr(a), alias, paths);
     double t0 = now_sec();
-    op->table = resident_table(op->keyspace_dir, paths);
+    op->table = resident_table(op->keyspace_dir, paths, &op->docs_read);
     op->query = Query::compile(op->table.get(), alias, op->condition.empty() ? nullptr : op->condition.c_str(), op->keys, op->aggregates);
     op->serv_sec = now_sec() - t0;
     if (outer_rest) *outer_rest = 0;
@@ -517,6 +694,7 @@ std::string GpuGroupAggregate::MarshalJSON() const {
     if (out_docs) stats += std::string(stats.empty() ? "" : ",") + "\"#itemsOut\":" + std::to_string(out_docs);
     if (exec_sec > 0) { stats += std::string(stats.empty() ? "" : ",") + "\"execTime\":"; json::quote(dur(exec_sec), stats); }
     if (serv_sec > 0) { stats += std::string(stats.empty() ? "" : ",") + "\"servTime\":"; json::quote(dur(serv_sec), stats); }
+    if (docs_read) stats += std::string(stats.empty() ? "" : ",") + "\"#docsRead\":" + std::to_string(docs_read);
     if (!stats.empty()) s += ",\"#stats\":{" + stats + "}";
     s += ",\"aggregates\":[";
     for (size_t i = 0; i < aggregates.size(); ++i) { if (i) s += ","; json::quote(aggregates[i], s); }

@@ -115,6 +115,7 @@ class GpuGroupAggregate {
     std::shared_ptr<Table> table;
     std::unique_ptr<Query> query;
     i64 in_docs = 0, out_docs = 0;
+    i64 docs_read = 0;  // documents read to build the table: all for a load, the changed ones for a refresh, 0 when reused
     double exec_sec = 0, serv_sec = 0;
     bool ran = false;
     // The operators after FinalGroup that this operator also replaces when all of them are within the subset

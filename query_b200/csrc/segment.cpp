@@ -62,8 +62,9 @@ struct Reader {
 };
 }  // namespace
 
-// Called by seal() once dictionaries are sorted and payloads hold ranks, before the host staging is dropped.
-void Table::write_segment() const {
+// Called by seal() once dictionaries are sorted and payloads hold ranks, before the host staging is dropped, or on a sealed
+// table whose columns live in HBM.
+void Table::write_segment(const std::string& segment_out, const std::string& segment_source) const {
     const std::string tmp = segment_out + ".tmp";
     std::ofstream f(tmp, std::ios::binary | std::ios::trunc);
     if (!f) N1_THROW(N1GPU_E_IO, "cannot write segment %s", tmp.c_str());
@@ -86,11 +87,29 @@ void Table::write_segment() const {
     auto put = [&](std::ofstream&, const void* p, size_t n) { w.put(p, n); };
     put(f, &hl, 8);
     put(f, h.data(), h.size());
+    // seal() writes from the host staging; a sealed table (a refreshed one) holds its columns in HBM only: they are copied
+    // back column by column
+    const bool device = sealed;
+    if (device && !have_device()) N1_THROW(N1GPU_E_INVALID, "a sealed table without a device has no columns to write");
+    std::vector<u8> dtags;
+    std::vector<char> dpay;
     for (auto& col : cols) {
         std::vector<i64> offs(col.dict.size() + 1, 0);
         for (size_t i = 0; i < col.dict.size(); ++i) offs[i + 1] = offs[i] + (i64)col.dict[i].size();
         put(f, offs.data(), offs.size() * 8);
         for (auto& s : col.dict) put(f, s.data(), s.size());
+        if (device) {
+            dtags.resize((size_t)nrows);
+            dpay.resize((size_t)nrows * (size_t)col.width);
+            if (nrows) {
+                CK(cudaMemcpyAsync(dtags.data(), col.d_tags.p, (size_t)nrows, cudaMemcpyDeviceToHost, nullptr));
+                if (col.width) CK(cudaMemcpyAsync(dpay.data(), col.d_payload.p, dpay.size(), cudaMemcpyDeviceToHost, nullptr));
+                CK(cudaStreamSynchronize(nullptr));
+            }
+            put(f, dpay.data(), dpay.size());
+            put(f, dtags.data(), dtags.size());
+            continue;
+        }
         if (col.width == 8) put(f, col.payload.data(), (size_t)nrows * 8);
         else if (col.width == 4) {
             std::vector<u32> narrow((size_t)nrows);

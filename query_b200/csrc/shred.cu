@@ -456,6 +456,84 @@ __global__ void k_patch(u8* tags, i64* payload, const i64* __restrict__ rows, co
     }
 }
 
+// ---- splice: a refreshed table's column from the old column and the re-read documents (execution.cpp, refresh) ---------
+// Row r of the new table comes from run k with new_lo[k] <= r < new_lo[k + 1]: row src_lo[k] + (r - new_lo[k]) of the old
+// column, or of the patch column when bit 63 of src_lo[k] is set.  A tile of SPLICE_TILE rows looks its first and last
+// runs up once; its rows then search only between those two (one run in the common case).
+#define SPLICE_TILE 256
+#define SPLICE_PATCH_BIT 0x8000000000000000ULL
+__device__ __forceinline__ i64 splice_find(const i64* __restrict__ new_lo, i64 lo, i64 hi, i64 row) {
+    while (lo < hi) { const i64 m = (lo + hi + 1) >> 1; if (new_lo[m] <= row) lo = m; else hi = m - 1; }
+    return lo;
+}
+__device__ __forceinline__ void splice_tile_runs(const i64* __restrict__ new_lo, i64 nruns, i64 t0, i64 nrows, i64* s_runs) {
+    if (threadIdx.x == 0) {
+        s_runs[0] = splice_find(new_lo, 0, nruns - 1, t0);
+        const i64 last = t0 + SPLICE_TILE - 1 < nrows ? t0 + SPLICE_TILE - 1 : nrows - 1;
+        s_runs[1] = splice_find(new_lo, s_runs[0], nruns - 1, last);
+    }
+    __syncthreads();
+}
+__device__ __forceinline__ i64 splice_payload(const i64* __restrict__ pay8, const u32* __restrict__ pay4, i64 row) {
+    return pay8 ? pay8[row] : (pay4 ? (i64)pay4[row] : 0);
+}
+// Pre-pass over the rows kept from the old column: the dictionary ranks they still use (bitmap) and their classes.
+__global__ void __launch_bounds__(SPLICE_TILE) k_splice_used(const i64* __restrict__ new_lo, const i64* __restrict__ src_lo, i64 nruns, i64 nrows,
+                                                            const u8* __restrict__ tags, const i64* __restrict__ pay8, const u32* __restrict__ pay4,
+                                                            u32* used, u64* class_mask) {
+    __shared__ i64 s_runs[2];
+    __shared__ u64 scratch[32];
+    u64 mask = 0;
+    for (i64 t0 = (i64)blockIdx.x * SPLICE_TILE; t0 < nrows; t0 += (i64)gridDim.x * SPLICE_TILE) {
+        splice_tile_runs(new_lo, nruns, t0, nrows, s_runs);
+        const i64 row = t0 + threadIdx.x;
+        if (row < nrows) {
+            const i64 k = splice_find(new_lo, s_runs[0], s_runs[1], row);
+            const u64 src = (u64)src_lo[k];
+            if (!(src & SPLICE_PATCH_BIT)) {
+                const i64 at = (i64)src + (row - new_lo[k]);
+                const int t = tags[at];
+                mask |= 1ULL << t;
+                if (t == C_STRING) { const u64 r = (u64)splice_payload(pay8, pay4, at); atomicOr(&used[r >> 5], 1u << (r & 31)); }
+            }
+        }
+        __syncthreads();  // s_runs is rewritten by the next tile
+    }
+    mask = block_reduce_word<OP_OR_U64>(mask, scratch);
+    if (threadIdx.x == 0 && mask) atomicOr(class_mask, mask);
+}
+// The new column: every padded row written once - spliced rows at the new width with ranks remapped into the new dictionary,
+// rows past nrows MISSING with a zero payload (as seal() pads them).
+__global__ void __launch_bounds__(SPLICE_TILE) k_splice_gather(const i64* __restrict__ new_lo, const i64* __restrict__ src_lo, i64 nruns, i64 nrows, i64 padded,
+                                                              const u8* __restrict__ o_tags, const i64* __restrict__ o_pay8, const u32* __restrict__ o_pay4,
+                                                              const u32* __restrict__ o_remap,
+                                                              const u8* __restrict__ p_tags, const i64* __restrict__ p_pay8, const u32* __restrict__ p_pay4,
+                                                              const u32* __restrict__ p_remap,
+                                                              u8* __restrict__ tags, i64* __restrict__ pay8, u32* __restrict__ pay4) {
+    __shared__ i64 s_runs[2];
+    for (i64 t0 = (i64)blockIdx.x * SPLICE_TILE; t0 < padded; t0 += (i64)gridDim.x * SPLICE_TILE) {
+        if (t0 < nrows) splice_tile_runs(new_lo, nruns, t0, nrows, s_runs);
+        const i64 row = t0 + threadIdx.x;
+        u8 t = C_MISSING;
+        i64 v = 0;
+        if (row < nrows) {
+            const i64 k = splice_find(new_lo, s_runs[0], s_runs[1], row);
+            const u64 src = (u64)src_lo[k];
+            const bool patch = (src & SPLICE_PATCH_BIT) != 0;
+            const i64 at = (i64)(src & ~SPLICE_PATCH_BIT) + (row - new_lo[k]);
+            t = patch ? p_tags[at] : o_tags[at];
+            v = patch ? splice_payload(p_pay8, p_pay4, at) : splice_payload(o_pay8, o_pay4, at);
+            if (t == C_STRING) v = (i64)(patch ? p_remap : o_remap)[v];
+        }
+        if (row < padded) {
+            tags[row] = t;
+            if (pay8) pay8[row] = v;
+            else if (pay4) pay4[row] = (u32)v;
+        }
+        if (t0 < nrows) __syncthreads();
+    }
+}
+
 static int sgrid(i64 n, int block) {
     i64 g = (n + block - 1) / block;
     if (g < 1) g = 1;
@@ -544,6 +622,19 @@ void launch_col_stats(const u8* tags, const i64* payload, i64 nrows, u64* stats,
 void launch_canon_floats(u8* tags, i64* payload, i64 nrows, cudaStream_t s) {
     if (nrows == 0) return;
     k_canon_floats<<<sgrid(nrows, 256), 256, 0, s>>>(tags, payload, nrows);
+    g_launches.fetch_add(1);
+    CK(cudaGetLastError());
+}
+void launch_splice_used(const SpliceRuns& r, const u8* tags, const i64* pay8, const u32* pay4, u32* used, u64* class_mask, cudaStream_t s) {
+    if (r.nrows == 0) return;
+    k_splice_used<<<sgrid(r.nrows, SPLICE_TILE), SPLICE_TILE, 0, s>>>(r.new_lo, r.src_lo, r.nruns, r.nrows, tags, pay8, pay4, used, class_mask);
+    g_launches.fetch_add(1);
+    CK(cudaGetLastError());
+}
+void launch_splice_gather(const SpliceRuns& r, i64 padded, const u8* o_tags, const i64* o_pay8, const u32* o_pay4, const u32* o_remap,
+                          const u8* p_tags, const i64* p_pay8, const u32* p_pay4, const u32* p_remap, u8* tags, i64* pay8, u32* pay4, cudaStream_t s) {
+    k_splice_gather<<<sgrid(padded, SPLICE_TILE), SPLICE_TILE, 0, s>>>(r.new_lo, r.src_lo, r.nruns, r.nrows, padded, o_tags, o_pay8, o_pay4, o_remap,
+                                                                      p_tags, p_pay8, p_pay4, p_remap, tags, pay8, pay4);
     g_launches.fetch_add(1);
     CK(cudaGetLastError());
 }

@@ -32,4 +32,14 @@ void launch_col_stats(const u8* tags, const i64* payload, i64 nrows, u64* stats,
 void launch_canon_floats(u8* tags, i64* payload, i64 nrows, cudaStream_t s);
 void launch_patch(u8* tags, i64* payload, const i64* rows, const u8* ptags, const i64* ppay, i64 n, cudaStream_t s);
 
+// The row map of a spliced column, in device memory: run k covers new rows [new_lo[k], new_lo[k + 1]) (new_lo[nruns] = nrows)
+// and reads them from row src_lo[k] on of the old column, or of the patch column when bit 63 of src_lo[k] is set.
+struct SpliceRuns { const i64* new_lo; const i64* src_lo; i64 nruns, nrows; };
+// ranks of the old dictionary used by the kept rows (a bitmap of ceil(ndict / 32) words, zeroed by the caller) and the
+// classes of those rows (OR-ed into *class_mask)
+void launch_splice_used(const SpliceRuns& r, const u8* tags, const i64* pay8, const u32* pay4, u32* used, u64* class_mask, cudaStream_t s);
+// writes all `padded` rows of the new column; a source or target payload pointer is null at that width (0: no payload)
+void launch_splice_gather(const SpliceRuns& r, i64 padded, const u8* o_tags, const i64* o_pay8, const u32* o_pay4, const u32* o_remap,
+                          const u8* p_tags, const i64* p_pay8, const u32* p_pay4, const u32* p_remap, u8* tags, i64* pay8, u32* pay4, cudaStream_t s);
+
 }  // namespace n1

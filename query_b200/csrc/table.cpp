@@ -15,6 +15,7 @@
 #include <unistd.h>
 
 #include <algorithm>
+#include <cerrno>
 #include <chrono>
 #include <fstream>
 #include <thread>
@@ -273,7 +274,17 @@ void Table::append_json(const char* buf, const i64* offsets, i64 ndocs, int thre
     shred_sec += now_sec() - t0;
 }
 
-void Table::load_dir(const std::string& dir, int threads) {
+DocFp DocFp::of(const struct stat& st) {
+    DocFp f;
+    f.state = DOC;
+    f.ino = (u64)st.st_ino;
+    f.size = (i64)st.st_size;
+    f.mtime_ns = (i64)st.st_mtim.tv_sec * 1000000000 + st.st_mtim.tv_nsec;
+    f.ctime_ns = (i64)st.st_ctim.tv_sec * 1000000000 + st.st_ctim.tv_nsec;
+    return f;
+}
+
+void Table::load_dir(const std::string& dir, int threads, std::vector<std::string>* entries, std::vector<DocFp>* fps) {
     DIR* d = opendir(dir.c_str());
     if (!d) N1_THROW(N1GPU_E_IO, "cannot open keyspace directory %s", dir.c_str());
     std::vector<std::string> names;
@@ -289,15 +300,23 @@ void Table::load_dir(const std::string& dir, int threads) {
     }
     closedir(d);
     std::sort(names.begin(), names.end());  // ioutil.ReadDir order
+    if (entries) *entries = names;
+    load_entries(dir, names, threads, fps);
+}
+
+std::string document_file(const std::string& entry) {
     // The primary index scans IDS, not files: every non-directory entry yields the id "name minus its last extension"
     // (documentPathToId, file.go:757-761), and Fetch reads <id>.json (file.go:346) - a missing file is silently no document
     // (file.go:319-322), an unreadable one is an error the request reports while it carries on.  So foo.txt is a document only
     // if foo.json exists (and a.json + a.txt are TWO rows of a.json), .DS_Store and editor backups are none.
-    for (auto& n : names) {
-        const size_t dot = n.rfind('.');
-        if (dot != std::string::npos) n.resize(dot);
-        n += ".json";
-    }
+    const size_t dot = entry.rfind('.');
+    return (dot == std::string::npos ? entry : entry.substr(0, dot)) + ".json";
+}
+
+void Table::load_entries(const std::string& dir, const std::vector<std::string>& entries, int threads, std::vector<DocFp>* fps) {
+    std::vector<std::string> names(entries.size());
+    for (size_t i = 0; i < entries.size(); ++i) names[i] = document_file(entries[i]);
+    if (fps) fps->assign(names.size(), DocFp());
     // The reference opens and reads one file per document, serially (file.go:732-743).  Here the reads of contiguous
     // ranges of the sorted names run on all cores - they are system calls on (mostly cached) small files - and the
     // documents are then laid end to end in primary-key order for the shredder.
@@ -315,11 +334,16 @@ void Table::load_dir(const std::string& dir, int threads) {
         for (size_t i = lo; i < hi; ++i) {
             path.assign(dir).append("/").append(names[i]);
             const int fd = open(path.c_str(), O_RDONLY | O_CLOEXEC);
-            if (fd < 0) continue;  // ENOENT: the id denotes no document; anything else: the reference reports and continues
+            if (fd < 0) {  // ENOENT: the id denotes no document; anything else: the reference reports and continues
+                if (fps) (*fps)[i].state = errno == ENOENT ? DocFp::ABSENT : DocFp::UNREADABLE;
+                continue;
+            }
             const size_t before = part.bytes.size();
             size_t cap = 4096;
             struct stat st;
-            if (fstat(fd, &st) == 0 && st.st_size > 0) cap = (size_t)st.st_size + 1;
+            DocFp fp;
+            fp.racy = true;  // no fingerprint: read again at the next check
+            if (fstat(fd, &st) == 0) { fp = DocFp::of(st); if (st.st_size > 0) cap = (size_t)st.st_size + 1; }
             bool failed = false;
             for (;;) {
                 part.bytes.resize(part.bytes.size() + cap);
@@ -329,6 +353,8 @@ void Table::load_dir(const std::string& dir, int threads) {
                 if (got == 0) break;
             }
             close(fd);
+            fp.state = failed ? DocFp::UNREADABLE : DocFp::DOC;
+            if (fps) (*fps)[i] = fp;
             if (!failed) part.sizes.push_back((i64)(part.bytes.size() - before));
         }
     };

@@ -7,6 +7,8 @@
 #include <unordered_map>
 #include <vector>
 
+#include <sys/stat.h>
+
 #include "common.hpp"
 
 namespace n1 {
@@ -67,6 +69,26 @@ struct Column {
     bool device_set = false;             // filled by set_column_device
 };
 
+// What the file a directory entry's row is read from (<id>.json, file.go:711-749) looked like when it was read or
+// stat-ed: the refresh of a resident keyspace keeps the rows of entries whose fingerprint still holds.
+struct DocFp {
+    enum State : u8 { ABSENT, DOC, UNREADABLE };  // no such file / read (the entry has a row) / there but not readable
+    State state = ABSENT;
+    bool racy = false;  // changed too close to the read for its timestamps to tell: treated as changed at the next check
+    u64 ino = 0;
+    i64 size = 0, mtime_ns = 0, ctime_ns = 0;
+    static DocFp of(const struct stat& st);
+    // the entry's row (or its absence) is still what a read would give
+    bool holds(const DocFp& now) const {
+        if (state == ABSENT) return now.state == ABSENT;
+        return state == DOC && !racy && now.state == DOC && ino == now.ino && size == now.size && mtime_ns == now.mtime_ns && ctime_ns == now.ctime_ns;
+    }
+};
+
+// One row run of a spliced table: rows [new_lo, new_lo + len) come from rows [src_lo, src_lo + len) of the old table or
+// of the patch (the re-read documents).
+struct SpliceRun { i64 new_lo; bool patch; i64 src_lo, len; };
+
 struct Table {
     std::vector<Column> cols;
     i64 nrows = 0;
@@ -78,7 +100,8 @@ struct Table {
 
     // persistent segment (segment.cpp): when set, seal() writes the shredded columns to this file under this source tag
     std::string segment_out, segment_source;
-    void write_segment() const;
+    void write_segment() const { write_segment(segment_out, segment_source); }
+    void write_segment(const std::string& file, const std::string& source) const;
     bool load_segment(const std::string& file, const std::string& source);
     void load_ndjson(const std::string& file, int threads);  // one document per line; threads as for load_dir
 
@@ -93,7 +116,16 @@ struct Table {
     int add_column(const std::string& path);
     int find_column(const std::string& path) const;
     void append_json(const char* buf, const i64* offsets, i64 ndocs, int threads);
-    void load_dir(const std::string& dir, int threads);
+    // entries / fps (optional): the directory entries in primary-key order and the fingerprint of what each one was read
+    // from; the rows are those of the entries whose state is DOC, in that order
+    void load_dir(const std::string& dir, int threads, std::vector<std::string>* entries = nullptr, std::vector<DocFp>* fps = nullptr);
+    // the documents of the given directory entries (sorted names; <id>.json of each is read)
+    void load_entries(const std::string& dir, const std::vector<std::string>& entries, int threads, std::vector<DocFp>* fps);
+    // Fills this table (columns declared, nothing appended) with `runs` of rows of `old` and `patch` (null when no run
+    // reads it), both sealed with their columns in HBM.  Dictionaries, statistics and widths are those a load of the
+    // spliced rows gives.
+    void splice(const Table& old, const Table* patch, const std::vector<SpliceRun>& runs);
+    double splice_sec = 0;
     void set_column(int col, int width, const void* payload, const u8* tags, i64 nrows, const char* blob,
                     const i64* offs, i64 ndict);
     // The same for a column that already lives in device memory (caller-owned device pointers, copied device to
@@ -120,6 +152,9 @@ struct HostShredOut {
 };
 void host_shred_docs(const std::vector<Column>& cols, const char* buf, const i64* offs, const i64* rows, i64 n,
                      std::vector<HostShredOut>& out);
+
+// The file a keyspace directory entry's row is read from: <name minus its last extension>.json (file.go:757-761, 346).
+std::string document_file(const std::string& entry);
 
 std::vector<std::string> split_path(const std::string& path);
 std::string join_path(const std::vector<std::string>& p, char sep);

@@ -427,6 +427,104 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
     shred_sec += now_sec() - t0;
 }
 
+void Table::splice(const Table& old, const Table* patch, const std::vector<SpliceRun>& runs) {
+    if (!have_device()) N1_THROW(N1GPU_E_CUDA, "splicing columns needs a CUDA device");
+    if (sealed || appended || nrows) N1_THROW(N1GPU_E_INVALID, "a splice fills an empty, unsealed table");
+    if (old.cols.size() != cols.size() || (patch && patch->cols.size() != cols.size())) N1_THROW(N1GPU_E_INVALID, "splice sources have other columns");
+    const double t0 = now_sec();
+    const size_t R = runs.size();
+    std::vector<i64> h_runs(2 * R + 1);  // new_lo[0..R], then src_lo[0..R)
+    for (size_t k = 0; k < R; ++k) {
+        const SpliceRun& r = runs[k];
+        const Table* src = r.patch ? patch : &old;
+        if (!src || r.len <= 0 || r.src_lo < 0 || r.src_lo + r.len > src->nrows || r.new_lo != (k ? h_runs[k - 1] + runs[k - 1].len : 0))
+            N1_THROW(N1GPU_E_INVALID, "splice run %zu does not follow its sources", k);
+        h_runs[k] = r.new_lo;
+        h_runs[R + 1 + k] = (i64)((u64)r.src_lo | (r.patch ? 0x8000000000000000ULL : 0));
+    }
+    nrows = R ? runs.back().new_lo + runs.back().len : 0;
+    h_runs[R] = nrows;
+    i64 pad = padded_rows();
+    if (pad == 0) pad = ROW_PAD;
+    cudaStream_t s = nullptr;
+    CK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamDestroy(s); } } sg{s};
+    DevBuf d_runs, d_used, d_stats, d_oremap, d_premap;
+    d_runs.alloc(h_runs.size() * 8);
+    CK(cudaMemcpyAsync(d_runs.p, h_runs.data(), h_runs.size() * 8, cudaMemcpyHostToDevice, s));
+    const SpliceRuns sr{d_runs.as<i64>(), d_runs.as<i64>() + R + 1, (i64)R, nrows};
+    d_stats.alloc(64);
+    auto pay8 = [](const Column& c) { return c.width == 8 ? c.d_payload.as<i64>() : nullptr; };
+    auto pay4 = [](const Column& c) { return c.width == 4 ? c.d_payload.as<u32>() : nullptr; };
+    for (size_t c = 0; c < cols.size(); ++c) {
+        const Column& oc = old.cols[c];
+        const Column* pc = patch ? &patch->cols[c] : nullptr;
+        Column& col = cols[c];
+        // the old ranks the kept rows still use, and the classes of those rows
+        const size_t words = (oc.dict.size() + 31) / 32, mask_at = (words * 4 + 7) / 8 * 8;  // bitmap, then the class mask
+        d_used.ensure(mask_at + 8);
+        CK(cudaMemsetAsync(d_used.p, 0, mask_at + 8, s));
+        u64* d_mask = (u64*)((char*)d_used.p + mask_at);
+        launch_splice_used(sr, oc.d_tags.as<u8>(), pay8(oc), pay4(oc), d_used.as<u32>(), d_mask, s);
+        std::vector<u32> used(words);
+        u64 mask = 0;
+        if (words) CK(cudaMemcpyAsync(used.data(), d_used.p, words * 4, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(&mask, d_mask, 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        if (pc) mask |= pc->stats.class_mask;
+        // new dictionary: the used old strings and the patch's, sorted and unique; both inputs are sorted, so one merge walk
+        // gives the new rank of every old and every patch rank
+        const std::vector<std::string>& od = oc.dict.vec();
+        static const std::vector<std::string> none;
+        const std::vector<std::string>& pd = pc ? pc->dict.vec() : none;
+        std::vector<u32> oremap(od.size(), 0), premap(pd.size(), 0);
+        std::vector<std::string> dict;
+        dict.reserve(pd.size() + od.size());
+        size_t i = 0, j = 0;
+        auto next_used = [&](size_t from) { while (from < od.size() && !((used[from >> 5] >> (from & 31)) & 1u)) ++from; return from; };
+        i = next_used(0);
+        while (i < od.size() || j < pd.size()) {
+            const bool take_old = j == pd.size() || (i < od.size() && od[i] <= pd[j]);
+            const bool take_patch = i == od.size() || (j < pd.size() && pd[j] <= od[i]);
+            const u32 rank = (u32)dict.size();
+            dict.push_back(take_old ? od[i] : pd[j]);
+            if (take_old) { oremap[i] = rank; i = next_used(i + 1); }
+            if (take_patch) premap[j++] = rank;
+        }
+        col.dict = std::move(dict);
+        col.width = (mask & M_NUM) ? 8 : ((mask & bit(C_STRING)) ? 4 : 0);
+        d_oremap.ensure(std::max<size_t>(oremap.size() * 4, 64));
+        d_premap.ensure(std::max<size_t>(premap.size() * 4, 64));
+        if (!oremap.empty()) CK(cudaMemcpyAsync(d_oremap.p, oremap.data(), oremap.size() * 4, cudaMemcpyHostToDevice, s));
+        if (!premap.empty()) CK(cudaMemcpyAsync(d_premap.p, premap.data(), premap.size() * 4, cudaMemcpyHostToDevice, s));
+        col.d_tags.alloc((size_t)pad);
+        col.d_payload.alloc(col.width ? (size_t)pad * (size_t)col.width : 256);
+        launch_splice_gather(sr, pad, oc.d_tags.as<u8>(), pay8(oc), pay4(oc), d_oremap.as<u32>(), pc ? pc->d_tags.as<u8>() : nullptr,
+                             pc ? pay8(*pc) : nullptr, pc ? pay4(*pc) : nullptr, d_premap.as<u32>(), col.d_tags.as<u8>(), pay8(col), pay4(col), s);
+        // statistics of the spliced column, as the device shredder computes them
+        u64 h_stats[8] = {0, (u64)INT64_MAX, (u64)INT64_MIN, 0, 0, 0, 0, 0};
+        CK(cudaMemcpyAsync(d_stats.p, h_stats, 64, cudaMemcpyHostToDevice, s));
+        if (nrows) launch_col_stats(col.d_tags.as<u8>(), pay8(col), nrows, d_stats.as<u64>(), s);
+        CK(cudaMemcpyAsync(h_stats, d_stats.p, 64, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        ColumnStats st;
+        st.class_mask = (u32)h_stats[0];
+        st.has_int = (st.class_mask & bit(C_INT)) != 0;
+        st.int_min = st.has_int ? (i64)h_stats[1] : 0;
+        st.int_max = st.has_int ? (i64)h_stats[2] : 0;
+        st.has_float = h_stats[3] != 0;
+        st.absent_rows = (i64)h_stats[4];
+        st.ndict = (i64)col.dict.size();
+        st.empty_rank = (!col.dict.empty() && col.dict[0].empty()) ? 0 : -1;
+        col.stats = st;
+        col.codes_are_ranks = true;
+    }
+    appended = true;
+    device_shredded = true;
+    sealed = true;
+    splice_sec += now_sec() - t0;
+}
+
 void Table::remap_ranks_device(int ci, const std::vector<u32>& remap) {
     Column& c = cols[(size_t)ci];
     DevBuf d_map;
