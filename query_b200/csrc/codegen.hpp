@@ -66,6 +66,8 @@ struct KernelPlan {
     // A COUNT(x) counter over a column whose values are mostly present counts the rows where x is MISSING / NULL instead
     // (the rarer event: fewer shared-memory atomics per row); finalize() reads it as rows-in-group minus the word.
     std::vector<bool> word_complement;
+    std::vector<int> complement_agg;     // complemented word -> the aggregate whose (plain column) operand it counts
+    int w_rows = -1;                     // the rows-per-group word (-1: none)
     std::vector<PackComp> keys;
     int key_bits = 0;
     i64 dense_slots = 0;
@@ -76,6 +78,7 @@ struct KernelPlan {
                                  // key, no key array, no probing) behind the shared-memory front cache of the hash mode
     bool dense_priv = false;     // tiny dense table: one private copy per THREAD in shared memory (no atomics at all)
     bool pdl = false;            // launched with programmatic stream serialization (ungrouped scans)
+    int min_blocks = 0;          // resident blocks per SM in __launch_bounds__ (0: none)
     int dyn_smem = 0;            // dynamic shared memory the kernel is launched with
     int block = 256;             // threads per block (a block scans block * 4 rows per iteration)
     bool cache_key32 = false;    // front-cache keys are u32, direct-mapped (packed key <= 31 bits)
@@ -88,6 +91,7 @@ struct KernelPlan {
     int cache_n32 = 0, cache_n64 = 0;
     std::vector<AggPlan> aggs;
     int ndistinct = 0, abits = 0, entry_bits = 0;
+    std::vector<bool> set_any;   // DISTINCT entry set -> holds every value > NULL (else numbers only)
     bool set128 = false;
     int set_passes = 1;          // bitmap beyond what the L2 keeps: scan passes, each filling one L2-resident slice of it
     bool set_bitmap = false;     // DISTINCT entries are few bits: the set is a bitmap indexed by the entry (no hashing)
