@@ -12,6 +12,11 @@
 
 using namespace n1;
 
+// the public class codes are the value classes of n1ql_value.cuh
+static_assert(N1GPU_C_MISSING == C_MISSING && N1GPU_C_NULL == C_NULL && N1GPU_C_FALSE == C_FALSE && N1GPU_C_TRUE == C_TRUE &&
+                  N1GPU_C_INT == C_INT && N1GPU_C_FLOAT == C_FLOAT && N1GPU_C_STRING == C_STRING && N1GPU_C_OTHER == C_OTHER,
+              "N1GPU_C_* differ from the value classes");
+
 struct n1gpu_table { Table t; };
 struct n1gpu_query { std::unique_ptr<Query> q; };
 struct n1gpu_result { std::unique_ptr<Result> r; };

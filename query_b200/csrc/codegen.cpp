@@ -43,9 +43,6 @@ const char* cls_name(int c) {
     return n[c];
 }
 
-// the INSET_* flags of n1ql_device.cuh
-enum : u32 { INSET_MISSING = 1, INSET_NULL = 2, INSET_VALUED = 4, INSET_FALSE = 8, INSET_TRUE = 16, INSET_IEMPTY = 32, INSET_P63 = 64 };
-
 // open-addressing table of `keys` at load <= 0.25 (short clusters: a warp waits for its longest probe), probed like
 // inset_probe (n1ql_device.cuh)
 std::vector<u64> inset_table(std::vector<u64> keys) {
@@ -57,7 +54,7 @@ std::vector<u64> inset_table(std::vector<u64> keys) {
     if (cap > ((u64)1 << 31)) N1_THROW(N1GPU_E_INELIGIBLE, "IN list of %zu numbers", keys.size());
     std::vector<u64> tab(cap, ~(u64)0);
     for (u64 k : keys) {
-        u64 s = ((u32)((u32)k ^ (u32)(k >> 32)) * 0x9E3779B1u) >> (1 + __builtin_clz((u32)cap));  // inset_slot
+        u64 s = inset_slot(k, (u32)cap);
         while (tab[s] != ~(u64)0) s = (s + 1) & (cap - 1);
         tab[s] = k;
     }
@@ -245,7 +242,7 @@ struct Gen {
                     int k;
                     if (it != in_set_of.end()) k = it->second;
                     else {
-                        if ((int)in_sets.size() >= MAX_IN_SETS) N1_THROW(N1GPU_E_INELIGIBLE, "more than %d IN sets in one chain", MAX_IN_SETS);
+                        if ((int)in_sets.size() >= NQ_MAX_INSETS) N1_THROW(N1GPU_E_INELIGIBLE, "more than %d IN sets in one chain", NQ_MAX_INSETS);
                         k = (int)in_sets.size();
                         in_sets.push_back(build_inset(t, list, str_opnd ? e.ops[0]->ti.dict_col : -1));
                         in_set_of[&e] = k;

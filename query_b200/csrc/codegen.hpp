@@ -33,13 +33,13 @@ struct PackComp {
     int bits() const { return cbits + pbits; }
 };
 
-// IN evaluated through a device-resident set (NqInSet, n1ql_device.cuh) instead of one in_arg per element: see
+// IN evaluated through a device-resident set (NqInSet, n1ql_value.cuh) instead of one in_arg per element: see
 // in_takes_set (expr.hpp).  The kernel text names only the set's slot, so every binding of a statement shares one cubin.
-constexpr int MAX_IN_SETS = 8;  // NQ_MAX_INSETS
+// A chain has at most NQ_MAX_INSETS of them.
 struct InSet {
     std::vector<u32> bits;         // STRING: bitmap over the operand column's dictionary ranks
     std::vector<u64> ikeys, fkeys; // INT / FLOAT hash tables (all ones = empty slot)
-    u32 flags = 0;                 // INSET_* of n1ql_device.cuh
+    u32 flags = 0;                 // INSET_*
 };
 
 // One aggregate: what finalises it (FinalAgg, final_group.hpp) and what only the code generator needs

@@ -17,8 +17,6 @@
 
 namespace n1 {
 
-enum : int { OP_ADD_U64 = 0, OP_ADD_F64 = 1, OP_MIN_I64 = 2, OP_MAX_I64 = 3, OP_MIN_U64 = 4, OP_MAX_U64 = 5, OP_OR_U64 = 6 };
-
 inline u32 bit(int c) { return 1u << c; }
 const u32 M_NUM = (1u << C_INT) | (1u << C_FLOAT);
 const u32 M_BOOL = (1u << C_FALSE) | (1u << C_TRUE);
@@ -55,7 +53,7 @@ struct HValue {
     i64 bits = 0;
     std::string s;
     HValue() = default;
-    HValue(FinalVal v) : cls((u8)v.cls), bits(v.bits) {}  // a number from final_group.hpp (new_num)
+    HValue(Val v) : cls((u8)v.c), bits(v.b) {}  // a value of n1ql_value.cuh (no string bytes)
     static HValue missing() { return HValue(); }
     static HValue null() { HValue v; v.cls = C_NULL; return v; }
     static HValue boolean(bool b) { HValue v; v.cls = b ? C_TRUE : C_FALSE; return v; }
@@ -108,9 +106,6 @@ struct PinnedBuf {
     template <class T> T* as() const { return (T*)p; }
 };
 
-inline u64 mix64(u64 x) {
-    x ^= x >> 30; x *= 0xbf58476d1ce4e5b9ULL; x ^= x >> 27; x *= 0x94d049bb133111ebULL; x ^= x >> 31; return x;
-}
 inline int bits_for(u64 n_values) {  // bits to represent values 0..n_values-1
     int b = 0;
     while (b < 64 && ((u64)1 << b) < n_values) ++b;

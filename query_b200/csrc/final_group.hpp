@@ -12,46 +12,12 @@
 //   execution/group_final.go:55-118   one item per group
 #pragma once
 #include <cstdint>
-#include <cstring>
 
-#ifdef __CUDACC__
-#define N1_HD __host__ __device__ __forceinline__
-#else
-#define N1_HD inline
-#endif
+#include "n1ql_value.cuh"
 
 namespace n1 {
 
-typedef long long i64;           // same types as the device library (n1ql_device.cuh)
-typedef unsigned long long u64;
-typedef uint32_t u32;
-typedef uint8_t u8;
-
-enum : int { C_MISSING = 0, C_NULL = 1, C_FALSE = 2, C_TRUE = 3, C_INT = 4, C_FLOAT = 5, C_STRING = 6, C_OTHER = 7 };
-
 enum class AggKind : signed char { COUNT, COUNTN, SUM, AVG, MIN, MAX };
-
-// A result value: class + payload (the INT, the FLOAT's bits, a string as dictionary column << 40 | rank)
-struct FinalVal {
-    int cls;
-    i64 bits;
-};
-
-N1_HD double as_f64(u64 b) { double d; memcpy(&d, &b, 8); return d; }
-N1_HD FinalVal flt_val(double d) { FinalVal v{C_FLOAT, 0}; memcpy(&v.bits, &d, 8); return v; }
-N1_HD double num_of(FinalVal v) { return v.cls == C_INT ? (double)v.bits : as_f64((u64)v.bits); }
-
-// Go's int64(float64) on amd64 and value.IsInt (value/integer.go:354-356)
-N1_HD i64 go_i64(double d) {
-    if (!(d >= -9223372036854775808.0 && d < 9223372036854775808.0)) return INT64_MIN;
-    return (i64)d;
-}
-N1_HD bool f_is_int(double d) { return d == (double)go_i64(d); }
-// value.NewValue(float64) (value/value.go:377-382)
-N1_HD FinalVal new_num(double d) { return f_is_int(d) ? FinalVal{C_INT, go_i64(d)} : flt_val(d); }
-
-// inverse of f64_ordered (n1ql_device.cuh): the float a MIN / MAX word holds
-N1_HD double f64_unordered(u64 k) { return as_f64((k >> 63) ? (k & 0x7fffffffffffffffULL) : ~k); }
 
 // One bit-packed component (PackComp as plain data): a group-key value or the value of a DISTINCT entry
 struct FinalComp {
@@ -101,7 +67,7 @@ N1_HD u64 take_bits(unsigned __int128& v, int n) {
 }
 
 // the next component of a packed key or DISTINCT entry
-N1_HD FinalVal decode_comp(const FinalComp& pc, unsigned __int128& bits) {
+N1_HD Val decode_comp(const FinalComp& pc, unsigned __int128& bits) {
     u64 ci = take_bits(bits, pc.cbits);
     u64 pv = take_bits(bits, pc.pbits);
     if (pc.nfree >= 0) {  // offset packing: one field
@@ -129,20 +95,20 @@ N1_HD void logical_words(const FinalDesc& D, const u64* pw, u64* w) {
 }
 
 // the SUM value as the reference's NumberValue chain would leave it (see the header comment)
-N1_HD FinalVal sum_value(__int128 itotal, u64 n_nonneg, u64 n_neg, u64 n_flt, double fsum, bool from_zero) {
+N1_HD Val sum_value(__int128 itotal, u64 n_nonneg, u64 n_neg, u64 n_flt, double fsum, bool from_zero) {
     const u64 nI = n_nonneg + n_neg;
     if (nI + n_flt == 0) return {C_NULL, 0};
     if (n_flt == 0) {
         const bool same_sign = from_zero ? (n_neg == 0) : (n_neg == 0 || n_nonneg == 0);
         if (same_sign && itotal >= (__int128)INT64_MIN && itotal <= (__int128)INT64_MAX) return {C_INT, (i64)itotal};
-        return flt_val((double)itotal);
+        return mkflt((double)itotal);
     }
-    if (nI == 0) return flt_val(fsum);
-    return flt_val((double)itotal + fsum);
+    if (nI == 0) return mkflt(fsum);
+    return mkflt((double)itotal + fsum);
 }
 
 // ComputeFinal of one aggregate from the group's logical words
-N1_HD FinalVal final_agg(const FinalAgg& ap, const u64* w) {
+N1_HD Val final_agg(const FinalAgg& ap, const u64* w) {
     if (ap.distinct) {
         const u64 count = w[ap.w_cnt];
         if (ap.kind == AggKind::COUNT || ap.kind == AggKind::COUNTN) return {C_INT, (i64)count};
@@ -153,18 +119,18 @@ N1_HD FinalVal final_agg(const FinalAgg& ap, const u64* w) {
         if (ap.w_ilo >= 0) itotal = (((__int128)(i64)w[ap.w_ihi]) << 32) + (__int128)w[ap.w_ilo];
         if (ap.w_neg >= 0) n_neg = w[ap.w_neg];
         if (ap.w_nflt >= 0) n_flt = w[ap.w_nflt];
-        if (ap.w_fsum >= 0) fsum = as_f64(w[ap.w_fsum]);
-        const FinalVal sv = sum_value(itotal, count - n_neg - n_flt, n_neg, n_flt, fsum, true);
-        return ap.kind == AggKind::SUM ? sv : new_num(num_of(sv) / (double)count);
+        if (ap.w_fsum >= 0) fsum = as_f((i64)w[ap.w_fsum]);
+        const Val sv = sum_value(itotal, count - n_neg - n_flt, n_neg, n_flt, fsum, true);
+        return ap.kind == AggKind::SUM ? sv : new_num(num_f(sv) / (double)count);
     }
     if (ap.kind == AggKind::COUNT || ap.kind == AggKind::COUNTN) return {C_INT, (i64)w[ap.w_cnt]};
     if (ap.fcarry) {
         const u64 count = w[ap.w_nnum], flags = (w[ap.w_flags] >> ap.flag_shift) & 7;
-        const double fs = as_f64(w[ap.w_fsum]);
+        const double fs = as_f((i64)w[ap.w_fsum]);
         if (count == 0) return {C_NULL, 0};
         // a float, or ints of both signs (intValue.Add went float): float; else the exact int total
-        const FinalVal sv = ((flags & 1) || ((flags & 2) && (flags & 4))) ? flt_val(fs) : FinalVal{C_INT, (i64)fs};
-        return ap.kind == AggKind::SUM ? sv : new_num(num_of(sv) / (double)count);
+        const Val sv = ((flags & 1) || ((flags & 2) && (flags & 4))) ? mkflt(fs) : Val{C_INT, (i64)fs};
+        return ap.kind == AggKind::SUM ? sv : new_num(num_f(sv) / (double)count);
     }
     if (ap.kind == AggKind::SUM || ap.kind == AggKind::AVG) {
         __int128 itotal = 0;
@@ -180,10 +146,10 @@ N1_HD FinalVal final_agg(const FinalAgg& ap, const u64* w) {
             n_nonneg = w[ap.w_nint] - n_neg;
         }
         if (ap.w_nflt >= 0) n_flt = w[ap.w_nflt];
-        if (ap.w_fsum >= 0) fsum = as_f64(w[ap.w_fsum]);
-        const FinalVal sv = sum_value(itotal, n_nonneg, n_neg, n_flt, fsum, false);
-        if (ap.kind == AggKind::SUM || sv.cls == C_NULL) return sv;
-        return new_num(num_of(sv) / (double)(n_nonneg + n_neg + n_flt));
+        if (ap.w_fsum >= 0) fsum = as_f((i64)w[ap.w_fsum]);
+        const Val sv = sum_value(itotal, n_nonneg, n_neg, n_flt, fsum, false);
+        if (ap.kind == AggKind::SUM || sv.c == C_NULL) return sv;
+        return new_num(num_f(sv) / (double)(n_nonneg + n_neg + n_flt));
     }
     // MIN / MAX: the collation winner over the classes seen
     const bool mn = ap.kind == AggKind::MIN;
@@ -191,12 +157,12 @@ N1_HD FinalVal final_agg(const FinalAgg& ap, const u64* w) {
     const bool hi = seen & (1ULL << C_INT), hf = seen & (1ULL << C_FLOAT);
     const i64 iv = ap.w_mi >= 0 ? (i64)w[ap.w_mi] : 0;
     const double fv = ap.w_mf >= 0 ? f64_unordered(w[ap.w_mf]) : 0;
-    FinalVal number;
+    Val number;
     if (hi && hf) {  // intValue.Collate(floatValue): float64 compare (value/integer.go:100-118)
         const double ad = (double)iv;
-        number = (mn ? (ad <= fv) : (ad >= fv)) ? FinalVal{C_INT, iv} : flt_val(fv);
-    } else number = hi ? FinalVal{C_INT, iv} : flt_val(fv);
-    const FinalVal str{C_STRING, ap.w_ms >= 0 ? (i64)(((u64)ap.dict_col << 40) | (w[ap.w_ms] & 0xffffffffffULL)) : 0};
+        number = (mn ? (ad <= fv) : (ad >= fv)) ? Val{C_INT, iv} : mkflt(fv);
+    } else number = hi ? Val{C_INT, iv} : mkflt(fv);
+    const Val str{C_STRING, ap.w_ms >= 0 ? (i64)(((u64)ap.dict_col << 40) | (w[ap.w_ms] & 0xffffffffffULL)) : 0};
     const u64 M_NUMB = (1ULL << C_INT) | (1ULL << C_FLOAT);
     if (seen == 0) return {C_NULL, 0};
     if (mn) {
@@ -217,14 +183,14 @@ N1_HD void final_group(const FinalDesc& D, const FinalComp* keys, int nkeys, u64
     logical_words(D, pw, w);
     unsigned __int128 kb = ((unsigned __int128)khi << 64) | klo;
     for (int k = 0; k < nkeys; ++k) {
-        const FinalVal v = decode_comp(keys[k], kb);
-        key_cls[k] = (u8)v.cls;
-        key_val[k] = v.bits;
+        const Val v = decode_comp(keys[k], kb);
+        key_cls[k] = (u8)v.c;
+        key_val[k] = v.b;
     }
     for (int a = 0; a < D.naggs; ++a) {
-        const FinalVal v = final_agg(D.aggs[a], w);
-        agg_cls[a] = (u8)v.cls;
-        agg_val[a] = v.bits;
+        const Val v = final_agg(D.aggs[a], w);
+        agg_cls[a] = (u8)v.c;
+        agg_val[a] = v.b;
     }
 }
 

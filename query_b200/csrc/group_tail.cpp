@@ -1,6 +1,6 @@
-// group_tail.cpp — see group_tail.hpp.  The expression semantics restated here on host values are the ones
-// n1ql_device.cuh holds for the scan kernel (same reference lines); strings are compared bytewise as strings here,
-// where the kernel compares dictionary ranks.
+// group_tail.cpp — see group_tail.hpp.  Numbers, logic and the MISSING / NULL folds are the value model of
+// n1ql_value.cuh, the one the scan kernel runs, applied to the (class, payload) of host values.  Only strings differ:
+// here they are compared and tested for truth as bytes, where the kernel compares dictionary ranks.
 #include "group_tail.hpp"
 
 #include <algorithm>
@@ -14,75 +14,22 @@ namespace execution {
 
 namespace {
 
-bool is_num(const HValue& v) { return v.cls == C_INT || v.cls == C_FLOAT; }
-int type_rank(int c) { return c <= C_NULL ? c : (c <= C_TRUE ? 2 : (c <= C_FLOAT ? 3 : 4)); }
 HValue missing() { return HValue::missing(); }
 HValue null() { return HValue::null(); }
 
-int collate_f(double t, double o) {  // value/float.go:123-172: NaN sorts first
-    const bool tn = t != t, on = o != o;
-    if (tn) return on ? 0 : -1;
-    if (on) return 1;
-    return t < o ? -1 : (t > o ? 1 : 0);
-}
+// A host value as n1ql_value.cuh sees it.  A string's payload says only whether it is non-empty, which is all that
+// v_truth (with empty2 = 0) reads of it: comparisons of two strings are made on the bytes (str_cmp below).
+Val val(const HValue& v) { return mkv(v.cls, v.cls == C_STRING ? (i64)!v.s.empty() : v.bits); }
+bool both_strings(const HValue& a, const HValue& b) { return a.cls == C_STRING && b.cls == C_STRING; }
+int str_cmp(const HValue& a, const HValue& b) { const int c = a.s.compare(b.s); return c < 0 ? -1 : (c > 0 ? 1 : 0); }
 
-enum { CMP_NULL = 8, CMP_MISSING = 9 };
 int compare(const HValue& a, const HValue& b) {  // Value.Compare
-    if (a.cls == C_MISSING || b.cls == C_MISSING) return CMP_MISSING;
-    if (a.cls == C_NULL || b.cls == C_NULL) return CMP_NULL;
-    const int c = collate_values(a, b);
-    return c < 0 ? -1 : (c > 0 ? 1 : 0);
+    return both_strings(a, b) ? str_cmp(a, b) : v_compare(val(a), val(b));
 }
-HValue cmp_result(int c, bool t) { return c == CMP_MISSING ? missing() : (c == CMP_NULL ? null() : HValue::boolean(t)); }
-
-HValue v_eq(const HValue& a, const HValue& b) {  // Value.Equals (comp_eq.go:76-78)
-    if (a.cls == C_MISSING || b.cls == C_MISSING) return missing();
-    if (a.cls == C_NULL || b.cls == C_NULL) return null();
-    const int ra = type_rank(a.cls), rb = type_rank(b.cls);
-    if (ra != rb) return HValue::boolean(false);
-    if (ra == 3) {
-        if (a.cls == C_INT && b.cls == C_INT) return HValue::boolean(a.bits == b.bits);
-        return HValue::boolean(a.num() == b.num());
-    }
-    if (ra == 2) return HValue::boolean(a.cls == b.cls);
-    return HValue::boolean(a.s == b.s);
+HValue eq(const HValue& a, const HValue& b) {  // Value.Equals (comp_eq.go:76-78)
+    return both_strings(a, b) ? HValue::boolean(a.s == b.s) : HValue(v_eq(val(a), val(b)));
 }
-
-bool truth(const HValue& v) {  // Value.Truth
-    switch (v.cls) {
-        case C_TRUE: return true;
-        case C_INT: return v.bits != 0;
-        case C_FLOAT: { const double d = v.f(); return d == d && d != 0.0; }
-        case C_STRING: return !v.s.empty();
-        default: return false;
-    }
-}
-
-HValue num_add(const HValue& a, const HValue& b) {  // integer.go:266-277, float.go:331-333
-    if (a.cls == C_INT && b.cls == C_INT) {
-        const i64 rv = (i64)((u64)a.bits + (u64)b.bits);
-        if ((a.bits >= 0 && b.bits >= 0 && rv >= 0) || (a.bits < 0 && b.bits < 0 && rv < 0)) return HValue::integer(rv);
-    }
-    return HValue::flt(a.num() + b.num());
-}
-HValue num_mult(const HValue& a, const HValue& b) {  // integer.go:319-329
-    if (a.cls == C_INT && b.cls == C_INT) {
-        const __int128 p = (__int128)a.bits * (__int128)b.bits;
-        bool ok = p >= (__int128)INT64_MIN && p <= (__int128)INT64_MAX;
-        if (a.bits == -1 && b.bits == INT64_MIN) ok = true;  // rv / this == n holds for the wrapped product
-        if (a.bits == INT64_MIN && b.bits == -1) ok = false;
-        if (ok) return HValue::integer((i64)((u64)a.bits * (u64)b.bits));
-    }
-    return HValue::flt(a.num() * b.num());
-}
-HValue num_neg(const HValue& a) {  // integer.go:331-337
-    if (a.cls == C_INT) return a.bits == INT64_MIN ? HValue::flt(-(double)a.bits) : HValue::integer(-a.bits);
-    return HValue::flt(-a.f());
-}
-HValue num_sub(const HValue& a, const HValue& b) {  // integer.go:339-348
-    if (a.cls == C_INT && b.cls == C_INT && b.bits > INT64_MIN) return num_add(a, HValue::integer(-b.bits));
-    return HValue::flt(a.num() - b.num());
-}
+bool truth(const HValue& v) { return v_truth(val(v), 0); }  // Value.Truth
 
 // What an expression node of the tail resolves to, decided once at add() time.
 enum { R_EVAL = 0, R_KEY = 1, R_AGG = 2, R_LET = 3, R_ALIAS = 4 };
@@ -151,35 +98,19 @@ HValue eval(const Expr& e, const Env& env) {
     switch (e.kind) {
         case EK::CONST: return e.cval;
         case EK::ADD: case EK::MULT: {  // arith_add.go:51-70, arith_mult.go:51-70
-            HValue acc = HValue::integer(e.kind == EK::ADD ? 0 : 1);
+            Val acc = mkint(e.kind == EK::ADD ? 0 : 1);
             bool m = false, n = false;
             for (auto& o : e.ops) {
-                const HValue a = eval(*o, env);
-                if (!n && is_num(a)) acc = e.kind == EK::ADD ? num_add(acc, a) : num_mult(acc, a);
-                else if (a.cls == C_MISSING) m = true;
-                else n = true;
+                const Val a = val(eval(*o, env));
+                if (e.kind == EK::ADD) add_arg(a, acc, m, n); else mult_arg(a, acc, m, n);
             }
-            return m ? missing() : (n ? null() : acc);
+            return arith_fin(acc, m, n);
         }
-        case EK::SUB: case EK::DIV: case EK::MOD: {
-            const HValue a = eval(*e.ops[0], env), b = eval(*e.ops[1], env);
-            if (e.kind == EK::SUB) {  // arith_sub.go:53-61
-                if (is_num(a) && is_num(b)) return num_sub(a, b);
-                return (a.cls == C_MISSING || b.cls == C_MISSING) ? missing() : null();
-            }
-            if (a.cls == C_MISSING || b.cls == C_MISSING) return missing();  // arith_div.go:46-64, arith_mod.go:48-66
-            if (is_num(b)) {
-                const double s = b.num();
-                if (s == 0.0) return null();
-                if (is_num(a)) return new_num(e.kind == EK::DIV ? a.num() / s : std::fmod(a.num(), s));
-            }
-            return null();
-        }
-        case EK::NEG: {
-            const HValue a = eval(*e.ops[0], env);
-            return is_num(a) ? num_neg(a) : (a.cls == C_MISSING ? a : null());
-        }
-        case EK::EQ: return v_eq(eval(*e.ops[0], env), eval(*e.ops[1], env));
+        case EK::SUB: return v_sub(val(eval(*e.ops[0], env)), val(eval(*e.ops[1], env)));
+        case EK::DIV: return v_div(val(eval(*e.ops[0], env)), val(eval(*e.ops[1], env)));
+        case EK::MOD: return v_mod(val(eval(*e.ops[0], env)), val(eval(*e.ops[1], env)));
+        case EK::NEG: return v_neg(val(eval(*e.ops[0], env)));
+        case EK::EQ: return eq(eval(*e.ops[0], env), eval(*e.ops[1], env));
         case EK::LT: { const int c = compare(eval(*e.ops[0], env), eval(*e.ops[1], env)); return cmp_result(c, c < 0); }
         case EK::LE: { const int c = compare(eval(*e.ops[0], env), eval(*e.ops[1], env)); return cmp_result(c, c <= 0); }
         case EK::BETWEEN: {  // comp_between.go:58-78
@@ -197,42 +128,30 @@ HValue eval(const Expr& e, const Env& env) {
             bool hit = false, m = false, n = false;
             for (auto& el : e.ops[1]->ops) {
                 const HValue ev = eval(*el, env);
-                if (x.cls > C_NULL && ev.cls > C_NULL) { if (v_eq(x, ev).cls == C_TRUE) hit = true; }
-                else if (ev.cls == C_MISSING) m = true;
-                else n = true;
+                if (both_strings(x, ev)) hit = hit || x.s == ev.s; else in_arg(val(x), val(ev), hit, m, n);
             }
-            if (x.cls == C_MISSING) return x;
-            return hit ? HValue::boolean(true) : (n ? null() : (m ? missing() : HValue::boolean(false)));
+            return in_fin(val(x), hit, m, n);
         }
         case EK::AND: {  // logic_and.go:64-88
             bool f = false, m = false, n = false;
-            for (auto& o : e.ops) {
-                const HValue a = eval(*o, env);
-                if (a.cls == C_NULL) n = true; else if (a.cls == C_MISSING) m = true; else if (!truth(a)) f = true;
-            }
-            return f ? HValue::boolean(false) : (m ? missing() : (n ? null() : HValue::boolean(true)));
+            for (auto& o : e.ops) and_arg(val(eval(*o, env)), 0, f, m, n);
+            return and_fin(f, m, n);
         }
         case EK::OR: {  // logic_or.go:98-122
             bool t = false, m = false, n = false;
-            for (auto& o : e.ops) {
-                const HValue a = eval(*o, env);
-                if (a.cls == C_NULL) n = true; else if (a.cls == C_MISSING) m = true; else if (truth(a)) t = true;
-            }
-            return t ? HValue::boolean(true) : (n ? null() : (m ? missing() : HValue::boolean(false)));
+            for (auto& o : e.ops) or_arg(val(eval(*o, env)), 0, t, m, n);
+            return or_fin(t, m, n);
         }
-        case EK::NOT: {  // logic_not.go:57-68
-            const HValue a = eval(*e.ops[0], env);
-            return a.cls <= C_NULL ? a : HValue::boolean(!truth(a));
-        }
+        case EK::NOT: return v_not(val(eval(*e.ops[0], env)), 0);  // logic_not.go:57-68
         case EK::ROUND: {  // expression/func_num.go:1304-1336 (Round.Apply) + :1715-1736 (roundFloat: half to even)
             const HValue a = eval(*e.ops[0], env);
             if (a.cls == C_MISSING) return a;
-            if (!is_num(a)) return null();
+            if (!is_num(a.cls)) return null();
             i64 prec = 0;
             if (e.ops.size() > 1) {
                 const HValue p = eval(*e.ops[1], env);
                 if (p.cls == C_MISSING) return p;
-                if (!is_num(p) || p.num() != std::trunc(p.num())) return null();
+                if (!is_num(p.cls) || p.num() != std::trunc(p.num())) return null();
                 prec = go_i64(p.num());  // Go: p = int(pf)
             }
             double x = a.num();
@@ -244,12 +163,12 @@ HValue eval(const Expr& e, const Env& env) {
             if (r == inter && std::fmod(r, 2.0) != 0) r -= 1;
             return new_num(sign * r / pw);
         }
-        case EK::IS_NULL: { const HValue a = eval(*e.ops[0], env); return a.cls == C_NULL ? HValue::boolean(true) : (a.cls == C_MISSING ? a : HValue::boolean(false)); }
-        case EK::IS_NOT_NULL: { const HValue a = eval(*e.ops[0], env); return a.cls == C_NULL ? HValue::boolean(false) : (a.cls == C_MISSING ? a : HValue::boolean(true)); }
-        case EK::IS_MISSING: return HValue::boolean(eval(*e.ops[0], env).cls == C_MISSING);
-        case EK::IS_NOT_MISSING: return HValue::boolean(eval(*e.ops[0], env).cls != C_MISSING);
-        case EK::IS_VALUED: return HValue::boolean(eval(*e.ops[0], env).cls > C_NULL);
-        case EK::IS_NOT_VALUED: return HValue::boolean(eval(*e.ops[0], env).cls <= C_NULL);
+        case EK::IS_NULL: return v_is_null(val(eval(*e.ops[0], env)));
+        case EK::IS_NOT_NULL: return v_is_not_null(val(eval(*e.ops[0], env)));
+        case EK::IS_MISSING: return v_is_missing(val(eval(*e.ops[0], env)));
+        case EK::IS_NOT_MISSING: return v_is_not_missing(val(eval(*e.ops[0], env)));
+        case EK::IS_VALUED: return v_is_valued(val(eval(*e.ops[0], env)));
+        case EK::IS_NOT_VALUED: return v_is_not_valued(val(eval(*e.ops[0], env)));
         default: break;
     }
     N1_THROW(N1GPU_E_INELIGIBLE, "expression %s cannot be evaluated over a group", e.str().c_str());
@@ -264,7 +183,7 @@ std::string expr_alias(const Expr& e) {
 
 bool integral_operand(const Expr& e, i64* out) {  // offset.go:53-72, limit.go:53-72: a number whose Trunc equals itself
     const HValue v = eval_constant(e);
-    if (!is_num(v)) return false;
+    if (!is_num(v.cls)) return false;
     const double d = v.num();
     if (std::trunc(d) != d) return false;
     *out = v.cls == C_INT ? v.bits : go_i64(d);
@@ -274,15 +193,7 @@ bool integral_operand(const Expr& e, i64* out) {  // offset.go:53-72, limit.go:5
 }  // namespace
 
 int collate_values(const HValue& a, const HValue& b) {
-    const int ra = type_rank(a.cls), rb = type_rank(b.cls);
-    if (ra != rb) return ra - rb;
-    if (ra == 3) {
-        if (a.cls == C_INT && b.cls == C_INT) return a.bits < b.bits ? -1 : (a.bits > b.bits ? 1 : 0);
-        return collate_f(a.num(), b.num());
-    }
-    if (ra == 2) return a.cls - b.cls;
-    if (ra == 4) { const int c = a.s.compare(b.s); return c < 0 ? -1 : (c > 0 ? 1 : 0); }
-    return 0;
+    return both_strings(a, b) ? str_cmp(a, b) : collate(val(a), val(b));
 }
 
 HValue eval_constant(const Expr& e) {

@@ -19,9 +19,12 @@
 
 namespace n1 {
 
-// n1ql_device.cuh embedded at build time (Makefile: device_src.inc)
+// n1ql_device.cuh and the n1ql_value.cuh it includes, embedded at build time (Makefile: device_src.inc, value_src.inc)
 static const char* k_device_header =
 #include "device_src.inc"
+    ;
+static const char* k_value_header =
+#include "value_src.inc"
     ;
 
 std::atomic<u64> g_launches{0};
@@ -162,7 +165,7 @@ std::string jit_compile_cubin(const std::string& source, std::string* log) {
     Nvrtc& rt = nvrtc();
     // Optional on-disk kernel cache (N1GPU_KERNEL_CACHE_DIR): NVRTC + ptxas cost 0.25-0.45 s per new query shape, which a
     // restarted server would otherwise pay again for every prepared statement.  The key covers everything the cubin
-    // depends on: generated source, device library, NVRTC version, target.
+    // depends on: generated source, device library and value model, NVRTC version, target.
     std::string cache_file;
     if (const char* dir = getenv("N1GPU_KERNEL_CACHE_DIR")) {
         if (*dir) {
@@ -170,6 +173,7 @@ std::string jit_compile_cubin(const std::string& source, std::string* log) {
             auto mix = [&](const char* p, size_t n) { for (size_t i = 0; i < n; ++i) { h ^= (unsigned char)p[i]; h *= 1099511628211ULL; } };
             mix(source.data(), source.size());
             mix(k_device_header, strlen(k_device_header));
+            mix(k_value_header, strlen(k_value_header));
             const std::string ver = strf("nvrtc %d.%d sm_100a fmad=false v1", rt.major, rt.minor);
             mix(ver.data(), ver.size());
             cache_file = std::string(dir) + strf("/nq_%016llx_%zu.cubin", (unsigned long long)h, source.size());
@@ -199,9 +203,9 @@ std::string jit_compile_cubin(const std::string& source, std::string* log) {
         }
     }
     nvrtcProgram prog;
-    const char* hdr_names[] = {"n1ql_device.cuh"};
-    const char* hdr_srcs[] = {k_device_header};
-    if (rt.CreateProgram(&prog, source.c_str(), "nq_scan.cu", 1, hdr_srcs, hdr_names) != NVRTC_SUCCESS)
+    const char* hdr_names[] = {"n1ql_device.cuh", "n1ql_value.cuh"};
+    const char* hdr_srcs[] = {k_device_header, k_value_header};
+    if (rt.CreateProgram(&prog, source.c_str(), "nq_scan.cu", 2, hdr_srcs, hdr_names) != NVRTC_SUCCESS)
         N1_THROW(N1GPU_E_CUDA, "nvrtcCreateProgram failed");
     // -fmad=false: float64 arithmetic must round like the reference's separate Go operations.
     // 256-bit global loads need the PTX ISA 8.8 assembler of CUDA >= 12.9; older NVRTC gets 2 x 128-bit.

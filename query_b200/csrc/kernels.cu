@@ -31,7 +31,7 @@ __device__ __forceinline__ void extract_bits(u64 lo, u64 hi, int pos, int n, u64
 }
 
 __device__ __forceinline__ int owner_of(u64 lo, u64 hi, int nranks) {
-    return nranks <= 1 ? 0 : (int)(::mix64(lo ^ ::mix64(hi ^ 0x9e3779b97f4a7c15ULL)) % (u64)nranks);
+    return nranks <= 1 ? 0 : (int)(mix64(lo ^ mix64(hi ^ 0x9e3779b97f4a7c15ULL)) % (u64)nranks);
 }
 
 // key of slot i and whether the slot holds a group.  kw: 0 dense (key = index, live iff word 0 > 0),
@@ -189,7 +189,7 @@ __device__ __forceinline__ void distinct_entry(u64 lo, u64 hi, int abits, int ke
         else slot = table_find128((const ulonglong2*)keys, cap - 1, klo, khi);
         if (slot < 0 || (u64)slot >= cap) return;  // group owned by another rank
         bool decoded = false;
-        FinalVal val{C_MISSING, 0};
+        Val val{C_MISSING, 0};
         for (int a = 0; a < D.n; ++a) {
             const DistinctDesc& d = D.d[a];
             if (d.sid != sid) continue;
@@ -197,15 +197,15 @@ __device__ __forceinline__ void distinct_entry(u64 lo, u64 hi, int abits, int ke
                 val = decode_comp(d.value, v);
                 decoded = true;
             }
-            if (d.numbers_only && !(val.cls == C_INT || val.cls == C_FLOAT)) continue;
+            if (d.numbers_only && !(val.c == C_INT || val.c == C_FLOAT)) continue;
             atomicAdd(&acc[(u64)d.w_cnt * cap + (u64)slot], 1ULL);
-            if (val.cls == C_INT && d.w_ilo >= 0) {
-                const i64 x = val.bits;
+            if (val.c == C_INT && d.w_ilo >= 0) {
+                const i64 x = val.b;
                 atomicAdd(&acc[(u64)d.w_ilo * cap + (u64)slot], (u64)x & 0xffffffffULL);
                 atomicAdd(&acc[(u64)d.w_ihi * cap + (u64)slot], (u64)(x >> 32));
                 if (x < 0) atomicAdd(&acc[(u64)d.w_neg * cap + (u64)slot], 1ULL);
-            } else if (val.cls == C_FLOAT && d.w_fsum >= 0) {
-                atomicAdd((double*)&acc[(u64)d.w_fsum * cap + (u64)slot], __longlong_as_double(val.bits));
+            } else if (val.c == C_FLOAT && d.w_fsum >= 0) {
+                atomicAdd((double*)&acc[(u64)d.w_fsum * cap + (u64)slot], __longlong_as_double(val.b));
                 atomicAdd(&acc[(u64)d.w_nflt * cap + (u64)slot], 1ULL);
             }
         }

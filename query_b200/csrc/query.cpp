@@ -7,42 +7,12 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstddef>
 #include <thread>
 #include <unordered_map>
 
 namespace n1 {
 
 namespace {
-// must mirror NqParams in n1ql_device.cuh
-struct NqParamsHost {
-    i64 nrows;
-    const void* col[16];
-    const u8* tag[16];
-    u64* acc;
-    u64* keys;
-    u64 cap_mask;
-    u64* set_keys;
-    u64 set_mask;
-    int* status;
-    u64 dense_groups;
-    u64* final_dev;
-    u64* final_host;
-    unsigned* ticket;
-    u64* partials;
-    u64* const* peer_mail;
-    int nranks, rank;
-    u64 mail_base;
-    u64 mail_words;
-    u64 mail_seq;
-    int set_pass, set_shift;
-    i64 cst[32];
-    const int* cancel;
-    InSetDesc inset[MAX_IN_SETS];
-};
-static_assert(sizeof(InSetDesc) == 32, "NqInSet layout");
-static_assert(offsetof(NqParamsHost, cancel) == 8 + 128 + 128 + 8 * 17 + 256, "NqParams layout");
-static_assert(sizeof(NqParamsHost) == 8 + 128 + 128 + 8 * 17 + 256 + 8 + 32 * MAX_IN_SETS, "NqParams layout");
 
 u64 pow2_at_least(u64 n) { u64 p = 1; while (p < n) p <<= 1; return p; }
 
@@ -142,7 +112,7 @@ void Query::upload_in_sets() {
     const u64* base = d_in_sets.as<u64>();
     in_descs.clear();
     for (size_t k = 0; k < S.size(); ++k) {
-        InSetDesc d{};
+        NqInSet d{};
         d.bits = S[k].bits.empty() ? nullptr : (const u32*)(base + at[k]);
         d.keys = base + at[k] + (S[k].bits.size() + 1) / 2;
         d.icap = (u32)S[k].ikeys.size();
@@ -272,7 +242,7 @@ void Query::launch_scan() {
     if (launched) N1_THROW(N1GPU_E_INVALID, "a scan is already outstanding on this query");
     launches_at_start = g_launches.load();
     if (peer_table) { peer_seq = ++mailbox->seq; ++peer_steps; }  // flags are numbered per mailbox, table buffers alternate per query (acc())
-    NqParamsHost p{};
+    NqParams p{};
     p.nrows = table->nrows;
     for (size_t c = 0; c < table->cols.size(); ++c) { p.col[c] = table->cols[c].d_payload.p; p.tag[c] = table->cols[c].d_tags.as<u8>(); }
     for (size_t k = 0; k < kp.consts.size() && k < 32; ++k) p.cst[k] = kp.consts[k];

@@ -99,14 +99,6 @@ struct Mailbox {
     ~Mailbox();
 };
 
-// must mirror NqInSet in n1ql_device.cuh
-struct InSetDesc {
-    const u32* bits;
-    const u64* keys;
-    u32 icap, fcap;
-    u32 flags, pad;
-};
-
 struct Query {
     Table* table = nullptr;
     Mailbox* mailbox = nullptr;
@@ -136,7 +128,7 @@ struct Query {
     }
     DistinctDescs distinct_descs() const;
     DevBuf d_in_sets;                  // every IN set of the chain (KernelPlan::in_sets), copied once at compile time
-    std::vector<InSetDesc> in_descs;   // NqParams::inset
+    std::vector<NqInSet> in_descs;     // NqParams::inset
     void upload_in_sets();
     OpsArr ops{};
 

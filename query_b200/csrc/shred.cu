@@ -8,7 +8,7 @@
 // shredder for that document only ("fix-up rows"); results are identical to table.cpp's host shredder,
 // which tests/test_gpu_shredder.py checks row by row.
 #include "shred.hpp"
-#include "n1ql_device.cuh"  // after common.hpp: its C_* / OP_* macros shadow the host enums of the same value
+#include "n1ql_device.cuh"
 
 namespace n1 {
 
@@ -203,7 +203,7 @@ __device__ int sh_document(const unsigned char* base, i64 b, i64 e, const ShredT
                 if (col >= 0) {
                     if (k == 3) return 2;
                     if (k == 1) out.put(col, C_INT, iv);
-                    else if (::f_is_int(dv)) out.put(col, C_INT, ::go_i64(dv));  // NewValue canonicalisation
+                    else if (f_is_int(dv)) out.put(col, C_INT, go_i64(dv));  // NewValue canonicalisation
                     else out.put(col, C_FLOAT, __double_as_longlong(dv));
                 }
             }
@@ -376,7 +376,7 @@ __global__ void k_dict_insert(const unsigned char* __restrict__ buf, const unsig
         const u64 len = ref & 0xffffff;
         u64 h = 1469598103934665603ULL;
         for (u64 i = 0; i < len; ++i) { h ^= p[i]; h *= 1099511628211ULL; }
-        u64 slot = ::mix64(h) & cap_mask;
+        u64 slot = mix64(h) & cap_mask;
         bool done = false;
         // (a probe sequence this long means the table is far too dense: every step compares string bytes)
         for (u64 probe = 0; probe <= cap_mask && probe < 128; ++probe) {
@@ -445,7 +445,7 @@ __global__ void k_canon_floats(u8* tags, i64* payload, i64 nrows) {
     for (i64 row = (i64)blockIdx.x * blockDim.x + threadIdx.x; row < nrows; row += (i64)gridDim.x * blockDim.x) {
         if (tags[row] != C_FLOAT) continue;
         const double d = __longlong_as_double(payload[row]);
-        if (::f_is_int(d)) { tags[row] = C_INT; payload[row] = ::go_i64(d); }
+        if (f_is_int(d)) { tags[row] = C_INT; payload[row] = go_i64(d); }
     }
 }
 // host fix-ups: (row, tag, payload) triples for one column

@@ -1,5 +1,5 @@
 """IN over array parameters and long literal lists: `x IN $p` binds a JSON array, and the list is probed as a device-resident
-set (NqInSet in n1ql_device.cuh) whose contents are kernel arguments, so every binding of a statement runs one cubin.
+set (NqInSet in n1ql_value.cuh) whose contents are kernel arguments, so every binding of a statement runs one cubin.
 Literal lists of at most IN_CHAIN_MAX elements keep the unrolled in_arg chain."""
 import functools
 import json

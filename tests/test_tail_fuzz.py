@@ -2,8 +2,8 @@
 oracle (which is pinned to the reference's goldens): seeded random expression trees over group keys, aggregates and
 constants - arithmetic with int64 overflow -> float64 promotion, collation across types, 4-valued logic, BETWEEN, IN,
 IS [NOT] NULL / MISSING / VALUED, ROUND - evaluated over random groups whose values range over MISSING, NULL, booleans,
-small and near-overflow ints, floats and strings.  The same semantics, from the same reference lines, are what
-n1ql_device.cuh implements for the scan kernel; the kernel itself is checked on the device by tests/test_gpu_parity.py."""
+small and near-overflow ints, floats and strings.  Numbers and logic are the code of n1ql_value.cuh, which the scan
+kernel runs too; the kernel itself is checked on the device by tests/test_gpu_parity.py."""
 import json
 import math
 import random
