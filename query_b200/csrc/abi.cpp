@@ -1,10 +1,6 @@
 // abi.cpp — the extern "C" surface declared in include/n1gpu.h.  Exceptions never cross it.
-#include <atomic>
 #include <cstring>
-#include <functional>
 #include <mutex>
-#include <string_view>
-#include <thread>
 
 #include "execution.hpp"
 #include "query.hpp"
@@ -106,10 +102,7 @@ int n1gpu_table_dict_export(n1gpu_table* t, int col, char* blob, int64_t blob_ca
                             int64_t* ndict, int64_t* blob_bytes) {
     return guard([&] {
         REQUIRE(t); REQUIRE(ndict); REQUIRE(blob_bytes);
-        if (col < 0 || col >= (int)t->t.cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column");
-        if (t->t.sealed) N1_THROW(N1GPU_E_INVALID, "dictionary exchange happens before seal");
-        t->t.build_dictionary(col);
-        const auto& d = t->t.cols[col].dict;
+        const auto& d = t->t.exchange_column(col).dict;
         i64 bytes = 0;
         for (auto& s : d) bytes += (i64)s.size();
         *ndict = (int64_t)d.size();
@@ -122,101 +115,13 @@ int n1gpu_table_dict_export(n1gpu_table* t, int col, char* blob, int64_t blob_ca
     });
 }
 int n1gpu_table_dict_import(n1gpu_table* t, int col, const char* blob, const int64_t* offsets, int64_t ndict) {
-    return guard([&] {
-        REQUIRE(t); REQUIRE(offsets);
-        if (col < 0 || col >= (int)t->t.cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column");
-        if (t->t.sealed) N1_THROW(N1GPU_E_INVALID, "dictionary exchange happens before seal");
-        t->t.build_dictionary(col);
-        std::vector<std::string> global;
-        global.reserve((size_t)ndict);
-        for (i64 i = 0; i < ndict; ++i) global.emplace_back(blob + offsets[i], blob + offsets[i + 1]);
-        for (size_t i = 1; i < global.size(); ++i)
-            if (!(global[i - 1] < global[i])) N1_THROW(N1GPU_E_INVALID, "global dictionary must be sorted bytewise and unique");
-        t->t.adopt_dictionary(col, global);
-    });
+    return guard([&] { REQUIRE(t); REQUIRE(offsets); t->t.import_dictionary(col, blob, (const i64*)offsets, ndict); });
 }
 int n1gpu_table_dict_merge(n1gpu_table* t, int col, int nparts, const char* const* blobs, const int64_t* const* offsets, const int64_t* ndicts) {
     return guard([&] {
         REQUIRE(t); REQUIRE(blobs); REQUIRE(offsets); REQUIRE(ndicts);
-        if (col < 0 || col >= (int)t->t.cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column");
-        if (t->t.sealed) N1_THROW(N1GPU_E_INVALID, "dictionary exchange happens before seal");
         if (nparts < 1) N1_THROW(N1GPU_E_INVALID, "no dictionaries to merge");
-        t->t.build_dictionary(col);
-        // k-way merge of the sorted, unique dictionaries (the column's own included) into the global sorted dictionary.
-        // The value range is cut at splitters taken from the longest list and every thread merges one cut (8 ranks x 100 k
-        // strings: 32 ms single-threaded, most of an end-to-end step at 8 GPUs).
-        struct List {
-            const char* blob; const int64_t* off; const std::vector<std::string>* own; i64 n;
-            std::string_view at(i64 i) const {
-                return own ? std::string_view((*own)[(size_t)i]) : std::string_view(blob + off[i], (size_t)(off[i + 1] - off[i]));
-            }
-            i64 lower_bound(std::string_view v) const {
-                i64 lo = 0, hi = n;
-                while (lo < hi) { const i64 m = (lo + hi) / 2; if (at(m) < v) lo = m + 1; else hi = m; }
-                return lo;
-            }
-        };
-        std::vector<List> lists;
-        for (int p = 0; p < nparts; ++p) if (ndicts[p] > 0) lists.push_back(List{blobs[p], offsets[p], nullptr, (i64)ndicts[p]});
-        const std::vector<std::string>& own = t->t.cols[col].dict.vec();
-        if (!own.empty()) lists.push_back(List{nullptr, nullptr, &own, (i64)own.size()});
-        std::vector<std::string> global;
-        if (!lists.empty()) {
-            size_t longest = 0;
-            i64 total = 0;
-            for (size_t l = 0; l < lists.size(); ++l) { total += lists[l].n; if (lists[l].n > lists[longest].n) longest = l; }
-            const int nthr = total < 32768 ? 1 : (int)std::min<i64>(std::max(1u, std::thread::hardware_concurrency()), 16);
-            std::vector<std::vector<std::string_view>> out((size_t)nthr);
-            std::atomic<bool> unsorted{false};
-            auto work = [&](int th) {
-                const List& L = lists[longest];
-                const bool first = th == 0, last = th == nthr - 1;
-                const std::string_view lo = first ? std::string_view() : L.at(L.n * th / nthr);
-                const std::string_view hi = last ? std::string_view() : L.at(L.n * (th + 1) / nthr);
-                std::vector<i64> at(lists.size()), end(lists.size());
-                i64 room = 0;
-                for (size_t l = 0; l < lists.size(); ++l) {
-                    at[l] = first ? 0 : lists[l].lower_bound(lo);
-                    end[l] = last ? lists[l].n : lists[l].lower_bound(hi);
-                    room = std::max(room, end[l] - at[l]);
-                }
-                auto& o = out[(size_t)th];
-                o.reserve((size_t)room + 64);
-                for (;;) {
-                    bool any = false;
-                    std::string_view best;
-                    for (size_t l = 0; l < lists.size(); ++l)
-                        if (at[l] < end[l]) { const std::string_view v = lists[l].at(at[l]); if (!any || v < best) { best = v; any = true; } }
-                    if (!any) break;
-                    o.push_back(best);
-                    for (size_t l = 0; l < lists.size(); ++l)
-                        if (at[l] < end[l]) {
-                            const std::string_view v = lists[l].at(at[l]);
-                            if (v.size() == best.size() && (v.data() == best.data() || memcmp(v.data(), best.data(), v.size()) == 0)) ++at[l];
-                        }
-                }
-            };
-            // strictly increasing lists are the premise of the cuts: checked first (every thread takes a stripe of every list)
-            auto check = [&](int th) {
-                for (const List& L : lists)
-                    for (i64 i = std::max<i64>(L.n * th / nthr, 1); i < L.n * (th + 1) / nthr; ++i)
-                        if (!(L.at(i - 1) < L.at(i))) { unsorted = true; return; }
-            };
-            auto run = [&](const std::function<void(int)>& f) {
-                if (nthr == 1) return f(0);
-                std::vector<std::thread> pool;
-                for (int th = 0; th < nthr; ++th) pool.emplace_back(f, th);
-                for (auto& th : pool) th.join();
-            };
-            run(check);
-            if (unsorted) N1_THROW(N1GPU_E_INVALID, "dictionaries to merge must be sorted bytewise and unique");
-            run(work);
-            size_t n = 0;
-            for (auto& o : out) n += o.size();
-            global.reserve(n);
-            for (auto& o : out) for (const std::string_view v : o) global.emplace_back(v);
-        }
-        t->t.adopt_dictionary(col, global);
+        t->t.merge_dictionaries(col, nparts, blobs, (const i64* const*)offsets, (const i64*)ndicts);
     });
 }
 int n1gpu_table_stats_get(n1gpu_table* t, int col, int64_t stats[8]) {
@@ -225,20 +130,9 @@ int n1gpu_table_stats_get(n1gpu_table* t, int col, int64_t stats[8]) {
         if (col < 0 || col >= (int)t->t.cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column");
         Column& c = t->t.cols[col];
         ColumnStats st = c.stats;
-        if (!t->t.sealed && !c.stats_forced && !t->t.device_shredded) {  // compute from staging
-            st = ColumnStats();
-            for (size_t i = 0; i < c.tags.size(); ++i) {
-                u8 tg = c.tags[i];
-                if (tg == C_FLOAT) { double d; memcpy(&d, &c.payload[i], 8); if (f_is_int(d)) tg = C_INT; else st.has_float = true; }
-                if (tg == C_INT) {
-                    i64 v = c.tags[i] == C_INT ? c.payload[i] : go_i64(*(double*)&c.payload[i]);
-                    if (!st.has_int) { st.int_min = st.int_max = v; st.has_int = true; }
-                    else { st.int_min = std::min(st.int_min, v); st.int_max = std::max(st.int_max, v); }
-                }
-                st.class_mask |= bit(tg);
-                st.absent_rows += tg <= C_NULL;
-            }
-            st.ndict = (i64)c.dict.size();
+        if (!t->t.sealed && !c.stats_forced && !t->t.rows_in_hbm()) {  // compute from staging
+            st = host_stats(c.tags, c.payload);
+            st.set_dictionary(c.dict);
         }
         stats[0] = st.class_mask; stats[1] = st.has_int; stats[2] = st.int_min; stats[3] = st.int_max;
         stats[4] = st.has_float; stats[5] = st.ndict; stats[6] = st.empty_rank; stats[7] = st.absent_rows;
@@ -250,9 +144,9 @@ int n1gpu_table_stats_set(n1gpu_table* t, int col, const int64_t stats[8]) {
         if (col < 0 || col >= (int)t->t.cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column");
         if (t->t.sealed) N1_THROW(N1GPU_E_INVALID, "statistics exchange happens before seal");
         Column& c = t->t.cols[col];
+        c.stats.set_dictionary(c.dict);  // empty_rank: the exchanged word 6 is ignored
         c.stats.class_mask = (u32)stats[0]; c.stats.has_int = stats[1] != 0; c.stats.int_min = stats[2]; c.stats.int_max = stats[3];
         c.stats.has_float = stats[4] != 0; c.stats.ndict = stats[5]; c.stats.absent_rows = stats[7];
-        c.stats.empty_rank = (!c.dict.empty() && c.dict[0].empty()) ? 0 : -1;
         c.stats_forced = true;
     });
 }

@@ -7,9 +7,11 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <exception>
 #include <memory>
 #include <stdexcept>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/n1gpu.h"
@@ -110,6 +112,18 @@ inline int bits_for(u64 n_values) {  // bits to represent values 0..n_values-1
     int b = 0;
     while (b < 64 && ((u64)1 << b) < n_values) ++b;
     return b;
+}
+
+// fn(0) .. fn(n - 1), each on its own thread (fn(0) on the caller's); returns when all have, rethrowing the first
+// exception one of them threw
+template <class F> void parallel_for(int n, F&& fn) {
+    std::vector<std::exception_ptr> errs((size_t)(n > 0 ? n : 0));
+    auto run = [&](int t) { try { fn(t); } catch (...) { errs[(size_t)t] = std::current_exception(); } };
+    std::vector<std::thread> pool;
+    try { for (int t = 1; t < n; ++t) pool.emplace_back(run, t); } catch (...) { for (auto& th : pool) th.join(); throw; }
+    if (n > 0) run(0);
+    for (auto& th : pool) th.join();
+    for (auto& e : errs) if (e) std::rethrow_exception(e);
 }
 
 double now_sec();

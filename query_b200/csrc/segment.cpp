@@ -22,7 +22,6 @@
 #include <cstdint>
 #include <fcntl.h>
 #include <unistd.h>
-#include <thread>
 #include "table.hpp"
 
 namespace n1 {
@@ -129,7 +128,7 @@ void Table::write_segment(const std::string& segment_out, const std::string& seg
 // a refused segment is not an error (the caller shreds the documents instead); N1GPU_TRACE says which check refused it
 #define REFUSE(check) do { if (getenv("N1GPU_TRACE")) fprintf(stderr, "[n1gpu segment] %s not loaded (check %d)\n", file.c_str(), check); return false; } while (0)
 bool Table::load_segment(const std::string& file, const std::string& source) {
-    if (sealed || appended || nrows) N1_THROW(N1GPU_E_INVALID, "a segment loads into an empty, unsealed table");
+    admit(Entry::LOAD_SEGMENT);
     std::ifstream f(file, std::ios::binary);
     if (!f) REFUSE(3);
     f.seekg(0, std::ios::end);
@@ -198,10 +197,10 @@ bool Table::load_segment(const std::string& file, const std::string& source) {
         col.payload = std::move(staged[c].payload);
         col.tags = std::move(staged[c].tags);
         col.local_strings.clear();
-        col.codes_are_ranks = true;
+        col.dict_staged = false;
     }
     nrows = n;
-    appended = true;  // like appended documents: no further input may be mixed in
+    filled = Fill::HOST_DOCS;  // like appended documents: no further input may be mixed in
     return true;
 }
 
@@ -231,26 +230,18 @@ void Table::load_ndjson(const std::string& file, int threads) {
     int nthr = (int)std::min<size_t>(std::max(1u, std::thread::hardware_concurrency()), 16);
     if ((size_t)nthr > size / ((size_t)4 << 20) + 1) nthr = (int)(size / ((size_t)4 << 20) + 1);
     auto slice = [&](int t) { return size * (size_t)t / (size_t)nthr; };
-    std::vector<std::string> errs((size_t)nthr);
-    auto run = [&](auto&& fn) {
-        if (nthr == 1) { fn(0); return; }
-        std::vector<std::thread> pool;
-        for (int t = 0; t < nthr; ++t) pool.emplace_back(fn, t);
-        for (auto& th : pool) th.join();
-    };
     // bytes [lo, hi) of the file, read by all threads at once
     auto read_range = [&](size_t lo, size_t hi) {
         const size_t span = hi - lo;
-        run([&](int t) {
+        parallel_for(nthr, [&](int t) {
             size_t at = lo + span * (size_t)t / (size_t)nthr;
             const size_t end = lo + span * (size_t)(t + 1) / (size_t)nthr;
             while (at < end) {
                 const ssize_t got = pread(fd, data + at, end - at, (off_t)at);
-                if (got <= 0) { errs[(size_t)t] = "short read of " + file; return; }
+                if (got <= 0) N1_THROW(N1GPU_E_IO, "short read of %s", file.c_str());
                 at += (size_t)got;
             }
         });
-        for (auto& e : errs) if (!e.empty()) N1_THROW(N1GPU_E_IO, "%s", e.c_str());
     };
     if (device && have_device()) {
         // the device finds the line starts itself (shred.cu k_ndjson_lines); the file is read chunk by chunk while the chunks
@@ -295,7 +286,7 @@ void Table::load_ndjson(const std::string& file, int threads) {
         for (; i < hi; ++i) if (data[i] == '\n' && i + 1 < size) consider(i + 1);
     };
     std::vector<size_t> run_at((size_t)nthr + 1, 0);
-    run([&](int t) { size_t n = 0; scan(t, [&](i64) { ++n; }); run_at[(size_t)t + 1] = n; });
+    parallel_for(nthr, [&](int t) { size_t n = 0; scan(t, [&](i64) { ++n; }); run_at[(size_t)t + 1] = n; });
     for (int t = 0; t < nthr; ++t) run_at[(size_t)t + 1] += run_at[(size_t)t];
     const size_t ndocs = run_at[(size_t)nthr];
     phase("count documents");
@@ -304,7 +295,7 @@ void Table::load_ndjson(const std::string& file, int threads) {
     i64* offsets = nullptr;
     if (device && have_device()) { pin_offs.ensure((ndocs + 1) * 8 + 64); offsets = pin_offs.as<i64>(); }
     else { heap_offs.resize(ndocs + 1); offsets = heap_offs.data(); }
-    run([&](int t) { i64* out = offsets + run_at[(size_t)t]; scan(t, [&](i64 s0) { *out++ = s0; }); });
+    parallel_for(nthr, [&](int t) { i64* out = offsets + run_at[(size_t)t]; scan(t, [&](i64 s0) { *out++ = s0; }); });
     offsets[ndocs] = (i64)size;
     if (ndocs == 0) offsets[0] = 0;
     phase("offsets");

@@ -18,6 +18,7 @@
 #include <cerrno>
 #include <chrono>
 #include <fstream>
+#include <string_view>
 #include <thread>
 
 #include "json.hpp"
@@ -45,8 +46,32 @@ std::string join_path(const std::vector<std::string>& p, char sep) {
     return s;
 }
 
+// The one place that decides which entry point may follow which: rows come in by one route (Fill), documents and segments
+// in full, columns one by one.
+void Table::admit(Entry e, int col) const {
+    const bool docs = filled == Fill::HOST_DOCS || filled == Fill::DEVICE_DOCS;  // documents, a segment or a splice: the rows are in
+    auto refuse = [](const char* why) { N1_THROW(N1GPU_E_INVALID, "%s", why); };
+    if (e == Entry::ADD_COLUMN) { if (sealed || docs) refuse("columns must be declared before documents are appended"); return; }
+    if (e == Entry::LOAD_SEGMENT) { if (sealed || docs || nrows) refuse("a segment loads into an empty, unsealed table"); return; }
+    if (e == Entry::SPLICE) { if (sealed || docs || nrows) refuse("a splice fills an empty, unsealed table"); return; }
+    if (sealed) refuse("table is sealed");
+    if (e == Entry::APPEND_HOST) {
+        if (rows_in_hbm()) refuse("table already holds device-shredded rows");
+        for (auto& c : cols)
+            if (!c.dict_staged) refuse("append after dictionary import / pre-shredded columns is not supported");
+    } else if (e == Entry::APPEND_DEVICE) {
+        if (!have_device()) N1_THROW(N1GPU_E_CUDA, "the device shredder needs a CUDA device (there is no CPU fallback for it; use host threads explicitly)");
+        if (docs || nrows) refuse("the device shredder takes the whole keyspace in one append");
+    } else {  // SET_COLUMN, SET_COLUMN_DEVICE (of column `col`)
+        if (docs) refuse("cannot mix appended documents and pre-shredded columns");
+        for (size_t c = 0; c < cols.size(); ++c)
+            if (e == Entry::SET_COLUMN ? filled == Fill::DEVICE_COLUMNS : c != (size_t)col && !cols[c].tags.empty())
+                refuse("cannot mix host and device columns in one table");
+    }
+}
+
 int Table::add_column(const std::string& path) {
-    if (appended || sealed) N1_THROW(N1GPU_E_INVALID, "columns must be declared before documents are appended");
+    admit(Entry::ADD_COLUMN);
     int f = find_column(path);
     if (f >= 0) return f;
     if (cols.size() >= 16) N1_THROW(N1GPU_E_INELIGIBLE, "more than 16 referenced columns");
@@ -204,35 +229,27 @@ void host_shred_docs(const std::vector<Column>& cols, const char* buf, const i64
 void Table::append_json(const char* buf, const i64* offsets, i64 ndocs, int threads) {
     if (sealed) N1_THROW(N1GPU_E_INVALID, "table is sealed");
     if (threads == -1) { append_json_device(buf, offsets, ndocs); return; }
-    if (device_shredded) N1_THROW(N1GPU_E_INVALID, "table already holds device-shredded rows");
-    for (auto& col : cols)
-        if (col.dict_global || col.codes_are_ranks) N1_THROW(N1GPU_E_INVALID, "append after dictionary import / pre-shredded columns is not supported");
+    admit(Entry::APPEND_HOST);
     if (ndocs < 0) N1_THROW(N1GPU_E_INVALID, "negative document count");
     double t0 = now_sec();
-    appended = true;
+    filled = Fill::HOST_DOCS;
     Trie trie;
     for (size_t c = 0; c < cols.size(); ++c) trie.add(cols[c].path, (int)c);
     int nthreads = threads > 0 ? threads : (int)std::thread::hardware_concurrency();
     if (nthreads < 1) nthreads = 1;
     if ((i64)nthreads > (ndocs + 4095) / 4096) nthreads = (int)std::max<i64>(1, (ndocs + 4095) / 4096);
     std::vector<std::vector<ChunkCol>> chunks(nthreads);
-    std::vector<std::thread> pool;
-    auto work = [&](int t) {
+    parallel_for(nthreads, [&](int t) {
         i64 lo = ndocs * t / nthreads, hi = ndocs * (t + 1) / nthreads;
         auto& cc = chunks[t];
         cc.resize(cols.size());
         for (auto& c : cc) { c.payload.assign((size_t)(hi - lo), 0); c.tags.assign((size_t)(hi - lo), C_MISSING); }
         Shredder sh(trie, cc);
         for (i64 d = lo; d < hi; ++d) sh.document(buf + offsets[d], buf + offsets[d + 1]);
-    };
-    if (nthreads == 1) work(0);
-    else {
-        for (int t = 0; t < nthreads; ++t) pool.emplace_back(work, t);
-        for (auto& th : pool) th.join();
-    }
+    });
     // merge chunk-local string codes into the column's staging dictionary (parallel over columns)
     std::vector<std::unordered_map<std::string, u32>> colindex(cols.size());
-    auto merge = [&](size_t c) {
+    auto merge = [&](int c) {
         Column& col = cols[c];
         auto& index = colindex[c];
         for (u32 i = 0; i < col.local_strings.size(); ++i) index.emplace(col.local_strings[i], i);
@@ -259,16 +276,8 @@ void Table::append_json(const char* buf, const i64* offsets, i64 ndocs, int thre
             at += n;
         }
     };
-    if (cols.size() > 1 && nthreads > 1) {
-        std::vector<std::thread> mp;
-        std::vector<std::string> errs(cols.size());
-        for (size_t c = 0; c < cols.size(); ++c)
-            mp.emplace_back([&, c] { try { merge(c); } catch (const std::exception& e) { errs[c] = e.what(); } });
-        for (auto& th : mp) th.join();
-        for (auto& e : errs) if (!e.empty()) N1_THROW(N1GPU_E_INVALID, "%s", e.c_str());
-    } else {
-        for (size_t c = 0; c < cols.size(); ++c) merge(c);
-    }
+    if (cols.size() > 1 && nthreads > 1) parallel_for((int)cols.size(), merge);
+    else for (int c = 0; c < (int)cols.size(); ++c) merge(c);
     nrows += ndocs;
     json_bytes += offsets[ndocs] - offsets[0];
     shred_sec += now_sec() - t0;
@@ -324,9 +333,9 @@ void Table::load_entries(const std::string& dir, const std::vector<std::string>&
     int nthreads = (int)std::thread::hardware_concurrency();
     if (nthreads < 1) nthreads = 1;
     if ((size_t)nthreads > (nfiles + 255) / 256) nthreads = (int)std::max<size_t>(1, (nfiles + 255) / 256);
-    struct Part { std::string bytes; std::vector<i64> sizes; std::string err; };
+    struct Part { std::string bytes; std::vector<i64> sizes; };
     std::vector<Part> parts((size_t)nthreads);
-    auto read_range = [&](int t) {
+    parallel_for(nthreads, [&](int t) {
         Part& part = parts[(size_t)t];
         const size_t lo = nfiles * (size_t)t / (size_t)nthreads, hi = nfiles * (size_t)(t + 1) / (size_t)nthreads;
         part.sizes.reserve(hi - lo);
@@ -357,15 +366,9 @@ void Table::load_entries(const std::string& dir, const std::vector<std::string>&
             if (fps) (*fps)[i] = fp;
             if (!failed) part.sizes.push_back((i64)(part.bytes.size() - before));
         }
-    };
-    if (nthreads == 1) read_range(0);
-    else {
-        std::vector<std::thread> pool;
-        for (int t = 0; t < nthreads; ++t) pool.emplace_back(read_range, t);
-        for (auto& th : pool) th.join();
-    }
+    });
     size_t total = 0;
-    for (auto& part : parts) { if (!part.err.empty()) N1_THROW(N1GPU_E_IO, "%s", part.err.c_str()); total += part.bytes.size(); }
+    for (auto& part : parts) total += part.bytes.size();
     // laid end to end - in pinned memory when the device shredder takes the text (its H2D copy then needs no staging)
     PinnedBuf pin;
     std::string heap;
@@ -380,27 +383,38 @@ void Table::load_entries(const std::string& dir, const std::vector<std::string>&
         part_at[i + 1] = part_at[i] + parts[i].bytes.size();
         for (i64 sz : parts[i].sizes) offsets.push_back(offsets.back() + sz);
     }
-    {
-        std::vector<std::thread> pool;
-        for (size_t i = 0; i < parts.size(); ++i)
-            pool.emplace_back([&, i] { if (!parts[i].bytes.empty()) memcpy(buf + part_at[i], parts[i].bytes.data(), parts[i].bytes.size()); std::string().swap(parts[i].bytes); });
-        for (auto& th : pool) th.join();
-    }
+    parallel_for((int)parts.size(), [&](int i) {
+        if (!parts[i].bytes.empty()) memcpy(buf + part_at[i], parts[i].bytes.data(), parts[i].bytes.size());
+        std::string().swap(parts[i].bytes);
+    });
     append_json(buf, offsets.data(), (i64)offsets.size() - 1, threads);  // ids without a document were skipped
+}
+
+std::vector<std::string> read_dictionary(const char* blob, const i64* offs, i64 n, const char* what) {
+    std::vector<std::string> d;
+    d.reserve((size_t)std::max<i64>(n, 0));
+    for (i64 i = 0; i < n; ++i) {
+        d.emplace_back(blob + offs[i], blob + offs[i + 1]);
+        if (i && !(d[(size_t)i - 1] < d[(size_t)i])) N1_THROW(N1GPU_E_INVALID, "%s must be sorted bytewise and unique", what);
+    }
+    return d;
+}
+
+void Table::check_column_args(int c, int width, i64 n) const {
+    if (c < 0 || c >= (int)cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column %d", c);
+    if (width != 8 && width != 4) N1_THROW(N1GPU_E_INVALID, "payload width must be 8 or 4");
+    if (n < 0) N1_THROW(N1GPU_E_INVALID, "negative row count");
 }
 
 void Table::set_column(int c, int width, const void* payload, const u8* tags, i64 n, const char* blob,
                        const i64* offs, i64 ndict) {
-    if (sealed) N1_THROW(N1GPU_E_INVALID, "table is sealed");
-    if (c < 0 || c >= (int)cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column %d", c);
-    if (width != 8 && width != 4) N1_THROW(N1GPU_E_INVALID, "payload width must be 8 or 4");
-    if (n < 0) N1_THROW(N1GPU_E_INVALID, "negative row count");
-    if (appended) N1_THROW(N1GPU_E_INVALID, "cannot mix appended documents and pre-shredded columns");
-    for (auto& other : cols)
-        if (other.device_set) N1_THROW(N1GPU_E_INVALID, "cannot mix host and device columns in one table");
+    admit(Entry::SET_COLUMN);
+    check_column_args(c, width, n);
     for (auto& other : cols)
         if (&other != &cols[c] && !other.tags.empty() && (i64)other.tags.size() != n)
             N1_THROW(N1GPU_E_INVALID, "column lengths differ (%lld vs %lld)", (long long)other.tags.size(), (long long)n);
+    std::vector<std::string> dict;
+    if (blob && offs) dict = read_dictionary(blob, offs, ndict, "dictionary");
     Column& col = cols[c];
     col.payload.resize((size_t)n);
     col.tags.resize((size_t)n);
@@ -408,14 +422,10 @@ void Table::set_column(int c, int width, const void* payload, const u8* tags, i6
     else for (i64 i = 0; i < n; ++i) col.payload[(size_t)i] = ((const u32*)payload)[i];
     if (tags) memcpy(col.tags.data(), tags, (size_t)n);
     else memset(col.tags.data(), width == 8 ? C_INT : C_STRING, (size_t)n);
-    col.dict.clear();
-    if (blob && offs) {
-        for (i64 i = 0; i < ndict; ++i) col.dict.emplace_back(blob + offs[i], blob + offs[i + 1]);
-        for (size_t i = 1; i < col.dict.size(); ++i)
-            if (!(col.dict[i - 1] < col.dict[i])) N1_THROW(N1GPU_E_INVALID, "dictionary must be sorted bytewise and unique");
-    }
-    col.codes_are_ranks = true;
+    col.dict = std::move(dict);
+    col.dict_staged = false;
     nrows = n;
+    filled = Fill::HOST_COLUMNS;
 }
 
 void Table::adopt_dictionary(int ci, std::vector<std::string>& global) {
@@ -430,17 +440,97 @@ void Table::adopt_dictionary(int ci, std::vector<std::string>& global) {
     bool identity = remap.size() == global.size();
     if (!identity || !remap.empty()) for (size_t i = 0; i < remap.size() && identity; ++i) identity = remap[i] == (u32)i;
     if (!identity && !remap.empty()) {
-        if (c.d_payload.p && (device_shredded || c.device_set)) remap_ranks_device(ci, remap);
+        if (c.d_payload.p && rows_in_hbm()) remap_ranks_device(ci, remap);
         else for (size_t r = 0; r < c.tags.size(); ++r) if (c.tags[r] == C_STRING) c.payload[r] = remap[(size_t)c.payload[r]];
     }
     c.dict.swap(global);
-    c.dict_global = true;
-    if (device_shredded || c.device_set) { c.stats.ndict = (i64)c.dict.size(); c.stats.empty_rank = (!c.dict.empty() && c.dict[0].empty()) ? 0 : -1; }
+    if (rows_in_hbm()) c.stats.set_dictionary(c.dict);  // (staged columns take theirs at seal)
+}
+
+Column& Table::exchange_column(int c) {
+    if (c < 0 || c >= (int)cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column");
+    if (sealed) N1_THROW(N1GPU_E_INVALID, "dictionary exchange happens before seal");
+    build_dictionary(c);
+    return cols[(size_t)c];
+}
+
+void Table::import_dictionary(int c, const char* blob, const i64* offs, i64 n) {
+    exchange_column(c);
+    std::vector<std::string> global = read_dictionary(blob, offs, n, "global dictionary");
+    adopt_dictionary(c, global);
+}
+
+// k-way merge of the sorted, unique dictionaries (the column's own included) into the global sorted dictionary.  The value
+// range is cut at splitters taken from the longest list and every thread merges one cut (8 ranks x 100 k strings: 32 ms
+// single-threaded, most of an end-to-end step at 8 GPUs).
+void Table::merge_dictionaries(int c, int nparts, const char* const* blobs, const i64* const* offsets, const i64* ndicts) {
+    const std::vector<std::string>& own = exchange_column(c).dict.vec();
+    struct List {
+        const char* blob; const i64* off; const std::vector<std::string>* own; i64 n;
+        std::string_view at(i64 i) const {
+            return own ? std::string_view((*own)[(size_t)i]) : std::string_view(blob + off[i], (size_t)(off[i + 1] - off[i]));
+        }
+        i64 lower_bound(std::string_view v) const {
+            i64 lo = 0, hi = n;
+            while (lo < hi) { const i64 m = (lo + hi) / 2; if (at(m) < v) lo = m + 1; else hi = m; }
+            return lo;
+        }
+    };
+    std::vector<List> lists;
+    for (int p = 0; p < nparts; ++p) if (ndicts[p] > 0) lists.push_back(List{blobs[p], offsets[p], nullptr, ndicts[p]});
+    if (!own.empty()) lists.push_back(List{nullptr, nullptr, &own, (i64)own.size()});
+    std::vector<std::string> global;
+    if (!lists.empty()) {
+        size_t longest = 0;
+        i64 total = 0;
+        for (size_t l = 0; l < lists.size(); ++l) { total += lists[l].n; if (lists[l].n > lists[longest].n) longest = l; }
+        const int nthr = total < 32768 ? 1 : (int)std::min<i64>(std::max(1u, std::thread::hardware_concurrency()), 16);
+        // strictly increasing lists are the premise of the cuts: checked first (every thread takes a stripe of every list)
+        parallel_for(nthr, [&](int th) {
+            for (const List& L : lists)
+                for (i64 i = std::max<i64>(L.n * th / nthr, 1); i < L.n * (th + 1) / nthr; ++i)
+                    if (!(L.at(i - 1) < L.at(i))) N1_THROW(N1GPU_E_INVALID, "dictionaries to merge must be sorted bytewise and unique");
+        });
+        std::vector<std::vector<std::string_view>> out((size_t)nthr);
+        parallel_for(nthr, [&](int th) {
+            const List& L = lists[longest];
+            const bool first = th == 0, last = th == nthr - 1;
+            const std::string_view lo = first ? std::string_view() : L.at(L.n * th / nthr);
+            const std::string_view hi = last ? std::string_view() : L.at(L.n * (th + 1) / nthr);
+            std::vector<i64> at(lists.size()), end(lists.size());
+            i64 room = 0;
+            for (size_t l = 0; l < lists.size(); ++l) {
+                at[l] = first ? 0 : lists[l].lower_bound(lo);
+                end[l] = last ? lists[l].n : lists[l].lower_bound(hi);
+                room = std::max(room, end[l] - at[l]);
+            }
+            auto& o = out[(size_t)th];
+            o.reserve((size_t)room + 64);
+            for (;;) {
+                bool any = false;
+                std::string_view best;
+                for (size_t l = 0; l < lists.size(); ++l)
+                    if (at[l] < end[l]) { const std::string_view v = lists[l].at(at[l]); if (!any || v < best) { best = v; any = true; } }
+                if (!any) break;
+                o.push_back(best);
+                for (size_t l = 0; l < lists.size(); ++l)
+                    if (at[l] < end[l]) {
+                        const std::string_view v = lists[l].at(at[l]);
+                        if (v.size() == best.size() && (v.data() == best.data() || memcmp(v.data(), best.data(), v.size()) == 0)) ++at[l];
+                    }
+            }
+        });
+        size_t n = 0;
+        for (auto& o : out) n += o.size();
+        global.reserve(n);
+        for (auto& o : out) for (const std::string_view v : o) global.emplace_back(v);
+    }
+    adopt_dictionary(c, global);
 }
 
 void Table::build_dictionary(int c) {
     Column& col = cols[c];
-    if (col.codes_are_ranks) return;
+    if (!col.dict_staged) return;
     std::vector<u32> order(col.local_strings.size());
     for (u32 i = 0; i < order.size(); ++i) order[i] = i;
     std::sort(order.begin(), order.end(), [&](u32 a, u32 b) { return col.local_strings[a] < col.local_strings[b]; });
@@ -451,7 +541,35 @@ void Table::build_dictionary(int c) {
         if (col.tags[i] == C_STRING) col.payload[i] = rank[(size_t)col.payload[i]];
     col.local_strings.clear();
     col.local_strings.shrink_to_fit();
-    col.codes_are_ranks = true;
+    col.dict_staged = false;
+}
+
+ColumnStats host_stats(const std::vector<u8>& tags, const std::vector<i64>& payload) {
+    ColumnStats st;
+    for (size_t i = 0; i < tags.size(); ++i) {
+        u8 t = tags[i];
+        i64 v = payload[i];
+        double d;
+        memcpy(&d, &v, 8);
+        if (t == C_FLOAT && f_is_int(d)) { t = C_INT; v = go_i64(d); }
+        st.has_float |= t == C_FLOAT;
+        if (t == C_INT) {
+            st.int_min = st.has_int ? std::min(st.int_min, v) : v;
+            st.int_max = st.has_int ? std::max(st.int_max, v) : v;
+            st.has_int = true;
+        }
+        st.class_mask |= bit(t);
+        st.absent_rows += t <= C_NULL;
+    }
+    return st;
+}
+
+DevBuf Table::device_rows(int width, int byte, cudaStream_t s) const {
+    const size_t bytes = (size_t)std::max(padded_rows(), ROW_PAD) * (size_t)width;
+    DevBuf b;
+    b.alloc(bytes ? bytes : 256);
+    if (bytes) CK(cudaMemsetAsync(b.p, byte, bytes, s));
+    return b;
 }
 
 int Table::scan_bytes(int c) const {
@@ -461,12 +579,12 @@ int Table::scan_bytes(int c) const {
 
 void Table::seal() {
     if (sealed) return;
-    if (device_shredded) {  // columns, dictionaries and statistics already final in HBM
+    if (rows_in_hbm()) {  // columns, dictionaries and statistics already final in HBM
         bool any_set = false;
-        for (auto& col : cols) any_set = any_set || col.device_set;
+        for (auto& col : cols) any_set = any_set || col.on_device;
         if (any_set)
             for (auto& col : cols)
-                if (!col.device_set) N1_THROW(N1GPU_E_INVALID, "column %s was never set", join_path(col.path, '.').c_str());
+                if (!col.on_device) N1_THROW(N1GPU_E_INVALID, "column %s was never set", join_path(col.path, '.').c_str());
         sealed = true;
         return;
     }
@@ -474,42 +592,24 @@ void Table::seal() {
     for (auto& col : cols)
         if ((i64)col.tags.size() != nrows) N1_THROW(N1GPU_E_INVALID, "column %s has %lld rows, table has %lld",
                                                     join_path(col.path, '.').c_str(), (long long)col.tags.size(), (long long)nrows);
-    auto finish = [&](size_t c) {
+    auto finish = [&](int c) {
         Column& col = cols[c];
-        build_dictionary((int)c);
-        ColumnStats st;
+        build_dictionary(c);
         for (size_t i = 0; i < col.tags.size(); ++i) {
-            u8 t = col.tags[i];
+            const u8 t = col.tags[i];
+            if (t > C_OTHER) N1_THROW(N1GPU_E_INVALID, "bad class byte %d", (int)t);
             if (t == C_FLOAT) {  // pre-shredded input may hold integral floats: canonicalise (NewValue)
                 double d; memcpy(&d, &col.payload[i], 8);
-                if (f_is_int(d)) { col.tags[i] = t = C_INT; col.payload[i] = go_i64(d); }
-                else {
-                    if (!st.has_float) { st.flt_min = st.flt_max = d; st.has_float = true; }
-                    else { st.flt_min = std::min(st.flt_min, d); st.flt_max = std::max(st.flt_max, d); }
-                }
+                if (f_is_int(d)) { col.tags[i] = C_INT; col.payload[i] = go_i64(d); }
             }
-            if (t == C_INT) {
-                i64 v = col.payload[i];
-                if (!st.has_int) { st.int_min = st.int_max = v; st.has_int = true; }
-                else { st.int_min = std::min(st.int_min, v); st.int_max = std::max(st.int_max, v); }
-            }
-            if (t > C_OTHER) N1_THROW(N1GPU_E_INVALID, "bad class byte %d", (int)t);
-            st.class_mask |= bit(t);
-            st.absent_rows += t <= C_NULL;
         }
-        st.ndict = (i64)col.dict.size();
-        st.empty_rank = (!col.dict.empty() && col.dict[0].empty()) ? 0 : -1;
-        if (!col.stats_forced) col.stats = st;
-        u32 m = col.stats.class_mask;
-        col.width = (m & M_NUM) ? 8 : ((m & bit(C_STRING)) ? 4 : 0);
+        if (!col.stats_forced) { col.stats = host_stats(col.tags, col.payload); col.stats.set_dictionary(col.dict); }
+        col.width = width_of(col.stats.class_mask);
     };
-    {
-        std::vector<std::thread> pool;
-        std::vector<std::string> errs(cols.size());
-        for (size_t c = 0; c < cols.size(); ++c)
-            pool.emplace_back([&, c] { try { finish(c); } catch (const std::exception& e) { errs[c] = e.what(); } });
-        for (auto& th : pool) th.join();
-        for (auto& e : errs) if (!e.empty()) N1_THROW(N1GPU_E_INVALID, "%s", e.c_str());
+    try {
+        parallel_for((int)cols.size(), finish);
+    } catch (const std::exception& e) {
+        N1_THROW(N1GPU_E_INVALID, "%s", e.what());
     }
     shred_sec += now_sec() - t0;
     if (!segment_out.empty()) write_segment();
@@ -521,24 +621,15 @@ void Table::seal() {
         sealed = true;
         return;
     }
-    i64 pad = padded_rows();
-    if (pad == 0) pad = ROW_PAD;
     for (auto& col : cols) {
-        col.d_tags.alloc((size_t)pad);
-        CK(cudaMemset(col.d_tags.p, C_MISSING, (size_t)pad));
+        col.d_tags = device_rows(1, C_MISSING, nullptr);
+        col.d_payload = device_rows(col.width, 0, nullptr);
         if (nrows) CK(cudaMemcpy(col.d_tags.p, col.tags.data(), (size_t)nrows, cudaMemcpyHostToDevice));
-        if (col.width == 8) {
-            col.d_payload.alloc((size_t)pad * 8);
-            CK(cudaMemset(col.d_payload.p, 0, (size_t)pad * 8));
-            if (nrows) CK(cudaMemcpy(col.d_payload.p, col.payload.data(), (size_t)nrows * 8, cudaMemcpyHostToDevice));
-        } else if (col.width == 4) {
+        if (col.width == 8 && nrows) CK(cudaMemcpy(col.d_payload.p, col.payload.data(), (size_t)nrows * 8, cudaMemcpyHostToDevice));
+        if (col.width == 4 && nrows) {
             std::vector<u32> narrow((size_t)nrows);
             for (i64 i = 0; i < nrows; ++i) narrow[(size_t)i] = (u32)col.payload[(size_t)i];
-            col.d_payload.alloc((size_t)pad * 4);
-            CK(cudaMemset(col.d_payload.p, 0, (size_t)pad * 4));
-            if (nrows) CK(cudaMemcpy(col.d_payload.p, narrow.data(), (size_t)nrows * 4, cudaMemcpyHostToDevice));
-        } else {
-            col.d_payload.alloc(256);
+            CK(cudaMemcpy(col.d_payload.p, narrow.data(), (size_t)nrows * 4, cudaMemcpyHostToDevice));
         }
         std::vector<i64>().swap(col.payload);
         std::vector<u8>().swap(col.tags);

@@ -45,13 +45,26 @@ struct ColumnStats {
     u32 class_mask = 0;  // classes that occur (bit per C_*)
     bool has_int = false;
     i64 int_min = 0, int_max = 0;
-    bool has_float = false;
-    double flt_min = 0, flt_max = 0;
+    bool has_float = false;  // a FLOAT that is not integral occurs
     i64 ndict = 0;
     i64 empty_rank = -1;  // rank of "" in the dictionary, -1 if absent
     i64 absent_rows = 0;  // rows whose class is MISSING or NULL (decides which way a COUNT(x) counter counts)
     bool uniform_tag() const { return class_mask != 0 && (class_mask & (class_mask - 1)) == 0; }
+    void set_dictionary(const SharedDict& d) { ndict = (i64)d.size(); empty_rank = (!d.empty() && d[0].empty()) ? 0 : -1; }
 };
+
+// Statistics of staged host rows (the dictionary's aside).  An integral FLOAT counts as the INT it canonicalises to
+// (NewValue); the rows are left as they are.
+ColumnStats host_stats(const std::vector<u8>& tags, const std::vector<i64>& payload);
+
+// Device payload width of a column whose classes are `class_mask`: 8 with numbers, 4 (string ranks) with strings, else 0.
+// seal() applies it to the column's statistics - those of all partitions when stats_set replaced them - while the device
+// shredder and set_column_device apply it to the classes of their own rows: two partitions whose rows differ in classes
+// can then give a device-shredded column different widths.
+inline int width_of(u32 class_mask) { return (class_mask & M_NUM) ? 8 : (class_mask & bit(C_STRING)) ? 4 : 0; }
+
+// The strings of a caller's dictionary (blob + offsets), which must be sorted bytewise and unique (`what` names it)
+std::vector<std::string> read_dictionary(const char* blob, const i64* offs, i64 n, const char* what);
 
 struct Column {
     std::vector<std::string> path;       // field names below the document root
@@ -59,14 +72,13 @@ struct Column {
     std::vector<i64> payload;            // 8 bytes per row while staging
     std::vector<u8> tags;
     SharedDict dict;                     // sorted, unique (after seal / import); results keep it alive (share())
-    bool dict_global = false;            // dictionary imported (multi-GPU): do not rebuild at seal
     std::vector<std::string> local_strings;  // staging: distinct strings, codes index this until seal
-    bool codes_are_ranks = false;        // set_column supplied ranks into `dict` already
+    bool dict_staged = true;             // STRING rows hold codes into local_strings, not ranks into dict (build_dictionary)
     ColumnStats stats;
     bool stats_forced = false;
     int width = 8;                       // device payload width: 8, 4 or 0
     DevBuf d_payload, d_tags;
-    bool device_set = false;             // filled by set_column_device
+    bool on_device = false;              // filled by set_column_device
 };
 
 // What the file a directory entry's row is read from (<id>.json, file.go:711-749) looked like when it was read or
@@ -94,7 +106,18 @@ struct Table {
     i64 nrows = 0;
     i64 global_rows = 0;  // rows of the whole keyspace over all partitions (0 = not declared)
     bool sealed = false;
-    bool appended = false;
+    // How the rows got in so far; which entry point may follow is decided by admit() alone
+    enum class Fill : u8 {
+        EMPTY,
+        HOST_DOCS,       // append_json / load_dir / load_ndjson on host threads, or load_segment: rows staged, seal() uploads
+        HOST_COLUMNS,    // set_column: rows staged, seal() uploads
+        DEVICE_DOCS,     // the device shredder or a splice: columns final in HBM
+        DEVICE_COLUMNS,  // set_column_device: columns in HBM, seal() checks that every one was set
+    };
+    Fill filled = Fill::EMPTY;
+    bool rows_in_hbm() const { return filled == Fill::DEVICE_DOCS || filled == Fill::DEVICE_COLUMNS; }
+    enum class Entry { ADD_COLUMN, APPEND_HOST, APPEND_DEVICE, SET_COLUMN, SET_COLUMN_DEVICE, LOAD_SEGMENT, SPLICE };
+    void admit(Entry e, int col = -1) const;  // refuses `e` (on column `col`) when it may not follow what filled the table
     double shred_sec = 0, upload_sec = 0;
     i64 json_bytes = 0;
 
@@ -104,8 +127,6 @@ struct Table {
     void write_segment(const std::string& file, const std::string& source) const;
     bool load_segment(const std::string& file, const std::string& source);
     void load_ndjson(const std::string& file, int threads);  // one document per line; threads as for load_dir
-
-    bool device_shredded = false;  // columns were produced in HBM by shred.cu (no host staging exists)
 
     // threads >= 0: host threads (0 = all cores); threads == -1: the device shredder (shred.cu)
     void append_json_device(const char* buf, const i64* offsets, i64 ndocs);
@@ -134,13 +155,24 @@ struct Table {
     void set_column_device(int col, int width, const void* dev_payload, const u8* dev_tags, i64 nrows, const char* blob,
                            const i64* offs, i64 ndict);
     void build_dictionary(int col);  // local strings -> sorted dict, codes -> ranks
+    // Dictionary exchange (multi-GPU), before seal: the column whose dictionary is exchanged, its dictionary built
+    Column& exchange_column(int col);
+    // The column's dictionary becomes `n` sorted strings that every partition agrees on (a superset of its own) /
+    // the k-way merge of the given sorted dictionaries with its own
+    void import_dictionary(int col, const char* blob, const i64* offs, i64 n);
+    void merge_dictionaries(int col, int nparts, const char* const* blobs, const i64* const* offs, const i64* ns);
     // Replaces the column's (sorted) dictionary by a sorted superset and remaps the rows' ranks - staged on the host, or
-    // already in HBM (device shredder, set_column_device).  Multi-GPU: the dictionary every partition agrees on.
+    // already in HBM (device shredder, set_column_device).
     void adopt_dictionary(int col, std::vector<std::string>& global);
     void remap_ranks_device(int col, const std::vector<u32>& remap);  // rows of a column resident in HBM: rank -> remap[rank]
     void seal();
     int scan_bytes(int col) const;
     i64 padded_rows() const { return (nrows + ROW_PAD - 1) / ROW_PAD * ROW_PAD; }
+    // A device column: padded_rows() (at least ROW_PAD) entries of `width` bytes, every byte `byte`, on stream `s` (MISSING
+    // tags, zero payload); a payload of width 0 is a 256-byte stub
+    DevBuf device_rows(int width, int byte, cudaStream_t s) const;
+private:
+    void check_column_args(int col, int width, i64 n) const;  // set_column / set_column_device
 };
 
 // The host shredder applied to selected documents (the device shredder's fix-up rows).  Per column: tags[n],

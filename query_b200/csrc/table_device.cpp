@@ -4,7 +4,6 @@
 // are re-shredded on the host (fix-up rows) and patched in.
 #include <algorithm>
 #include <cstdlib>
-#include <map>
 #include <functional>
 #include <thread>
 
@@ -53,6 +52,35 @@ void build_trie(const std::vector<Column>& cols, ShredTrie& T) {
 
 u64 pow2_at_least(u64 n) { u64 p = 1; while (p < n) p <<= 1; return p; }
 
+// A column in device memory: class bytes and, for 8-byte payloads, the payload words (k_col_stats reads those of INT rows)
+struct DevColumn { const u8* tags; const i64* pay8; i64 rows; };
+
+// Statistics of device columns (the dictionary's aside), k_col_stats on `s` - one round trip for all of them
+std::vector<ColumnStats> device_stats(const std::vector<DevColumn>& cols, cudaStream_t s) {
+    const size_t n = cols.size();
+    if (!n) return {};
+    std::vector<u64> w(n * 8, 0);  // per column: class mask, int min, int max, has float, absent rows, (unused)
+    for (size_t c = 0; c < n; ++c) { w[c * 8 + 1] = (u64)INT64_MAX; w[c * 8 + 2] = (u64)INT64_MIN; }
+    DevBuf d;
+    d.alloc(n * 64);
+    CK(cudaMemcpyAsync(d.p, w.data(), n * 64, cudaMemcpyHostToDevice, s));
+    for (size_t c = 0; c < n; ++c)
+        if (cols[c].rows) launch_col_stats(cols[c].tags, cols[c].pay8, cols[c].rows, d.as<u64>() + c * 8, s);
+    CK(cudaMemcpyAsync(w.data(), d.p, n * 64, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    std::vector<ColumnStats> out(n);
+    for (size_t c = 0; c < n; ++c) {
+        const u64* x = &w[c * 8];
+        ColumnStats& st = out[c];
+        st.class_mask = (u32)x[0];
+        st.has_int = (st.class_mask & bit(C_INT)) != 0;
+        if (st.has_int) { st.int_min = (i64)x[1]; st.int_max = (i64)x[2]; }
+        st.has_float = x[3] != 0;
+        st.absent_rows = (i64)x[4];
+    }
+    return out;
+}
+
 }  // namespace
 
 void Table::append_json_device(const char* buf, const i64* offsets, i64 ndocs) {
@@ -66,14 +94,11 @@ void Table::append_ndjson_device(const char* text, i64 size, const std::function
 
 void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i64 text_size, const std::function<void(i64, i64)>& fill) {
     const bool lines = offsets == nullptr;  // NDJSON: offsets come from the device
-    if (sealed) N1_THROW(N1GPU_E_INVALID, "table is sealed");
-    if (!have_device()) N1_THROW(N1GPU_E_CUDA, "the device shredder needs a CUDA device (there is no CPU fallback for it; use host threads explicitly)");
-    if (appended || nrows != 0) N1_THROW(N1GPU_E_INVALID, "the device shredder takes the whole keyspace in one append");
+    admit(Entry::APPEND_DEVICE);
     if (cols.empty() && lines) N1_THROW(N1GPU_E_INVALID, "a table without columns cannot split lines on the device");
     if (cols.empty()) {  // a chain that references no field (COUNT(*) only): rows are all that matters
         nrows = ndocs;
-        appended = true;
-        device_shredded = true;
+        filled = Fill::DEVICE_DOCS;
         return;
     }
     double t0 = now_sec();
@@ -132,16 +157,13 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
     }
 
     nrows = ndocs;
-    i64 pad = padded_rows();
-    if (pad == 0) pad = ROW_PAD;
+    const i64 pad = std::max(padded_rows(), ROW_PAD);
     std::vector<DevBuf> pay8((size_t)ncols);
     std::vector<u8*> h_tags((size_t)ncols);
     std::vector<i64*> h_pay((size_t)ncols);
     for (int c = 0; c < ncols; ++c) {
-        cols[c].d_tags.alloc((size_t)pad);
-        CK(cudaMemsetAsync(cols[c].d_tags.p, C_MISSING, (size_t)pad, s));
-        pay8[c].alloc((size_t)pad * 8);
-        CK(cudaMemsetAsync(pay8[c].p, 0, (size_t)pad * 8, s));
+        cols[c].d_tags = device_rows(1, C_MISSING, s);
+        pay8[c] = device_rows(8, 0, s);
         h_tags[c] = cols[c].d_tags.as<u8>();
         h_pay[c] = pay8[c].as<i64>();
     }
@@ -251,15 +273,9 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
 
     phase("fix-up rows");
     // ---- statistics (class mask, int range) -------------------------------------------------------------------------
-    DevBuf d_stats;
-    d_stats.alloc((size_t)ncols * 64);
-    std::vector<u64> h_stats((size_t)ncols * 8, 0);
-    for (int c = 0; c < ncols; ++c) { h_stats[c * 8 + 1] = (u64)INT64_MAX; h_stats[c * 8 + 2] = (u64)INT64_MIN; }
-    CK(cudaMemcpyAsync(d_stats.p, h_stats.data(), h_stats.size() * 8, cudaMemcpyHostToDevice, s));
-    if (ndocs)
-        for (int c = 0; c < ncols; ++c) launch_col_stats(cols[c].d_tags.as<u8>(), pay8[c].as<i64>(), ndocs, d_stats.as<u64>() + c * 8, s);
-    CK(cudaMemcpyAsync(h_stats.data(), d_stats.p, h_stats.size() * 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    std::vector<DevColumn> dc;
+    for (int c = 0; c < ncols; ++c) dc.push_back(DevColumn{cols[c].d_tags.as<u8>(), pay8[c].as<i64>(), ndocs});
+    std::vector<ColumnStats> stats = device_stats(dc, s);
 
     phase("statistics");
     // ---- dictionaries + final payload width ------------------------------------------------------------------------------
@@ -268,16 +284,10 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
     d_count.alloc(64);
     for (int c = 0; c < ncols; ++c) {
         Column& col = cols[c];
-        ColumnStats st;
-        st.class_mask = (u32)h_stats[c * 8 + 0];
-        st.has_int = (st.class_mask & bit(C_INT)) != 0;
-        st.int_min = st.has_int ? (i64)h_stats[c * 8 + 1] : 0;
-        st.int_max = st.has_int ? (i64)h_stats[c * 8 + 2] : 0;
-        st.has_float = h_stats[c * 8 + 3] != 0;
-        st.absent_rows = (i64)h_stats[c * 8 + 4];
+        ColumnStats& st = stats[c];
         col.dict.clear();
         const bool has_str = st.class_mask & bit(C_STRING);
-        col.width = (st.class_mask & M_NUM) ? 8 : (has_str ? 4 : 0);
+        col.width = width_of(st.class_mask);
         if (has_str) {
             d_slots.ensure((size_t)pad * 8);
             // (a sparse table is cheap - 8 bytes per slot, cleared by a memset - a dense one costs string compares per probe)
@@ -326,15 +336,8 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
             std::vector<u32> starts(nent + 1, 0);
             for (size_t i = 0; i < nent; ++i) starts[i + 1] = starts[i] + (u32)(orefs[i] & 0xffffff);
             std::string compact((size_t)starts[nent], '\0');
-            const size_t nthr = nent < 20000 ? 1 : std::min<size_t>(std::max(1u, std::thread::hardware_concurrency()), 16);
-            auto parallel = [&](size_t parts, const std::function<void(size_t)>& fn) {
-                if (parts <= 1) { fn(0); return; }
-                std::vector<std::thread> pool;
-                for (size_t r = 1; r < parts; ++r) pool.emplace_back(fn, r);
-                fn(0);
-                for (auto& th : pool) th.join();
-            };
-            parallel(nthr, [&](size_t r) {
+            const int nthr = nent < 20000 ? 1 : (int)std::min<size_t>(std::max(1u, std::thread::hardware_concurrency()), 16);
+            parallel_for(nthr, [&](size_t r) {
                 for (size_t i = nent * r / nthr; i < nent * (r + 1) / nthr; ++i) {
                     const u64 ref = orefs[i];
                     const u64 off = (ref & ~0x8000000000000000ULL) >> 24;
@@ -357,7 +360,7 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
             if (nthr > 1) {
                 // sample sort: buckets by splitters drawn from the prefixes (equal prefixes share a bucket), every bucket sorted on
                 // its own core - no merge levels.  Strings that all share their first 8 bytes degenerate to one bucket.
-                const size_t B = nthr, S = 64 * B;
+                const size_t B = (size_t)nthr, S = 64 * B;
                 std::vector<u64> sample(S);
                 for (size_t i = 0; i < S; ++i) sample[i] = ents[nent * i / S].prefix;
                 std::sort(sample.begin(), sample.end());
@@ -365,7 +368,7 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
                 for (size_t k = 0; k + 1 < B; ++k) split[k] = sample[(k + 1) * S / B];
                 std::vector<u32> bucket(nent);
                 std::vector<std::vector<size_t>> cnt(B, std::vector<size_t>(B, 0));  // [thread][bucket]
-                parallel(B, [&](size_t r) {
+                parallel_for(nthr, [&](size_t r) {
                     for (size_t i = nent * r / B; i < nent * (r + 1) / B; ++i) {
                         const u32 k = (u32)(std::upper_bound(split.begin(), split.end(), ents[i].prefix) - split.begin());
                         bucket[i] = k;
@@ -377,13 +380,13 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
                 for (size_t k = 0; k < B; ++k) { size_t tot = 0; for (size_t r = 0; r < B; ++r) tot += cnt[r][k]; count[k + 1] = count[k] + tot; }
                 phase("    buckets counted");
                 std::vector<Ent> sorted(nent);
-                parallel(B, [&](size_t r) {
+                parallel_for(nthr, [&](size_t r) {
                     std::vector<size_t> cursor(B);
                     for (size_t k = 0; k < B; ++k) { size_t at = count[k]; for (size_t q = 0; q < r; ++q) at += cnt[q][k]; cursor[k] = at; }
                     for (size_t i = nent * r / B; i < nent * (r + 1) / B; ++i) sorted[cursor[bucket[i]]++] = ents[i];
                 });
                 phase("    buckets filled");
-                parallel(B, [&](size_t k) { std::sort(sorted.begin() + (i64)count[k], sorted.begin() + (i64)count[k + 1], less); });
+                parallel_for(nthr, [&](size_t k) { std::sort(sorted.begin() + (i64)count[k], sorted.begin() + (i64)count[k + 1], less); });
                 ents.swap(sorted);
             } else {
                 std::sort(ents.begin(), ents.end(), less);
@@ -392,7 +395,7 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
             // rank of every occupied slot: the (few) slots travel in rank order and a kernel scatters their ranks
             std::vector<u64> slot_of_rank(ents.size());
             col.dict.resize(ents.size());
-            parallel(nthr, [&](size_t t) {
+            parallel_for(nthr, [&](size_t t) {
                 for (size_t r = ents.size() * t / nthr; r < ents.size() * (t + 1) / nthr; ++r) {
                     slot_of_rank[r] = ents[r].slot;
                     col.dict[r].assign(cb + ents[r].at, ents[r].len);
@@ -405,8 +408,7 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
             launch_dict_ranks(d_oslots.as<u64>(), (u64)slot_of_rank.size(), d_rank.as<u32>(), s);
             u32* out32 = nullptr;
             if (col.width == 4) {
-                col.d_payload.alloc((size_t)pad * 4);
-                CK(cudaMemsetAsync(col.d_payload.p, 0, (size_t)pad * 4, s));
+                col.d_payload = device_rows(4, 0, s);
                 out32 = col.d_payload.as<u32>();
             }
             launch_dict_remap(col.d_tags.as<u8>(), d_slots.as<i64>(), pay8[c].as<i64>(), out32, ndocs, d_rank.as<u32>(), s);
@@ -414,22 +416,20 @@ void Table::append_text_device(const char* buf, const i64* offsets, i64 ndocs, i
             phase("  dictionary remap");
         }
         if (col.width == 8) col.d_payload = std::move(pay8[c]);
-        else { pay8[c].release(); if (col.width == 0) col.d_payload.alloc(256); }
-        st.ndict = (i64)col.dict.size();
-        st.empty_rank = (!col.dict.empty() && col.dict[0].empty()) ? 0 : -1;
+        else { pay8[c].release(); if (col.width == 0) col.d_payload = device_rows(0, 0, s); }
+        st.set_dictionary(col.dict);
         if (!col.stats_forced) col.stats = st;
-        col.codes_are_ranks = true;
+        col.dict_staged = false;
     }
     phase("dictionaries");
-    appended = true;
-    device_shredded = true;
+    filled = Fill::DEVICE_DOCS;
     json_bytes += nbytes;
     shred_sec += now_sec() - t0;
 }
 
 void Table::splice(const Table& old, const Table* patch, const std::vector<SpliceRun>& runs) {
     if (!have_device()) N1_THROW(N1GPU_E_CUDA, "splicing columns needs a CUDA device");
-    if (sealed || appended || nrows) N1_THROW(N1GPU_E_INVALID, "a splice fills an empty, unsealed table");
+    admit(Entry::SPLICE);
     if (old.cols.size() != cols.size() || (patch && patch->cols.size() != cols.size())) N1_THROW(N1GPU_E_INVALID, "splice sources have other columns");
     const double t0 = now_sec();
     const size_t R = runs.size();
@@ -444,16 +444,14 @@ void Table::splice(const Table& old, const Table* patch, const std::vector<Splic
     }
     nrows = R ? runs.back().new_lo + runs.back().len : 0;
     h_runs[R] = nrows;
-    i64 pad = padded_rows();
-    if (pad == 0) pad = ROW_PAD;
+    const i64 pad = std::max(padded_rows(), ROW_PAD);
     cudaStream_t s = nullptr;
     CK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamDestroy(s); } } sg{s};
-    DevBuf d_runs, d_used, d_stats, d_oremap, d_premap;
+    DevBuf d_runs, d_used, d_oremap, d_premap;
     d_runs.alloc(h_runs.size() * 8);
     CK(cudaMemcpyAsync(d_runs.p, h_runs.data(), h_runs.size() * 8, cudaMemcpyHostToDevice, s));
     const SpliceRuns sr{d_runs.as<i64>(), d_runs.as<i64>() + R + 1, (i64)R, nrows};
-    d_stats.alloc(64);
     auto pay8 = [](const Column& c) { return c.width == 8 ? c.d_payload.as<i64>() : nullptr; };
     auto pay4 = [](const Column& c) { return c.width == 4 ? c.d_payload.as<u32>() : nullptr; };
     for (size_t c = 0; c < cols.size(); ++c) {
@@ -492,35 +490,26 @@ void Table::splice(const Table& old, const Table* patch, const std::vector<Splic
             if (take_patch) premap[j++] = rank;
         }
         col.dict = std::move(dict);
-        col.width = (mask & M_NUM) ? 8 : ((mask & bit(C_STRING)) ? 4 : 0);
+        col.width = width_of((u32)mask);
         d_oremap.ensure(std::max<size_t>(oremap.size() * 4, 64));
         d_premap.ensure(std::max<size_t>(premap.size() * 4, 64));
         if (!oremap.empty()) CK(cudaMemcpyAsync(d_oremap.p, oremap.data(), oremap.size() * 4, cudaMemcpyHostToDevice, s));
         if (!premap.empty()) CK(cudaMemcpyAsync(d_premap.p, premap.data(), premap.size() * 4, cudaMemcpyHostToDevice, s));
-        col.d_tags.alloc((size_t)pad);
-        col.d_payload.alloc(col.width ? (size_t)pad * (size_t)col.width : 256);
+        col.d_tags = device_rows(1, C_MISSING, s);
+        col.d_payload = device_rows(col.width, 0, s);
         launch_splice_gather(sr, pad, oc.d_tags.as<u8>(), pay8(oc), pay4(oc), d_oremap.as<u32>(), pc ? pc->d_tags.as<u8>() : nullptr,
                              pc ? pay8(*pc) : nullptr, pc ? pay4(*pc) : nullptr, d_premap.as<u32>(), col.d_tags.as<u8>(), pay8(col), pay4(col), s);
-        // statistics of the spliced column, as the device shredder computes them
-        u64 h_stats[8] = {0, (u64)INT64_MAX, (u64)INT64_MIN, 0, 0, 0, 0, 0};
-        CK(cudaMemcpyAsync(d_stats.p, h_stats, 64, cudaMemcpyHostToDevice, s));
-        if (nrows) launch_col_stats(col.d_tags.as<u8>(), pay8(col), nrows, d_stats.as<u64>(), s);
-        CK(cudaMemcpyAsync(h_stats, d_stats.p, 64, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        ColumnStats st;
-        st.class_mask = (u32)h_stats[0];
-        st.has_int = (st.class_mask & bit(C_INT)) != 0;
-        st.int_min = st.has_int ? (i64)h_stats[1] : 0;
-        st.int_max = st.has_int ? (i64)h_stats[2] : 0;
-        st.has_float = h_stats[3] != 0;
-        st.absent_rows = (i64)h_stats[4];
-        st.ndict = (i64)col.dict.size();
-        st.empty_rank = (!col.dict.empty() && col.dict[0].empty()) ? 0 : -1;
-        col.stats = st;
-        col.codes_are_ranks = true;
+        col.dict_staged = false;
     }
-    appended = true;
-    device_shredded = true;
+    // statistics of the spliced columns, as the device shredder computes them
+    std::vector<DevColumn> dc;
+    for (auto& col : cols) dc.push_back(DevColumn{col.d_tags.as<u8>(), pay8(col), nrows});
+    std::vector<ColumnStats> stats = device_stats(dc, s);
+    for (size_t c = 0; c < cols.size(); ++c) {
+        cols[c].stats = stats[c];
+        cols[c].stats.set_dictionary(cols[c].dict);
+    }
+    filled = Fill::DEVICE_DOCS;
     sealed = true;
     splice_sec += now_sec() - t0;
 }
@@ -538,64 +527,38 @@ void Table::remap_ranks_device(int ci, const std::vector<u32>& remap) {
 void Table::set_column_device(int c, int width, const void* dev_payload, const u8* dev_tags, i64 n, const char* blob,
                               const i64* offs, i64 ndict) {
     if (!have_device()) N1_THROW(N1GPU_E_CUDA, "no CUDA device: device columns need one");
-    if (sealed) N1_THROW(N1GPU_E_INVALID, "table is sealed");
-    if (c < 0 || c >= (int)cols.size()) N1_THROW(N1GPU_E_INVALID, "no such column %d", c);
-    if (width != 8 && width != 4) N1_THROW(N1GPU_E_INVALID, "payload width must be 8 or 4");
-    if (n < 0) N1_THROW(N1GPU_E_INVALID, "negative row count");
-    if (appended) N1_THROW(N1GPU_E_INVALID, "cannot mix appended documents and pre-shredded columns");
-    for (auto& other : cols) {
-        if (&other == &cols[c]) continue;
-        if (!other.tags.empty()) N1_THROW(N1GPU_E_INVALID, "cannot mix host and device columns in one table");
-        if (other.device_set && nrows != n) N1_THROW(N1GPU_E_INVALID, "column lengths differ (%lld vs %lld)", (long long)nrows, (long long)n);
-    }
+    admit(Entry::SET_COLUMN_DEVICE, c);
+    check_column_args(c, width, n);
+    for (auto& other : cols)
+        if (&other != &cols[c] && other.on_device && nrows != n)
+            N1_THROW(N1GPU_E_INVALID, "column lengths differ (%lld vs %lld)", (long long)nrows, (long long)n);
+    std::vector<std::string> dict;
+    if (blob && offs) dict = read_dictionary(blob, offs, ndict, "dictionary");
     Column& col = cols[c];
     nrows = n;
-    i64 pad = padded_rows();
-    if (pad == 0) pad = ROW_PAD;
-    col.d_tags.alloc((size_t)pad);
-    CK(cudaMemset(col.d_tags.p, C_MISSING, (size_t)pad));
+    col.d_tags = device_rows(1, C_MISSING, nullptr);
     if (n) {
         if (dev_tags) CK(cudaMemcpy(col.d_tags.p, dev_tags, (size_t)n, cudaMemcpyDeviceToDevice));
         else CK(cudaMemset(col.d_tags.p, width == 8 ? C_INT : C_STRING, (size_t)n));
     }
-    col.d_payload.alloc((size_t)pad * width);
-    CK(cudaMemset(col.d_payload.p, 0, (size_t)pad * width));
+    col.d_payload = device_rows(width, 0, nullptr);
     if (n) CK(cudaMemcpy(col.d_payload.p, dev_payload, (size_t)n * width, cudaMemcpyDeviceToDevice));
-    col.dict.clear();
-    if (blob && offs) {
-        for (i64 i = 0; i < ndict; ++i) col.dict.emplace_back(blob + offs[i], blob + offs[i + 1]);
-        for (size_t i = 1; i < col.dict.size(); ++i)
-            if (!(col.dict[i - 1] < col.dict[i])) N1_THROW(N1GPU_E_INVALID, "dictionary must be sorted bytewise and unique");
-    }
-    col.codes_are_ranks = true;
+    col.dict = std::move(dict);
+    col.dict_staged = false;
     // canonical numbers + statistics, on the device
     if (width == 8) launch_canon_floats(col.d_tags.as<u8>(), col.d_payload.as<i64>(), n, nullptr);
-    DevBuf d_stats;
-    d_stats.alloc(64);
-    u64 h_stats[8] = {0, (u64)INT64_MAX, (u64)INT64_MIN, 0, 0, 0, 0, 0};
-    CK(cudaMemcpy(d_stats.p, h_stats, 64, cudaMemcpyHostToDevice));
     // a 4-byte column holds string ranks only: the kernel reads payload words of INT rows, of which there are none
-    if (n) launch_col_stats(col.d_tags.as<u8>(), width == 8 ? col.d_payload.as<i64>() : nullptr, n, d_stats.as<u64>(), nullptr);
-    CK(cudaMemcpy(h_stats, d_stats.p, 64, cudaMemcpyDeviceToHost));
-    ColumnStats st;
-    st.class_mask = (u32)h_stats[0];
+    ColumnStats st = device_stats({DevColumn{col.d_tags.as<u8>(), width == 8 ? col.d_payload.as<i64>() : nullptr, n}}, nullptr)[0];
     if (st.class_mask >> (C_OTHER + 1)) N1_THROW(N1GPU_E_INVALID, "bad class byte in column %d", c);
     if (width == 4 && (st.class_mask & M_NUM)) N1_THROW(N1GPU_E_INVALID, "a 4-byte column cannot hold numbers");
     if (width == 8 && !(st.class_mask & M_NUM) && (st.class_mask & bit(C_STRING)))
         N1_THROW(N1GPU_E_INVALID, "a column of strings only must be passed as 4-byte ranks");
-    st.has_int = (st.class_mask & bit(C_INT)) != 0;
-    st.int_min = st.has_int ? (i64)h_stats[1] : 0;
-    st.int_max = st.has_int ? (i64)h_stats[2] : 0;
-    st.has_float = h_stats[3] != 0;
-    st.absent_rows = (i64)h_stats[4];
-    st.ndict = (i64)col.dict.size();
-    st.empty_rank = (!col.dict.empty() && col.dict[0].empty()) ? 0 : -1;
+    st.set_dictionary(col.dict);
     if (!col.stats_forced) col.stats = st;
-    const u32 m = col.stats.class_mask;
-    col.width = (m & M_NUM) ? 8 : ((m & bit(C_STRING)) ? 4 : 0);
-    if (col.width == 0) col.d_payload.alloc(256);
-    col.device_set = true;
-    device_shredded = true;  // nothing left to do at seal
+    col.width = width_of(col.stats.class_mask);
+    if (col.width == 0) col.d_payload = device_rows(0, 0, nullptr);
+    col.on_device = true;
+    filled = Fill::DEVICE_COLUMNS;  // nothing left to do at seal
 }
 
 }  // namespace n1
