@@ -177,7 +177,8 @@ const char* n1gpu_query_kernel_source(const n1gpu_query* q);
 /* The partitioning kernel of a chain that runs as a partitioned DISTINCT aggregation ("" otherwise): many groups, one
  * DISTINCT operand of few bits, no other per-row accumulator than COUNT(*) - BASELINE config 4's shape.                */
 const char* n1gpu_query_part_source(const n1gpu_query* q);
-/* info[0]=mode (0 ungrouped, 1 dense shared-memory table, 2 HBM hash 64-bit keys, 3 HBM hash 128-bit)
+/* info[0]=mode (0 ungrouped, 1 dense shared-memory table, 2 HBM hash 64-bit keys, 3 HBM hash 128-bit, 4 HBM
+ *           direct-indexed, 5 HBM hash of keys wider than 127 bits: KW = ceil(key bits / 64) words per group)
  * info[1]=accumulator words per group  info[2]=registers/thread  info[3]=grid  info[4]=block
  * info[5]=scan bytes per row  info[6]=static shared bytes  info[7]=dense slots / hash capacity      */
 int n1gpu_query_info(const n1gpu_query* q, int64_t info[8]);
@@ -201,8 +202,10 @@ int n1gpu_query_free(n1gpu_query* q);
  * One process per GPU.  Each rank scans its row range and exports its partial groups as fixed-size
  * records in DEVICE memory; the caller moves records between ranks (NCCL all-to-all / all-gather over
  * NVLink - torch.distributed in this repo, ncclSend/Recv from Go); the owner imports and finalises.
- * Record layout: record_words 64-bit words = [key_lo, key_hi, acc words...]; DISTINCT entries travel
- * as 2-word records [lo, hi].  owner(record) = mix(key) % nranks, computed by partial_partition.     */
+ * Record layout: record_words 64-bit words = [key_lo, key_hi, acc words...]; a chain of mode 5 (keys wider than
+ * 127 bits, never with DISTINCT) sends [k0 .. k(KW-1), acc words...] instead, record_words = KW + acc words.
+ * DISTINCT entries travel as 2-word records [lo, hi].  owner(record) = mix(key) % nranks, computed by
+ * partial_partition.                                                                                   */
 int n1gpu_query_scan_partial(n1gpu_query* q);                       /* scan only, state stays on device */
 int n1gpu_query_partial_counts(n1gpu_query* q, int64_t* ngroups, int64_t* ndistinct, int* record_words);
 /* Writes the partial groups, bucketed by owner rank, into dev_records (capacity in records) and the

@@ -375,7 +375,7 @@ class Result:
             pass
 
 
-MODES = {0: "ungrouped", 1: "dense-shared-memory", 2: "hbm-hash-64", 3: "hbm-hash-128", 4: "hbm-direct"}
+MODES = {0: "ungrouped", 1: "dense-shared-memory", 2: "hbm-hash-64", 3: "hbm-hash-128", 4: "hbm-direct", 5: "hbm-hash-wide"}
 
 
 class Query:

@@ -384,7 +384,7 @@ int n1gpu_query_partial_counts(n1gpu_query* q, int64_t* ngroups, int64_t* ndisti
         REQUIRE(q); REQUIRE(ngroups); REQUIRE(ndistinct); REQUIRE(record_words);
         i64 g = 0, d = 0;
         q->q->partial_counts(&g, &d);
-        *ngroups = g; *ndistinct = d; *record_words = 2 + q->q->ops.n;
+        *ngroups = g; *ndistinct = d; *record_words = q->q->record_words();
     });
 }
 int n1gpu_query_partial_export(n1gpu_query* q, int nranks, void* dev_records, int64_t cap_records, int64_t* counts,

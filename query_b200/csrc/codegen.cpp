@@ -11,6 +11,7 @@
 //                   copies for a handful of groups), else direct-indexed in HBM (dense_global) behind the
 //                   shared-memory front cache
 //   MODE_HASH64/128 an HBM open-addressing table claimed with 64-/128-bit CAS (64: behind the front cache)
+//   MODE_HASHW      the same for keys wider than 127 bits: a tag word claimed with a CAS, then the key words
 // DISTINCT aggregates add bit-packed (set, group, value) entries to a bitmap or an HBM hash set.
 // The planner (plan_layout and its stages) turns static type analysis (expr.cpp), column statistics and the N1GPU_*
 // knobs into the KernelPlan: which accumulator words exist, how wide keys and entries are, which layout above is
@@ -366,23 +367,25 @@ std::string payload_field(const PackComp& pc, const std::string& v) {
     return e;
 }
 
-// Emits code packing Val `v` as component pc into (lo,hi,pos) variables; with `radix` also adds the component's packed
-// value times `radix_stride` to the variable of that name (mixed-radix slot of a dense shared-memory table).
+// Emits code packing Val `v` as component pc into (lo,hi,pos) variables, or with hi == nullptr into the u64 array `lo`
+// (MODE_HASHW keys); with `radix` also adds the component's packed value times `radix_stride` to the variable of that
+// name (mixed-radix slot of a dense shared-memory table).
 void emit_pack(Gen& g, const PackComp& pc, const std::string& v, const char* lo, const char* hi, const char* pos,
                const char* radix = nullptr, u64 radix_stride = 0) {
+    const std::string dst = hi ? strf("%s, %s, %s", lo, hi, pos) : strf("%s, %s", lo, pos);
     if (radix && pc.bits() > 0) {
         // the whole component as one value: class index in the low cbits, payload above
         std::string cv = g.nv("cv");
         if (pc.nfree >= 0) g.line(strf("const u64 %s = %s;", cv.c_str(), offset_field(pc, v).c_str()));
         else g.line(strf("const u64 %s = %s | (%s << %d);", cv.c_str(), pc.cbits ? class_field(pc, v, "ULL").c_str() : "0ULL",
                          pc.pbits ? payload_field(pc, v).c_str() : "0ULL", pc.cbits));
-        g.line(strf("pack_bits(%s, %s, %s, %s, %d);", lo, hi, pos, cv.c_str(), pc.bits()));
+        g.line(strf("pack_bits(%s, %s, %d);", dst.c_str(), cv.c_str(), pc.bits()));
         g.line(strf("%s += %s * %lluULL;", radix, cv.c_str(), (unsigned long long)radix_stride));
         return;
     }
-    if (pc.nfree >= 0) { g.line(strf("pack_bits(%s, %s, %s, %s, %d);", lo, hi, pos, offset_field(pc, v).c_str(), pc.pbits)); return; }
-    if (pc.cbits) g.line(strf("pack_bits(%s, %s, %s, (u64)%s, %d);", lo, hi, pos, class_field(pc, v, "").c_str(), pc.cbits));
-    if (pc.pbits) g.line(strf("pack_bits(%s, %s, %s, %s, %d);", lo, hi, pos, payload_field(pc, v).c_str(), pc.pbits));
+    if (pc.nfree >= 0) { g.line(strf("pack_bits(%s, %s, %d);", dst.c_str(), offset_field(pc, v).c_str(), pc.pbits)); return; }
+    if (pc.cbits) g.line(strf("pack_bits(%s, (u64)%s, %d);", dst.c_str(), class_field(pc, v, "").c_str(), pc.cbits));
+    if (pc.pbits) g.line(strf("pack_bits(%s, %s, %d);", dst.c_str(), payload_field(pc, v).c_str(), pc.pbits));
 }
 
 double comp_domain(const Table& t, const PackComp& pc) {
@@ -666,7 +669,14 @@ void plan_mode(KernelPlan& kp, const Table& t, i64 layout_rows) {
         }
     }
     else if (kp.key_bits <= 127) kp.mode = MODE_HASH128;
-    else N1_THROW(N1GPU_E_INELIGIBLE, "group key needs %d bits (> 127) after packing", kp.key_bits);
+    else if (kp.keys.size() <= 16) {
+        // Two mixed INT / FLOAT columns already pack into 130 bits.  No front cache: its cells are keyed by one word, and
+        // without it there are neither packed nor complemented counters.  A DISTINCT entry would embed the whole key:
+        // plan_distinct refuses it (entry > 127 bits).
+        kp.mode = MODE_HASHW;
+        kp.key_words = (kp.key_bits + 63) / 64;
+    }
+    else N1_THROW(N1GPU_E_INELIGIBLE, "group key of %zu components needs %d bits (> 127) after packing", kp.keys.size(), kp.key_bits);
     kp.est_groups = (i64)std::min(est, 4e18);
     kp.min_blocks = min_blocks != 0 ? min_blocks : (kp.cache_slots > 0 ? cache_blocks : 0);
 }
@@ -823,7 +833,13 @@ RowCode emit_row_code(Gen& g, const KernelPlan& kp, const Expr* where, const std
     g.body.clear();
     const bool cached = kp.cache_slots > 0;
     g.ind = "                    ";
-    if (kp.mode != MODE_UNGROUPED) {
+    if (kp.mode == MODE_HASHW) {
+        // the key words stay in registers: every pack_bits index is a constant once the row code is unrolled
+        g.line(strf("u64 kwd[%d] = {}; int kpos = 0;", kp.key_words));
+        for (size_t k = 0; k < keys.size(); ++k) emit_pack(g, kp.keys[k], canon(g, *keys[k], g.emit(*keys[k], nullptr), "k"), "kwd", nullptr, "kpos");
+        g.line(strf("const i64 slot = table_insert_wide<%d>(p.keys, p.cap_mask, kwd);", kp.key_words));
+        g.line("if (slot < 0) { if (slot == -1) p.status[0] = 1; else p.status[1] = NQ_WIDE_STUCK; continue; }");
+    } else if (kp.mode != MODE_UNGROUPED) {
         g.line("u64 klo = 0, khi = 0; int kpos = 0;");
         const bool radix = !kp.dense_dom.empty();
         if (radix) g.line("u64 kslot = 0;");

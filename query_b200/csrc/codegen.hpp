@@ -10,7 +10,9 @@
 
 namespace n1 {
 
-enum : int { MODE_UNGROUPED = 0, MODE_DENSE = 1, MODE_HASH64 = 2, MODE_HASH128 = 3 };
+// MODE_HASHW (a key wider than 127 bits, KernelPlan::key_words words per group) is 5 because n1gpu_query_info reports a
+// direct-indexed MODE_DENSE table (KernelPlan::dense_global) as 4
+enum : int { MODE_UNGROUPED = 0, MODE_DENSE = 1, MODE_HASH64 = 2, MODE_HASH128 = 3, MODE_HASHW = 5 };
 enum : int { CK_CNT = 0, CK_WIDE = 1, CK_MM32 = 2, CK_OR32 = 3, CK_64 = 4, CK_WIDE1 = 5 };
 // threads per block of the partitioning kernel (KernelPlan::part), one block per SM.  Two 512-thread blocks with half
 // the bins each lost (config 4, 200 M rows: 1.59 -> 1.78 ms; four 256-thread blocks 2.55 ms; DESIGN.md section 9)
@@ -70,6 +72,8 @@ struct KernelPlan {
     int w_rows = -1;                     // the rows-per-group word (-1: none)
     std::vector<PackComp> keys;
     int key_bits = 0;
+    int key_words = 0;           // MODE_HASHW: 64-bit words of the packed key, ceil(key_bits / 64) (at most 17: 16
+                                 // components of 3 class bits and 64 payload bits)
     i64 dense_slots = 0;
     // shared-memory dense tables index slots by the mixed-radix number of the key components (TPC-H Q1: 3 x 2 = 6 slots
     // instead of the 2^3 = 8 of the bit-packed key); dense_dom[i] = values component i takes (empty: slot == packed key)

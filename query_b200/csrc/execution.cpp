@@ -739,7 +739,7 @@ std::string GpuGroupAggregate::MarshalJSON() const {
         s += "]";
     }
     if (query) {
-        static const char* modes[] = {"ungrouped", "dense-shared-memory", "hbm-hash-64", "hbm-hash-128"};
+        static const char* modes[] = {"ungrouped", "dense-shared-memory", "hbm-hash-64", "hbm-hash-128", "hbm-direct", "hbm-hash-wide"};
         s += std::string(",\"kernel\":{\"mode\":\"") + (query->kp.dense_global ? "hbm-direct" : modes[query->kp.mode]) + "\",\"accumulator_words\":" + std::to_string(query->ops.n) +
              ",\"scan_bytes_per_row\":" + std::to_string(query->kp.scan_bytes_per_row) + "}";
     }

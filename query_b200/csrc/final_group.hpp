@@ -66,8 +66,22 @@ N1_HD u64 take_bits(unsigned __int128& v, int n) {
     return r;
 }
 
-// the next component of a packed key or DISTINCT entry
-N1_HD Val decode_comp(const FinalComp& pc, unsigned __int128& bits) {
+// the next n bits of a key wider than 128 bits (MODE_HASHW): its key words w, low bits first, from bit pos on
+struct WordBits {
+    const u64* w;
+    int pos;
+};
+N1_HD u64 take_bits(WordBits& r, int n) {
+    if (n == 0) return 0;
+    const int i = r.pos >> 6, s = r.pos & 63;
+    u64 v = r.w[i] >> s;
+    if (s + n > 64) v |= r.w[i + 1] << (64 - s);
+    r.pos += n;
+    return n >= 64 ? v : (v & ((1ULL << n) - 1));
+}
+
+// the next component of a packed key or DISTINCT entry (bits: unsigned __int128 or WordBits)
+template <class Bits> N1_HD Val decode_comp(const FinalComp& pc, Bits& bits) {
     u64 ci = take_bits(bits, pc.cbits);
     u64 pv = take_bits(bits, pc.pbits);
     if (pc.nfree >= 0) {  // offset packing: one field
@@ -175,13 +189,14 @@ N1_HD Val final_agg(const FinalAgg& ap, const u64* w) {
     return {(seen & (1ULL << C_TRUE)) ? C_TRUE : C_FALSE, 0};
 }
 
-// FinalGroup of one group: its nkeys key components decoded from the packed key (khi:klo), its aggregates finalised from
-// its physical words pw, into key_cls / key_val [nkeys] and agg_cls / agg_val [D.naggs]
-N1_HD void final_group(const FinalDesc& D, const FinalComp* keys, int nkeys, u64 klo, u64 khi, const u64* pw, u8* key_cls,
-                       i64* key_val, u8* agg_cls, i64* agg_val) {
+// FinalGroup of one group: its nkeys key components decoded from the packed key kb (an unsigned __int128, or WordBits
+// over the words of a wide key), its aggregates finalised from its physical words pw, into key_cls / key_val [nkeys] and
+// agg_cls / agg_val [D.naggs]
+template <class Bits>
+N1_HD void final_group_bits(const FinalDesc& D, const FinalComp* keys, int nkeys, Bits kb, const u64* pw, u8* key_cls, i64* key_val,
+                            u8* agg_cls, i64* agg_val) {
     u64 w[64];
     logical_words(D, pw, w);
-    unsigned __int128 kb = ((unsigned __int128)khi << 64) | klo;
     for (int k = 0; k < nkeys; ++k) {
         const Val v = decode_comp(keys[k], kb);
         key_cls[k] = (u8)v.c;
@@ -192,6 +207,11 @@ N1_HD void final_group(const FinalDesc& D, const FinalComp* keys, int nkeys, u64
         agg_cls[a] = (u8)v.c;
         agg_val[a] = v.b;
     }
+}
+// a key of at most 128 bits (khi:klo)
+N1_HD void final_group(const FinalDesc& D, const FinalComp* keys, int nkeys, u64 klo, u64 khi, const u64* pw, u8* key_cls,
+                       i64* key_val, u8* agg_cls, i64* agg_val) {
+    final_group_bits(D, keys, nkeys, ((unsigned __int128)khi << 64) | klo, pw, key_cls, key_val, agg_cls, agg_val);
 }
 
 }  // namespace n1

@@ -35,7 +35,8 @@ __device__ __forceinline__ int owner_of(u64 lo, u64 hi, int nranks) {
 }
 
 // key of slot i and whether the slot holds a group.  kw: 0 dense (key = index, live iff word 0 > 0),
-// 1: u64 keys, 2: 128-bit keys, 3: single ungrouped slot (always live)
+// 1: u64 keys, 2: 128-bit keys, 3: single ungrouped slot (always live); wide tables (KW_WIDE + key words) have kernels of
+// their own (k_*_wide)
 __device__ __forceinline__ bool slot_key(int kw, const u64* keys, const u64* acc, u64 i, u64& lo, u64& hi) {
     if (kw == 0) { lo = i; hi = 0; return acc[i] != 0; }
     if (kw == 1) { lo = keys[i]; hi = 0; return lo != NQ_U64_MAX; }
@@ -172,6 +173,53 @@ __global__ void k_merge_records(int kw, u64* keys, u64* acc, u64 cap, OpsArr ops
     }
 }
 
+// ---- wide-key tables (MODE_HASHW): slot i is keys[i * (kw + 1) ..] = [tag, k0 .. k(kw-1)] (n1ql_device.cuh), a record is
+// [k0 .. k(kw-1), physical words].  Kernels of their own, so that the loops over key words stay out of the other paths.
+// The owner mixes the table hash once more: owner and home slot must not share bits (an owner's groups would crowd into
+// every nranks-th slot of its table).
+__device__ __forceinline__ int owner_wide(const u64* key, int kw, int nranks) {
+    return nranks <= 1 ? 0 : (int)(mix64(wide_hash(key, kw) ^ 0x9e3779b97f4a7c15ULL) % (u64)nranks);
+}
+__global__ void k_count_owners_wide(int kw, const u64* keys, u64 cap, int nranks, unsigned long long* counts) {
+    const u64 stride = (u64)gridDim.x * blockDim.x;
+    for (u64 i0 = (u64)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < cap; i0 += stride) {  // warp-uniform trip count
+        const u64 i = i0 + (threadIdx.x & 31);
+        const u64* s = keys + i * (u64)(kw + 1);
+        const bool live = i < cap && s[0] != NQ_U64_MAX;
+        warp_claim(counts, live ? owner_wide(s + 1, kw, nranks) : 0, live);
+    }
+}
+__global__ void k_export_records_wide(int kw, const u64* keys, const u64* acc, u64 cap, int W, int nranks, unsigned long long* cursor, u64* out,
+                                      u64 out_cap) {
+    const int rw = kw + W;
+    const u64 stride = (u64)gridDim.x * blockDim.x;
+    for (u64 i0 = (u64)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < cap; i0 += stride) {
+        const u64 i = i0 + (threadIdx.x & 31);
+        const u64* s = keys + i * (u64)(kw + 1);
+        const bool live = i < cap && s[0] != NQ_U64_MAX;
+        const u64 at = warp_claim(cursor, live ? owner_wide(s + 1, kw, nranks) : 0, live);
+        if (!live || at >= out_cap) continue;
+        u64* r = out + at * rw;
+        for (int k = 0; k < kw; ++k) r[k] = s[1 + k];
+        for (int w = 0; w < W; ++w) r[kw + w] = acc[(u64)w * cap + i];
+    }
+}
+__global__ void k_merge_records_wide(int kw, u64* keys, u64* acc, u64 cap, OpsArr ops, const u64* __restrict__ recs, u64 n, int* status) {
+    const int rw = kw + ops.n;
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        const u64* r = recs + i * rw;
+        const i64 slot = table_insert_wide_n(keys, cap - 1, r, kw);
+        if (slot < 0) {
+            if (slot == -1) status[0] = 1; else status[1] = NQ_WIDE_STUCK;
+            continue;
+        }
+        for (int w = 0; w < ops.n; ++w) {
+            const u64 v = r[kw + w];
+            if (v != word_identity(ops.op[w])) atomic_word_dyn(ops.op[w], &acc[(u64)w * cap + (u64)slot], v);
+        }
+    }
+}
+
 // DISTINCT finalisation (ComputeFinal of count/countn/sum/avg DISTINCT: algebra/agg_*_distinct.go): every entry of the
 // (aggregate, group, value) set adds 1 to its group's distinct count and, for SUM/AVG, its value to the group's exact
 // split integer sum / float sum.  kw: how the group slot is found (3 ungrouped, 0 dense, 1 / 2 hash 64 / 128).
@@ -281,6 +329,7 @@ __global__ void k_merge_mailbox(const u64* mail, int nranks, u64 slot_base, u64 
 // through a warp-aggregated cursor and finalised by final_group (final_group.hpp, the restatement of ComputeFinal and of
 // the key decoding that the host finalisation shares; execution/group_final.go:55-118 sends one item per group).  Strings
 // leave as (dictionary column << 40 | rank); the host resolves them.
+template <bool WIDE>
 __global__ void __launch_bounds__(256) k_finalize_groups(const FinalDesc D, int kw, const u64* __restrict__ keys, const PeerTables T, const OpsArr ops,
                                                          u64 ws, u64 ss, u64 slot0, u64 slot1, unsigned long long* counter, u64 out_cap,
                                                          u8* key_cls, i64* key_val, u8* agg_cls, i64* agg_val) {
@@ -293,7 +342,8 @@ __global__ void __launch_bounds__(256) k_finalize_groups(const FinalDesc D, int 
         u64 klo = 0, khi = 0;
         u64 pw[64];
         if (live) {
-            if (kw == 1) { klo = keys[i]; live = klo != NQ_U64_MAX; }
+            if (WIDE) live = keys[i * (u64)(kw + 1)] != NQ_U64_MAX;  // kw: key words; the tag of slot i
+            else if (kw == 1) { klo = keys[i]; live = klo != NQ_U64_MAX; }
             else if (kw == 2) { klo = keys[2 * i]; khi = keys[2 * i + 1]; live = !(klo == NQ_U64_MAX && khi == NQ_U64_MAX); }
             else if (kw == 0) klo = i;
         }
@@ -303,7 +353,7 @@ __global__ void __launch_bounds__(256) k_finalize_groups(const FinalDesc D, int 
                 for (int t = 1; t < T.n; ++t) v = word_combine(ops.op[P], v, __ldcg(&T.acc[t][(u64)P * ws + i * ss]));
                 pw[P] = v;
             }
-            if (kw == 0) {  // direct-indexed: a slot holds a group iff its row counter (logical word 0) is not zero
+            if (!WIDE && kw == 0) {  // direct-indexed: a slot holds a group iff its row counter (logical word 0) is not zero
                 const u64 v = pw[D.phys_of[0]];
                 live = (D.bits_of[0] == 64 ? v : (v >> D.shift_of[0]) & 0xffffffffULL) != 0;
             }
@@ -316,8 +366,12 @@ __global__ void __launch_bounds__(256) k_finalize_groups(const FinalDesc D, int 
         if (!live) continue;
         const u64 g = base + (u64)__popc(m & ((1u << lane) - 1u));
         if (g >= out_cap) continue;
-        final_group(D, D.keys, D.nkeys, klo, khi, pw, key_cls + g * D.nkeys, key_val + g * D.nkeys, agg_cls + g * D.naggs,
-                    agg_val + g * D.naggs);
+        if constexpr (WIDE)
+            final_group_bits(D, D.keys, D.nkeys, WordBits{keys + i * (u64)(kw + 1) + 1, 0}, pw, key_cls + g * D.nkeys, key_val + g * D.nkeys,
+                             agg_cls + g * D.naggs, agg_val + g * D.naggs);
+        else
+            final_group(D, D.keys, D.nkeys, klo, khi, pw, key_cls + g * D.nkeys, key_val + g * D.nkeys, agg_cls + g * D.naggs,
+                        agg_val + g * D.naggs);
     }
 }
 
@@ -464,8 +518,12 @@ void launch_finalize_groups(const FinalDesc& D, int kw, const u64* keys, const P
         g_launches.fetch_add(1);
     }
     if (slot1 <= slot0) return;
-    k_finalize_groups<<<grid_for(slot1 - slot0), 256, 0, s>>>(D, kw, keys, T, ops, ws, ss, slot0, slot1, counter, out_cap, key_cls, key_val,
-                                                              agg_cls, agg_val);
+    if (kw >= KW_WIDE)
+        k_finalize_groups<true><<<grid_for(slot1 - slot0), 256, 0, s>>>(D, kw - KW_WIDE, keys, T, ops, ws, ss, slot0, slot1, counter, out_cap, key_cls,
+                                                                        key_val, agg_cls, agg_val);
+    else
+        k_finalize_groups<false><<<grid_for(slot1 - slot0), 256, 0, s>>>(D, kw, keys, T, ops, ws, ss, slot0, slot1, counter, out_cap, key_cls,
+                                                                         key_val, agg_cls, agg_val);
     g_launches.fetch_add(1);
     CK(cudaGetLastError());
 }
@@ -492,19 +550,22 @@ void launch_fill_u64(u64* p, u64 n, u64 v, cudaStream_t s) {
 }
 void launch_count_owners(int kw, const u64* keys, const u64* acc, u64 cap, int nranks, int gk_pos, int gk_bits,
                          unsigned long long* counts, cudaStream_t s) {
-    k_count_owners<<<grid_for(kw == 4 ? cap >> 6 : cap), 256, 0, s>>>(kw, keys, acc, cap, nranks, gk_pos, gk_bits, counts);
+    if (kw >= KW_WIDE) k_count_owners_wide<<<grid_for(cap), 256, 0, s>>>(kw - KW_WIDE, keys, cap, nranks, counts);
+    else k_count_owners<<<grid_for(kw == 4 ? cap >> 6 : cap), 256, 0, s>>>(kw, keys, acc, cap, nranks, gk_pos, gk_bits, counts);
     g_launches.fetch_add(1);
     CK(cudaGetLastError());
 }
 void launch_export_records(int kw, const u64* keys, const u64* acc, u64 cap, int W, int nranks, int gk_pos, int gk_bits,
                            unsigned long long* cursor, u64* out, u64 out_cap, cudaStream_t s) {
-    k_export_records<<<grid_for(kw == 4 ? cap >> 6 : cap), 256, 0, s>>>(kw, keys, acc, cap, W, nranks, gk_pos, gk_bits, cursor, out, out_cap);
+    if (kw >= KW_WIDE) k_export_records_wide<<<grid_for(cap), 256, 0, s>>>(kw - KW_WIDE, keys, acc, cap, W, nranks, cursor, out, out_cap);
+    else k_export_records<<<grid_for(kw == 4 ? cap >> 6 : cap), 256, 0, s>>>(kw, keys, acc, cap, W, nranks, gk_pos, gk_bits, cursor, out, out_cap);
     g_launches.fetch_add(1);
     CK(cudaGetLastError());
 }
 void launch_merge_records(int kw, u64* keys, u64* acc, u64 cap, const OpsArr& ops, const u64* recs, u64 n, int* status, cudaStream_t s) {
     if (n == 0) return;
-    k_merge_records<<<grid_for(n), 256, 0, s>>>(kw, keys, acc, cap, ops, recs, n, status);
+    if (kw >= KW_WIDE) k_merge_records_wide<<<grid_for(n), 256, 0, s>>>(kw - KW_WIDE, keys, acc, cap, ops, recs, n, status);
+    else k_merge_records<<<grid_for(n), 256, 0, s>>>(kw, keys, acc, cap, ops, recs, n, status);
     g_launches.fetch_add(1);
     CK(cudaGetLastError());
 }

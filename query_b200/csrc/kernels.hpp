@@ -10,6 +10,11 @@ struct OpsArr {
     int op[64];
 };
 
+// `kw` of the launchers below: how a table holds its group keys.  0 direct-indexed (slot = key), 1 u64 keys, 2 128-bit
+// keys, 3 the single ungrouped slot, 4 a DISTINCT bitmap, KW_WIDE + n a wide-key table of n key words per slot
+// ([tag, k0 .. k(n-1)], MODE_HASHW), whose records are [k0 .. k(n-1), words] instead of [lo, hi, words]
+constexpr int KW_WIDE = 16;
+
 // one DISTINCT aggregate: where its result words live and how its value component is packed in a set entry
 struct DistinctDesc {
     int sid;           // entry set this aggregate reads (aggregates over the same operand share one)

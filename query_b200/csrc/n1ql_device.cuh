@@ -160,6 +160,77 @@ NQ_DEV i64 table_find128(const ulonglong2* __restrict__ keys, u64 cap_mask, u64 
 }
 #endif
 
+// Keys wider than 127 bits (MODE_HASHW): u64[cap][1 + kw], slot-major - [tag, k0 .. k(kw-1)] - so that one probe reads
+// one contiguous run of words.  tag: EMPTY (all ones), BUSY (claimed, key words being written) or READY (62 bits of the
+// key's hash, top bits clear).  No CAS covers a whole key, so the claim is published after the write: CAS EMPTY -> BUSY,
+// plain stores of the key words, a fence, then a release store of the READY tag; probes acquire the tag before they read
+// words.  A tag only ever moves EMPTY -> BUSY -> READY.  Exact: a slot matches only when all kw words are equal.
+#define NQ_WIDE_BUSY (NQ_U64_MAX - 1)
+NQ_DEV u64 ld_acquire_u64(const u64* p) { u64 v; asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory"); return v; }
+NQ_DEV void st_release_u64(u64* p, u64 v) { asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory"); }
+NQ_DEV u64 wide_hash(const u64* key, int kw) {
+    u64 h = 0x9e3779b97f4a7c15ULL;
+    for (int i = 0; i < kw; ++i) h = mix64(h ^ key[i]);
+    return h;
+}
+NQ_DEV bool wide_equal(const u64* slot_words, const u64* key, int kw) {
+    bool eq = true;
+    for (int i = 0; i < kw; ++i) eq = eq && __ldcg(&slot_words[i]) == key[i];
+    return eq;
+}
+// returns the slot; -1 when the probe budget is exhausted (the host grows the table and reruns); -2 when a claimed slot
+// stayed unpublished for ~1 s (status NQ_WIDE_STUCK: a defect, reported as an error rather than spun on forever)
+NQ_DEV i64 table_insert_wide_n(u64* __restrict__ keys, u64 cap_mask, const u64* key, int kw) {
+    const u64 h = wide_hash(key, kw), tag = h >> 2;
+    u64 slot = h & cap_mask;
+    for (u64 probe = 0; probe <= cap_mask; ++probe) {
+        u64* const s = keys + slot * (u64)(kw + 1);
+        u64 cur = ld_acquire_u64(s);
+        if (cur == NQ_U64_MAX) {
+            if (atomicCAS(s, NQ_U64_MAX, NQ_WIDE_BUSY) == NQ_U64_MAX) {
+                for (int i = 0; i < kw; ++i) s[1 + i] = key[i];
+                __threadfence();
+                st_release_u64(s, tag);
+                return (i64)slot;
+            }
+            cur = ld_acquire_u64(s);  // lost the claim: BUSY or READY now
+        }
+        if (cur == NQ_WIDE_BUSY) {
+            // the claimer is a running thread - with independent thread scheduling also when it is a lane of this warp -
+            // and publishes after kw stores and a fence
+            const long long t0 = clock64();
+            do {
+                __nanosleep(64);
+                if (clock64() - t0 > 2000000000LL) return -2;
+                cur = ld_acquire_u64(s);
+            } while (cur == NQ_WIDE_BUSY);
+        }
+        if (cur == tag && wide_equal(s + 1, key, kw)) return (i64)slot;
+        slot = (slot + 1) & cap_mask;
+        if (probe > 4096) break;
+    }
+    return -1;
+}
+// lookup in a table no thread is writing; -1: absent
+NQ_DEV i64 table_find_wide_n(const u64* __restrict__ keys, u64 cap_mask, const u64* key, int kw) {
+    const u64 h = wide_hash(key, kw), tag = h >> 2;
+    u64 slot = h & cap_mask;
+    for (u64 probe = 0; probe <= cap_mask; ++probe) {
+        const u64* const s = keys + slot * (u64)(kw + 1);
+        if (s[0] == NQ_U64_MAX) return -1;
+        if (s[0] == tag && wide_equal(s + 1, key, kw)) return (i64)slot;
+        slot = (slot + 1) & cap_mask;
+    }
+    return -1;
+}
+// the forms of the generated kernels: KW is a constant, so the loops unroll and the key stays in registers
+template <int KW> NQ_DEV i64 table_insert_wide(u64* __restrict__ keys, u64 cap_mask, const u64 (&key)[KW]) {
+    return table_insert_wide_n(keys, cap_mask, key, KW);
+}
+template <int KW> NQ_DEV i64 table_find_wide(const u64* __restrict__ keys, u64 cap_mask, const u64 (&key)[KW]) {
+    return table_find_wide_n(keys, cap_mask, key, KW);
+}
+
 // 32-bit shared-state-space addresses of the front cache.  Through a generic pointer the compiler rebuilds the block's
 // shared window (S2R SR_CgaCtaId + LEA) at every cache access of the row loop (config 5: 8 times per tile); the address
 // made once by smem_addr is opaque to it, so it stays in a register and every access is one LDS / ATOMS [reg + imm].
@@ -264,6 +335,14 @@ NQ_DEV void pack_bits(u64& lo, u64& hi, int& pos, u64 v, int nbits) {
     } else {
         hi |= v << (pos - 64);
     }
+    pos += nbits;
+}
+// the same into the key words w[] of a wide key (nbits <= 64)
+NQ_DEV void pack_bits(u64* w, int& pos, u64 v, int nbits) {
+    if (nbits == 0) return;
+    const int i = pos >> 6, s = pos & 63;
+    w[i] |= v << s;
+    if (s + nbits > 64) w[i + 1] |= v >> (64 - s);
     pos += nbits;
 }
 

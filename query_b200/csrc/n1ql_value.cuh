@@ -285,17 +285,21 @@ N1_HD u32 inset_slot(u64 key, u32 cap) {
 #endif
 }
 
+// status[1] of a wide-key table (MODE_HASHW) whose slot stayed claimed but unpublished past the wait bound: a defect,
+// reported as an error (never a hang, never a silently lost row)
+#define NQ_WIDE_STUCK 5
+
 // kernel parameter block shared by every generated scan kernel
 struct NqParams {
     i64 nrows;             // rows in this partition
     const void* col[16];   // payload arrays (i64* or u32*), 32-byte aligned, padded to a multiple of 4096 rows
     const u8* tag[16];     // class byte per row
     u64* acc;              // UNGROUPED: per-block partials [grid][nwords]; DENSE/HASH: table words [nwords][cap]
-    u64* keys;             // HASH: slot keys (u64[cap] or ulonglong2[cap])
+    u64* keys;             // HASH: slot keys (u64[cap], ulonglong2[cap], or u64[cap][1 + key words] for wide keys)
     u64 cap_mask;          // HASH: capacity-1
     u64* set_keys;         // DISTINCT entry set (ulonglong2[set_cap] or u64[set_cap])
     u64 set_mask;
-    int* status;           // [0] != 0: a table overflowed (host grows it and reruns)
+    int* status;           // [0] != 0: a table overflowed (host grows it and reruns); [1]: NQ_WIDE_STUCK
     u64 dense_groups;      // DENSE: number of dense slots
     u64* final_dev;        // UNGROUPED: final words [nwords] in HBM (written by the last block to finish)
     u64* final_host;       // UNGROUPED/DENSE: the same words in mapped pinned host memory (zero-copy result)

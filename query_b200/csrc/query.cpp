@@ -155,7 +155,7 @@ void Query::alloc_state() {
             double want = 2.0 * std::min((double)std::max<i64>(table->nrows, 1), (double)std::max<i64>(kp.est_groups, 1));
             cap = pow2_at_least((u64)std::min(std::max(want, 1024.0), 67108864.0));
         }
-        d_keys.ensure((size_t)cap * (kp.mode == MODE_HASH128 ? 16 : 8));
+        d_keys.ensure(key_bytes());
     }
     d_acc.ensure((size_t)cap * W * 8);
     if (kp.ndistinct) {
@@ -193,7 +193,7 @@ void Query::alloc_state() {
     if (small_state()) h_records.ensure((size_t)cap * W * 8);
 }
 
-bool Query::uses_status() const { return kp.mode == MODE_HASH64 || kp.mode == MODE_HASH128 || kp.ndistinct > 0 || mailbox != nullptr; }
+bool Query::uses_status() const { return hashed() || kp.ndistinct > 0 || mailbox != nullptr; }
 
 void Query::attach_mailbox(Mailbox* mb) {
     if (launched) N1_THROW(N1GPU_E_INVALID, "a scan is outstanding");
@@ -233,7 +233,7 @@ Mailbox::~Mailbox() {
 void Query::reset_state() {
     if (uses_status()) CK(cudaMemsetAsync(d_status.p, 0, 64, stream));
     if (kp.mode != MODE_UNGROUPED) launch_init_words(acc(), cap, ops, stream);
-    if (kp.mode == MODE_HASH64 || kp.mode == MODE_HASH128) CK(cudaMemsetAsync(d_keys.p, 0xff, (size_t)cap * (kp.mode == MODE_HASH128 ? 16 : 8), stream));
+    if (hashed()) CK(cudaMemsetAsync(d_keys.p, 0xff, key_bytes(), stream));
     if (kp.ndistinct) CK(cudaMemsetAsync(d_set.p, kp.set_bitmap ? 0 : 0xff, set_bytes(), stream));
 }
 
@@ -372,10 +372,11 @@ bool Query::wait_scan() {
         part_done = false;
         return false;
     }
+    if (kp.mode == MODE_HASHW && h_status.as<int>()[1] == NQ_WIDE_STUCK) N1_THROW(N1GPU_E_CUDA, "a wide-key table slot was claimed and never published");
     if (st == 1) {
         if (cap >= ((u64)1 << 31)) N1_THROW(N1GPU_E_NOMEM, "group table would exceed 2^31 slots");
         cap *= 4;
-        d_keys.alloc((size_t)cap * (kp.mode == MODE_HASH128 ? 16 : 8));
+        d_keys.alloc(key_bytes());
         d_acc.alloc((size_t)cap * ops.n * 8);
         return false;
     }
@@ -457,14 +458,15 @@ void Query::partial_import(const void* dev_records, i64 n, const void* dev_disti
         CK(cudaStreamSynchronize(stream));
         int s0 = h_status.as<int>()[0], s1 = h_status.as<int>()[1];
         if (!s0 && !s1) break;
+        if (kp.mode == MODE_HASHW && s1 == NQ_WIDE_STUCK) N1_THROW(N1GPU_E_CUDA, "a wide-key table slot was claimed and never published");
         // The owner's table (sized for its own partition's groups) is too small for everybody's records: grow what
         // overflowed, clear the state (a half-applied merge cannot be kept: additions are not idempotent) and merge again -
         // the records are still in the caller's buffers.
         if (s0) {
-            if (kp.mode != MODE_HASH64 && kp.mode != MODE_HASH128) N1_THROW(N1GPU_E_INVALID, "a record does not belong to this rank's table (bad key)");
+            if (!hashed()) N1_THROW(N1GPU_E_INVALID, "a record does not belong to this rank's table (bad key)");
             if (cap >= ((u64)1 << 31)) N1_THROW(N1GPU_E_NOMEM, "group table would exceed 2^31 slots");
             cap *= 4;
-            d_keys.alloc((size_t)cap * (kp.mode == MODE_HASH128 ? 16 : 8));
+            d_keys.alloc(key_bytes());
             d_acc.alloc((size_t)cap * ops.n * 8);
         }
         if (s1) {

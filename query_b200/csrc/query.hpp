@@ -178,7 +178,15 @@ struct Query {
                                           const std::vector<ParamValue>& params = {});
     // the scan publishes the whole table to pinned host memory (and may push it through the peer mailbox)
     bool small_state() const { return kp.mode == MODE_UNGROUPED || (kp.mode == MODE_DENSE && !kp.dense_global); }
-    int kw() const { return kp.mode == MODE_UNGROUPED ? 3 : (kp.mode == MODE_DENSE ? 0 : (kp.mode == MODE_HASH64 ? 1 : 2)); }
+    int kw() const {
+        if (kp.mode == MODE_HASHW) return KW_WIDE + kp.key_words;
+        return kp.mode == MODE_UNGROUPED ? 3 : (kp.mode == MODE_DENSE ? 0 : (kp.mode == MODE_HASH64 ? 1 : 2));
+    }
+    bool hashed() const { return kp.mode == MODE_HASH64 || kp.mode == MODE_HASH128 || kp.mode == MODE_HASHW; }
+    size_t key_bytes() const {  // the key array of a hash table
+        return (size_t)cap * 8 * (kp.mode == MODE_HASHW ? 1 + kp.key_words : (kp.mode == MODE_HASH128 ? 2 : 1));
+    }
+    int record_words() const { return (kp.mode == MODE_HASHW ? kp.key_words : 2) + ops.n; }  // n1gpu_query_partial_counts
     void alloc_state();
     bool uses_status() const;         // hash tables / DISTINCT sets can overflow and report it
     void reset_state();               // clears tables (async on stream)
