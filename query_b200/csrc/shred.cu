@@ -603,6 +603,15 @@ void launch_rank_remap(const u8* tags, i64* pay8, u32* pay4, i64 nrows, const u3
     g_launches.fetch_add(1);
     CK(cudaGetLastError());
 }
+__global__ void k_widen_ranks(const u32* __restrict__ pay4, i64* __restrict__ pay8, i64 nrows) {
+    for (i64 row = (i64)blockIdx.x * blockDim.x + threadIdx.x; row < nrows; row += (i64)gridDim.x * blockDim.x) pay8[row] = (i64)pay4[row];
+}
+void launch_widen_ranks(const u32* pay4, i64* pay8, i64 nrows, cudaStream_t s) {
+    if (nrows == 0) return;
+    k_widen_ranks<<<sgrid(nrows, 256), 256, 0, s>>>(pay4, pay8, nrows);
+    g_launches.fetch_add(1);
+    CK(cudaGetLastError());
+}
 void launch_dict_ranks(const u64* slot_of_rank, u64 n, u32* rank, cudaStream_t s) {
     if (n == 0) return;
     k_dict_ranks<<<sgrid((i64)n, 256), 256, 0, s>>>(slot_of_rank, n, rank);

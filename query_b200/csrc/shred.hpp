@@ -26,6 +26,8 @@ void launch_ndjson_scan(const unsigned* counts, i64 nseg, i64* first, i64* tile_
 void launch_ndjson_write(const unsigned char* text, i64 size, const i64* first, i64* offs, cudaStream_t s);
 void launch_gather_offsets(const i64* offs, const i64* rows, i64 n, i64* out, cudaStream_t s);
 void launch_rank_remap(const u8* tags, i64* pay8, u32* pay4, i64 nrows, const u32* remap, u32 n, cudaStream_t s);
+// 4-byte string ranks -> 8-byte payloads, zero-extended (an 8-byte column stores a rank as it is)
+void launch_widen_ranks(const u32* pay4, i64* pay8, i64 nrows, cudaStream_t s);
 void launch_dict_ranks(const u64* slot_of_rank, u64 n, u32* rank, cudaStream_t s);
 void launch_dict_remap(const u8* tags, const i64* slots, i64* payload, u32* out32, i64 nrows, const u32* rank, cudaStream_t s);
 void launch_col_stats(const u8* tags, const i64* payload, i64 nrows, u64* stats, cudaStream_t s);

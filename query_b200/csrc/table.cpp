@@ -585,6 +585,7 @@ void Table::seal() {
         if (any_set)
             for (auto& col : cols)
                 if (!col.on_device) N1_THROW(N1GPU_E_INVALID, "column %s was never set", join_path(col.path, '.').c_str());
+        widen_device_payloads();
         sealed = true;
         return;
     }

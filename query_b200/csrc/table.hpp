@@ -58,9 +58,9 @@ struct ColumnStats {
 ColumnStats host_stats(const std::vector<u8>& tags, const std::vector<i64>& payload);
 
 // Device payload width of a column whose classes are `class_mask`: 8 with numbers, 4 (string ranks) with strings, else 0.
-// seal() applies it to the column's statistics - those of all partitions when stats_set replaced them - while the device
-// shredder and set_column_device apply it to the classes of their own rows: two partitions whose rows differ in classes
-// can then give a device-shredded column different widths.
+// seal() gives every column the width of its statistics - those of all partitions when stats_set replaced them - so that
+// partitions whose rows differ in classes compile the same kernel.  The device shredder and set_column_device first size
+// a column by the classes of their own rows; seal() then widens it (Table::widen_device_payloads).
 inline int width_of(u32 class_mask) { return (class_mask & M_NUM) ? 8 : (class_mask & bit(C_STRING)) ? 4 : 0; }
 
 // The strings of a caller's dictionary (blob + offsets), which must be sorted bytewise and unique (`what` names it)
@@ -173,6 +173,9 @@ struct Table {
     DevBuf device_rows(int width, int byte, cudaStream_t s) const;
 private:
     void check_column_args(int col, int width, i64 n) const;  // set_column / set_column_device
+    // seal() of rows in HBM: columns narrower than width_of(their statistics) get a payload of that width (4-byte ranks
+    // zero-extended, a width-0 column zeros)
+    void widen_device_payloads();
 };
 
 // The host shredder applied to selected documents (the device shredder's fix-up rows).  Per column: tags[n],

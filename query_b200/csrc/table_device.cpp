@@ -524,6 +524,21 @@ void Table::remap_ranks_device(int ci, const std::vector<u32>& remap) {
     CK(cudaDeviceSynchronize());
 }
 
+void Table::widen_device_payloads() {
+    bool any = false;
+    for (auto& col : cols) {
+        const int w = width_of(col.stats.class_mask);
+        if (w == col.width) continue;
+        if (w < col.width) N1_THROW(N1GPU_E_INVALID, "column %s: its statistics lack classes its rows hold", join_path(col.path, '.').c_str());
+        DevBuf wide = device_rows(w, 0, nullptr);  // a width-0 column had no payload: zeros
+        if (col.width == 4) launch_widen_ranks(col.d_payload.as<u32>(), wide.as<i64>(), nrows, nullptr);
+        col.d_payload = std::move(wide);
+        col.width = w;
+        any = true;
+    }
+    if (any) CK(cudaDeviceSynchronize());
+}
+
 void Table::set_column_device(int c, int width, const void* dev_payload, const u8* dev_tags, i64 n, const char* blob,
                               const i64* offs, i64 ndict) {
     if (!have_device()) N1_THROW(N1GPU_E_CUDA, "no CUDA device: device columns need one");
@@ -555,7 +570,7 @@ void Table::set_column_device(int c, int width, const void* dev_payload, const u
         N1_THROW(N1GPU_E_INVALID, "a column of strings only must be passed as 4-byte ranks");
     st.set_dictionary(col.dict);
     if (!col.stats_forced) col.stats = st;
-    col.width = width_of(col.stats.class_mask);
+    col.width = width_of(st.class_mask);  // of its own rows, as the device shredder; seal() widens it to the statistics'
     if (col.width == 0) col.d_payload = device_rows(0, 0, nullptr);
     col.on_device = true;
     filled = Fill::DEVICE_COLUMNS;  // nothing left to do at seal

@@ -102,7 +102,7 @@ def test_send_stop_aborts_a_running_scan(monkeypatch):
     import torch
     import workloads as wl
     monkeypatch.setenv("N1GPU_NO_CACHE", "1")  # every row of a hot Zipf key is an L2 atomic on one address: a slow scan
-    w = wl.Config5(scale=0.1)
+    w = wl.Config5(scale=0.2)  # a scan of about 20 ms on a B200: long enough to stop well before its end
     t = w.sealed_table()
     qq = w.query(t)
     qq.execute()
